@@ -62,7 +62,12 @@ def parse():
     ap.add_argument("--group", type=int, default=GROUP,
                     help="consecutive sessions per trace (default 64: every 64-thread block of the fused kernel follows "
                          "one trace and stages it in shared memory; 1 = trace = session mod n_traces, global path)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy: the [48][n] "
+                         "trajectories of a fixed sample of the sessions and the statistics vector (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     globals()["GROUP"] = args.group
     return args
 
@@ -265,6 +270,28 @@ def parity_mpc(menv, H, act, sample=2048):
                 seconds=time.perf_counter() - t0)
 
 
+DUMP_SESSIONS = 16384               # sessions in the --dump-outputs sample: 48 x 16 384 x (5 x 8 + 4) B = 34.6 MB
+
+
+def dump_outputs(path, out, stats):
+    """--dump-outputs: what the last timed step handed back to its caller, as <path>/<name>.npy.  The five [48][N] fp64
+    trajectories and end_of_video (as float32) are reduced to the same fixed, seeded sample of session columns (ascending
+    order), so the files stay far below 64 MB at any --sessions; the statistics vector is written whole.  The inputs
+    depend on the arguments only (seeded synthetic traces, video and sessions), so two builds run with the same
+    arguments can be compared file by file.  Under torchrun rank 0 writes its own shard."""
+    import numpy as np
+    import torch
+    N = out["reward"].shape[1]
+    cols = np.sort(np.random.default_rng(SEED).choice(N, size=min(N, DUMP_SESSIONS), replace=False))
+    ix = torch.from_numpy(cols).to(out["reward"].device)
+    arrays = {k: out[k].index_select(1, ix).cpu().numpy() for k in ("delay", "sleep", "buffer", "rebuffer", "reward")}
+    arrays["end_of_video"] = out["end_of_video"].index_select(1, ix).cpu().numpy().astype(np.float32)
+    arrays["stats"] = stats.cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def workload_config(args):
     return dict(workload="configs[1]: random-policy chunk-step sweep, fused 48-chunk episodes",
                 sessions_per_gpu=args.sessions, chunks=V, bitrates=A, n_traces=N_TRACES, trace_segments=T_TRACE,
@@ -299,6 +326,9 @@ class ClockSampler:
                                          stderr=subprocess.DEVNULL, text=True)
         except Exception:
             self.proc = None
+            return
+        import atexit
+        atexit.register(self.proc.kill)                        # a run that fails before stop() leaves no poller behind
 
     def pause(self, on=True):
         """SIGSTOP / SIGCONT the poller: nvidia-smi queries take driver locks that the launch- and sync-latency
@@ -442,6 +472,8 @@ def run_ours(args):
         events.append((e0, e1, k0, k1))
     barrier()
     wall = time.perf_counter() - wall0
+    if rank == 0 and args.dump_outputs:                        # before any later leg overwrites `out`
+        dump_outputs(args.dump_outputs, out, stats)
     step_ms = [e0.elapsed_time(e1) for e0, e1, _, _ in events]
     kern_ms = [k0.elapsed_time(k1) for _, _, k0, k1 in events]
     launches = _lib.launch_count() - launches0

@@ -1,5 +1,5 @@
-import sys, ctypes as C
-sys.path.insert(0, "/root/repo")
+import os, sys, ctypes as C
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from abrsimulator_b200 import synth, _lib
 from abrsimulator_b200.env import BatchedABREnv
