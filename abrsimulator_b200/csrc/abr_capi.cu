@@ -8,7 +8,6 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
-#include <type_traits>
 #include <vector>
 
 #include "abr_common.cuh"
@@ -292,10 +291,32 @@ int abr_sort_by_trace(const int32_t* d_trace_id, int n_sessions, int n_traces, i
     return ABR_OK;
 }
 
+static int check_capacity(const AbrEnv* env, int n_sessions) {
+    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    return ABR_OK;
+}
+
+// A batch of n_sessions fits the environment and the session order installed for it, if any.
+static int check_batch(const AbrEnv* env, int n_sessions) {
+    if (int rc = check_capacity(env, n_sessions)) return rc;
+    if (env->v.perm && env->n_order != n_sessions)
+        return fail(ABR_ERR_STATE, "the installed session order has %d entries, the batch %d (abr_env_set_order)", env->n_order, n_sessions);
+    return ABR_OK;
+}
+
+// What a reset does to the handle: a batch of n_sessions, numbered from session_base, with no steps taken yet.
+static void begin_batch(AbrEnv* env, int n_sessions, long long session_base) {
+    env->v.n = n_sessions;
+    env->v.session_base = session_base;
+    env->fresh_partials = 0;
+    env->was_reset = true;
+    env->step_base = 0;
+}
+
 int abr_env_set_order(AbrEnv* env, const int32_t* d_perm, int n_sessions, void* stream) {
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
     if (!d_perm) { env->v.perm = nullptr; env->n_order = 0; return ABR_OK; }
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    if (int rc = check_capacity(env, n_sessions)) return rc;
     if (!env->d_perm) CUDA_TRY(env->alloc(&env->d_perm, (size_t)env->v.cap));
     CUDA_TRY(cudaMemcpyAsync(env->d_perm, d_perm, sizeof(int32_t) * n_sessions, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     env->v.perm = env->d_perm;
@@ -306,14 +327,8 @@ int abr_env_set_order(AbrEnv* env, const int32_t* d_perm, int n_sessions, void* 
 int abr_env_reset(AbrEnv* env, const int32_t* d_trace_id, const double* d_start_offset, int n_sessions,
                   long long session_base, void* stream) {
     if (!env || (!d_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
-    if (env->v.perm && env->n_order != n_sessions)
-        return fail(ABR_ERR_STATE, "the installed session order has %d entries, the batch %d (abr_env_set_order)", env->n_order, n_sessions);
-    env->v.n = n_sessions;
-    env->v.session_base = session_base;
-    env->fresh_partials = 0;
-    env->was_reset = true;
-    env->step_base = 0;
+    if (int rc = check_batch(env, n_sessions)) return rc;
+    begin_batch(env, n_sessions, session_base);
     CUDA_TRY(launch_reset(env->v, d_trace_id, d_start_offset, env->d_draw_counter, (cudaStream_t)stream));
     return ABR_OK;
 }
@@ -329,7 +344,7 @@ int abr_env_get_order(AbrEnv* env, int32_t* d_perm, int n_sessions, void* stream
 int abr_env_reset_sorted(AbrEnv* env, const int32_t* d_trace_id, const double* d_start_offset, int n_sessions,
                          long long session_base, void* stream) {
     if (!env || (!d_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    if (int rc = check_capacity(env, n_sessions)) return rc;
     if (d_trace_id == env->d_trace_id || (d_start_offset && d_start_offset == env->d_offset))
         return fail(ABR_ERR_INVALID, "the inputs alias the environment's own scratch");
     cudaStream_t st = (cudaStream_t)stream;
@@ -365,7 +380,7 @@ int abr_env_reset_sorted(AbrEnv* env, const int32_t* d_trace_id, const double* d
 int abr_env_reset_host(AbrEnv* env, const int32_t* h_trace_id, const double* h_start_offset, int n_sessions,
                        long long session_base, void* stream) {
     if (!env || (!h_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    if (int rc = check_capacity(env, n_sessions)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     CUDA_TRY(cudaMemcpyAsync(env->d_trace_id, h_trace_id, sizeof(int32_t) * n_sessions, cudaMemcpyHostToDevice, st));
     if (h_start_offset)
@@ -383,8 +398,10 @@ static int env_step_any(AbrEnv* env, const int32_t* d_action, const double* d_sp
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
     env->fresh_partials = 0;
-    CUDA_TRY(launch_step(env->v, d_action, d_speed, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_latency,
-                         d_next_sizes, d_end_of_video, d_throughput, (cudaStream_t)stream));
+    StepOutputs<OT> o;
+    o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
+    o.eov = d_end_of_video; o.latency = d_latency; o.thr = d_throughput; o.next_sizes = d_next_sizes;
+    CUDA_TRY(launch_step(env->v, d_action, d_speed, o, (cudaStream_t)stream));
     return ABR_OK;
 }
 }  // extern "C++"
@@ -414,8 +431,10 @@ int abr_env_step_policy(AbrEnv* env, const float* d_logits, int sample, uint64_t
         pol.s_delay = spec->delay_scale; pol.s_size = spec->size_scale;
     }
     env->fresh_partials = 0;
-    CUDA_TRY(launch_step_policy(env->v, pol, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_end_of_video,
-                                env->d_draw_counter, (cudaStream_t)stream));
+    StepOutputs<double> o;
+    o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
+    o.eov = d_end_of_video;
+    CUDA_TRY(launch_step_policy(env->v, pol, o, env->d_draw_counter, (cudaStream_t)stream));
     return ABR_OK;
 }
 
@@ -457,15 +476,11 @@ static int env_rollout_any(AbrEnv* env, int policy, uint64_t seed, int steps, co
     if ((unsigned long long)steps * (unsigned long long)env->v.n > 0xffffffffull)
         return fail(ABR_ERR_RANGE, "steps * sessions = %llu exceeds 2^32 - 1: split the episode into several calls",
                     (unsigned long long)steps * (unsigned long long)env->v.n);
-    if constexpr (std::is_same<OT, double>::value) {
-        CUDA_TRY(launch_rollout(env->v, policy, seed, steps, d_actions_in, d_speed, d_delay, d_sleep, d_buffer, d_rebuf,
-                                d_reward, d_latency, d_end_of_video, d_actions_out, env->d_stats_partials,
-                                (cudaStream_t)stream, fused, env->step_base));
-    } else {
-        CUDA_TRY(launch_rollout(env->v, policy, seed, steps, d_actions_in, d_speed, d_delay, d_sleep, d_buffer, d_rebuf,
-                                d_reward, d_latency, d_end_of_video, d_actions_out, env->d_stats_partials,
-                                (cudaStream_t)stream, env->step_base));
-    }
+    StepOutputs<OT> o;
+    o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
+    o.eov = d_end_of_video; o.actions = d_actions_out; o.latency = d_latency;
+    CUDA_TRY(launch_rollout(env->v, policy, seed, steps, env->step_base, d_actions_in, d_speed, o, env->d_stats_partials,
+                            fused, (cudaStream_t)stream));
     env->step_base += (uint32_t)steps;
     env->fresh_partials = steps > 0 ? rollout_num_blocks(env->v.n) : 0;
     return ABR_OK;
@@ -586,20 +601,15 @@ int abr_env_run(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t
                 double* d_delay, double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward,
                 uint8_t* d_end_of_video, int32_t* d_actions_out, double* d_qoe_cost, double* d_stats, void* stream) {
     if (!env || (!d_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    int rc = check_capacity(env, n_sessions);
+    if (rc) return rc;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
     if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BBA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
     if (policy == ABR_POLICY_FIXED && !d_actions_in && n_sessions > 0 && steps > 0)
         return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
-    int rc;
-    if (env->v.perm && env->n_order != n_sessions)
-        return fail(ABR_ERR_STATE, "the installed session order has %d entries, the batch %d (abr_env_set_order)", env->n_order, n_sessions);
+    if ((rc = check_batch(env, n_sessions))) return rc;
     if (n_sessions > 0 && steps > 0) {   // the episode kernel resets the sessions itself and writes the session cost
-        env->v.n = n_sessions;
-        env->v.session_base = session_base;
-        env->fresh_partials = 0;
-        env->was_reset = true;
-        env->step_base = 0;
+        begin_batch(env, n_sessions, session_base);
         RolloutFused fused;
         fused.in_trace_id = d_trace_id; fused.in_offset = d_start_offset; fused.out_cost = d_qoe_cost;
         fused.out_stats = d_stats; fused.scratch = env->stats_scratch;   // statistics by the kernel's own blocks
@@ -635,11 +645,11 @@ int abr_env_run_host(AbrEnv* env, int policy, uint64_t seed, int steps, const in
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
     if (!h_trace_id && n_sessions > 0) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (n_sessions < 0 || n_sessions > env->v.cap) return fail(ABR_ERR_RANGE, "n_sessions %d exceeds capacity %d", n_sessions, env->v.cap);
+    int rc = check_capacity(env, n_sessions);
+    if (rc) return rc;
     if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BBA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
     if (policy == ABR_POLICY_FIXED && !h_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs h_actions_in");
-    if (env->v.perm && env->n_order != n_sessions)
-        return fail(ABR_ERR_STATE, "the installed session order has %d entries, the batch %d (abr_env_set_order)", env->n_order, n_sessions);
+    if ((rc = check_batch(env, n_sessions))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // inputs: device aliases of page-locked buffers (read over PCIe by the kernel), else staged copies
     const int32_t* tid = (const int32_t*)device_alias(h_trace_id);
@@ -660,13 +670,8 @@ int abr_env_run_host(AbrEnv* env, int policy, uint64_t seed, int steps, const in
     // no episode to run; the per-session cost goes straight to a page-locked h_qoe_cost from the same kernel.
     const bool fuse = n_sessions > 0 && steps > 0;
     double* z_cost = fuse ? (double*)device_alias(h_qoe_cost) : nullptr;
-    int rc;
     if (fuse) {
-        env->v.n = n_sessions;
-        env->v.session_base = session_base;
-        env->fresh_partials = 0;
-        env->was_reset = true;
-        env->step_base = 0;
+        begin_batch(env, n_sessions, session_base);
     } else {
         rc = abr_env_reset(env, tid, off, n_sessions, session_base, stream);
         if (rc) return rc;

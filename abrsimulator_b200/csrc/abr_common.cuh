@@ -140,12 +140,30 @@ struct StepPolicy {
     double s_buffer = 1.0, s_thr = 1.0, s_delay = 1.0, s_size = 1.0;   // observation scales
     double* __restrict__ reward_sum = nullptr;     // [N]: += reward, nullable
 };
-cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, double* d_delay, double* d_sleep, double* d_buffer,
-                               double* d_rebuf, double* d_reward, uint8_t* d_eov, uint32_t* d_draw_counter,
-                               cudaStream_t st);
-cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, double* d_delay,
-                        double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward, double* d_latency,
-                        double* d_next_sizes, uint8_t* d_eov, double* d_thr, cudaStream_t st);
+// Per-step outputs of both step launchers: element ix of each array ([N] for a step, [steps][N] for an episode,
+// next_sizes [N][A]); every pointer is nullable.  OT: double, or float for the fp32-output mode (the arithmetic stays
+// fp64, an output is rounded once on the store).
+template <typename OT>
+struct StepOutputs {
+    OT* __restrict__ delay = nullptr; OT* __restrict__ sleep = nullptr; OT* __restrict__ buffer = nullptr;
+    OT* __restrict__ rebuf = nullptr; OT* __restrict__ reward = nullptr; uint8_t* __restrict__ eov = nullptr;
+    int32_t* __restrict__ actions = nullptr;      // episode only: the action of every step
+    OT* __restrict__ latency = nullptr;           // live mode (SPEC §7); the per-step kernel writes 0 outside it
+    OT* __restrict__ thr = nullptr;               // per-step kernel only
+    OT* __restrict__ next_sizes = nullptr;        // per-step kernel only
+    // the five f64 outputs and end_of_video, which the FAST kernels store without null checks
+    bool has_core() const { return delay && sleep && buffer && rebuf && reward && eov; }
+    // no output at all: the NOOUT episode kernels
+    bool none() const {
+        return !delay && !sleep && !buffer && !rebuf && !reward && !eov && !actions && !latency && !thr && !next_sizes;
+    }
+};
+cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const StepOutputs<double>& o,
+                               uint32_t* d_draw_counter, cudaStream_t st);
+// d_speed (live mode): the playback speed of content chunk k of session i is d_speed[k * N + i]; nullable = 1.0
+template <typename OT>
+cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, const StepOutputs<OT>& o,
+                        cudaStream_t st, const StepPolicy* policy = nullptr);
 // Fused reset + episode + session cost (abr_env_run_host): with in_trace_id the episode kernel resets every session
 // itself (SPEC §2) and out_cost receives Simulator.calculate_qoe per session; the pointers may alias pinned host memory.
 // Scratch of the statistics reduction (SPEC §6): one sum per group of block partials, and the counters of finished
@@ -156,19 +174,11 @@ struct RolloutFused {
     const int32_t* in_trace_id = nullptr; const double* in_offset = nullptr; double* out_cost = nullptr;
     double* out_stats = nullptr; StatsScratch scratch;
 };
-cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, const int32_t* d_actions_in,
-                           const double* d_speed, double* d_delay, double* d_sleep, double* d_buffer, double* d_rebuf,
-                           double* d_reward, double* d_latency, uint8_t* d_eov, int32_t* d_actions_out,
-                           double* d_block_partials, cudaStream_t st, const RolloutFused& f = RolloutFused{},
-                           uint32_t step_base = 0);
-// fp32-output overloads (arithmetic stays fp64; outputs are rounded once on the store)
-cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, float* d_delay,
-                        float* d_sleep, float* d_buffer, float* d_rebuf, float* d_reward, float* d_latency,
-                        float* d_next_sizes, uint8_t* d_eov, float* d_thr, cudaStream_t st);
-cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, const int32_t* d_actions_in,
-                           const double* d_speed, float* d_delay, float* d_sleep, float* d_buffer, float* d_rebuf,
-                           float* d_reward, float* d_latency, uint8_t* d_eov, int32_t* d_actions_out,
-                           double* d_block_partials, cudaStream_t st, uint32_t step_base = 0);
+// step_base: episode steps since the last reset (the random policy's counter, SPEC §4)
+template <typename OT>
+cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, uint32_t step_base,
+                           const int32_t* d_actions_in, const double* d_speed, const StepOutputs<OT>& o,
+                           double* d_block_partials, const RolloutFused& f, cudaStream_t st);
 cudaError_t launch_stats(const EnvView& v, double* d_partials, int n_partials, bool have_partials, double* d_out,
                          const StatsScratch& scratch,
                          cudaStream_t st);

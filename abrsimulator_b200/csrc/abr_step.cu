@@ -739,39 +739,74 @@ __device__ __forceinline__ int policy_action(const EnvView& v, const StepPolicy&
     return arg;
 }
 
-// `q`: the action, already clamped to [0, A); `lk`: the step's table reads (the caller issues them as soon as it holds
-// the session's state words, next to the read of the trace record, so that the two L2 round trips overlap).
-template <bool SMEM, bool FAST, bool LIVE, bool POL, typename OT>
-__device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const int i, const int q, const Lookup& lk,
-                                             const StepPolicy& pol,
-                                             const double* __restrict__ speed, OT* __restrict__ o_delay,
-                                             OT* __restrict__ o_sleep, OT* __restrict__ o_buffer,
-                                             OT* __restrict__ o_rebuf, OT* __restrict__ o_reward,
-                                             OT* __restrict__ o_latency, OT* __restrict__ o_next_sizes,
-                                             uint8_t* __restrict__ o_eov, OT* __restrict__ o_thr) {
-    if (LIVE) {
+// Live-mode words of session i (SPEC §7): from the SoA state, or those of a fresh reset.  speed: the [V][N] table of
+// playback speeds (the speed of content chunk k is speed[k][i]), nullable = 1.0.
+__device__ __forceinline__ void load_live(const EnvView& v, Sess& s, const int i, const double* __restrict__ speed,
+                                          const bool fresh) {
+    if (fresh) { s.t_now = 0.0; s.play_time = 0.0; s.play_len = 0.0; s.play_id = 0; s.started = v.p.start_up_length <= 0.0; }
+    else {
         s.t_now = v.t_now[i]; s.play_time = v.play_time[i]; s.started = v.started[i] != 0;
         s.play_id = v.play_id[i]; s.play_len = v.play_len[i];
-        s.speed = speed ? speed + i : nullptr;   // [V][N] table: the speed of content chunk k is speed[k][i]
-        s.speed_stride = (size_t)v.n; s.V = v.V; s.bad_speed = false;
     }
+    s.speed = speed ? speed + i : nullptr;
+    s.speed_stride = (size_t)v.n; s.V = v.V; s.bad_speed = false;
+}
+
+// The SoA state words a step changes (LIVE: with the live-mode ones).
+template <bool LIVE>
+__device__ __forceinline__ void store_state(const EnvView& v, const Sess& s, const int i) {
+    v.seg[i] = s.seg; v.chunk[i] = s.chunk; v.last_q[i] = s.last_q; v.phi[i] = s.phi; v.pos[i] = s.pos;
+    v.buffer[i] = s.buffer;
+    if (LIVE) {
+        v.t_now[i] = s.t_now; v.play_time[i] = s.play_time; v.started[i] = s.started ? 1 : 0;
+        v.play_id[i] = s.play_id; v.play_len[i] = s.play_len;
+    }
+}
+
+// A step's trajectory outputs at element ix of [steps][N], streamed out (st.global.cs).  FAST: the five f64 outputs and
+// end_of_video are all requested and stored without null checks; NOOUT: none is requested; LIVE: the latency too,
+// where requested.
+template <bool FAST, bool NOOUT, bool LIVE, typename OT>
+__device__ __forceinline__ void store_step(const StepOutputs<OT>& o, const uint32_t ix, const StepRes& r) {
+    if (NOOUT) {
+    } else if (FAST) {
+        __stcs(o.delay + ix, (OT)r.delay); __stcs(o.sleep + ix, (OT)r.sleep); __stcs(o.buffer + ix, (OT)r.buffer);
+        __stcs(o.rebuf + ix, (OT)r.rebuf); __stcs(o.reward + ix, (OT)r.reward);
+        o.eov[ix] = r.eov ? 1 : 0;
+    } else {
+        if (o.delay) __stcs(o.delay + ix, (OT)r.delay);
+        if (o.sleep) __stcs(o.sleep + ix, (OT)r.sleep);
+        if (o.buffer) __stcs(o.buffer + ix, (OT)r.buffer);
+        if (o.rebuf) __stcs(o.rebuf + ix, (OT)r.rebuf);
+        if (o.reward) __stcs(o.reward + ix, (OT)r.reward);
+        if (o.eov) o.eov[ix] = r.eov ? 1 : 0;
+        if (LIVE && o.latency) __stcs(o.latency + ix, (OT)r.latency);
+    }
+}
+
+// `q`: the action, already clamped to [0, A); `lk`: the step's table reads (the caller issues them as soon as it holds
+// the session's state words, next to the read of the trace record, so that the two L2 round trips overlap).
+// The outputs arrive as __restrict__ parameters (of the kernel and of this function), not as StepOutputs: nvcc drops
+// the qualifier on struct members, and without it the per-step kernels lose the no-alias facts their schedule is built
+// on (both forms measured slower on a B200: 0.2-0.3 us of 104 per launch at 4 Mi sessions).
+template <bool SMEM, bool FAST, bool LIVE, bool POL, typename OT>
+__device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const int i, const int q, const Lookup& lk,
+                                             const StepPolicy& pol, const double* __restrict__ speed,
+                                             OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer,
+                                             OT* __restrict__ o_rebuf, OT* __restrict__ o_reward, uint8_t* __restrict__ o_eov,
+                                             OT* __restrict__ o_latency, OT* __restrict__ o_thr, OT* __restrict__ o_next_sizes) {
+    if (LIVE) load_live(v, s, i, speed, false);
     StepRes r;
     step_core<SMEM, FAST, LIVE>(v, s, q, lk, r, (!FAST && v.p.track_history) || o_thr != nullptr || (POL && pol.obs));
     if (r.walk_error || (LIVE && s.bad_speed)) atomicAdd(v.errors, 1ull);
     if (FAST) {
-        v.seg[i] = s.seg; v.chunk[i] = s.chunk; v.last_q[i] = s.last_q; v.phi[i] = s.phi; v.pos[i] = s.pos;
-        v.buffer[i] = s.buffer;
+        store_state<false>(v, s, i);
         __stcs(o_delay + i, (OT)r.delay); __stcs(o_sleep + i, (OT)r.sleep); __stcs(o_buffer + i, (OT)r.buffer);
         __stcs(o_rebuf + i, (OT)r.rebuf); __stcs(o_reward + i, (OT)r.reward);
         o_eov[i] = r.eov ? 1 : 0;
     } else {
         if (!r.inert) {
-            v.seg[i] = s.seg; v.chunk[i] = s.chunk; v.last_q[i] = s.last_q; v.phi[i] = s.phi; v.pos[i] = s.pos;
-            v.buffer[i] = s.buffer;
-            if (LIVE) {
-                v.t_now[i] = s.t_now; v.play_time[i] = s.play_time; v.started[i] = s.started ? 1 : 0;
-                v.play_id[i] = s.play_id; v.play_len[i] = s.play_len;
-            }
+            store_state<LIVE>(v, s, i);
             if (v.p.track_history) {
                 // ring slot of this sample = (hist_len before the step) mod K; after an auto-reset hist_len is 0
                 const int prev_len = r.reset_mpc ? 0 : s.hist_len - 1;
@@ -819,7 +854,7 @@ __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const in
                        (float)((!FAST && s.done) ? 0.0 : dmul(__ldg(v.sizes + s.chunk * A + a), pol.s_size)));
         }
     }
-    if (o_latency) __stcs(o_latency + i, (OT)r.latency);
+    if (o_latency) __stcs(o_latency + i, (OT)r.latency);   // 0 outside live mode
     if (o_thr) __stcs(o_thr + i, (OT)r.thr);
     if (o_next_sizes) {
         const int A = v.A;
@@ -838,14 +873,12 @@ __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const in
 template <bool FAST, bool LIVE, bool POL, typename OT>
 __global__ void __launch_bounds__(kTile, (LIVE || POL) ? 4 : kTileBlocksPerSM)
 abr_step_kernel(EnvView v, const int32_t* __restrict__ action, const double* __restrict__ speed,
-                OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer,
-                OT* __restrict__ o_rebuf, OT* __restrict__ o_reward, OT* __restrict__ o_latency,
-                OT* __restrict__ o_next_sizes, uint8_t* __restrict__ o_eov, OT* __restrict__ o_thr,
-                int smem_doubles, int tiles_per_block, const StepPolicy pol) {
+                OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer, OT* __restrict__ o_rebuf,
+                OT* __restrict__ o_reward, OT* __restrict__ o_latency, OT* __restrict__ o_next_sizes,
+                uint8_t* __restrict__ o_eov, OT* __restrict__ o_thr, int smem_doubles, int tiles_per_block, const StepPolicy pol) {
     extern __shared__ __align__(16) double2 s_row2[];
     __shared__ __align__(8) unsigned long long s_mbar;
     __shared__ Quad s_meta;                      // the record of the trace whose rows are staged
-#define ABR_STEP_SESSION_ARGS v, s, i, q_cur, lk, pol, speed, o_delay, o_sleep, o_buffer, o_rebuf, o_reward, o_latency, o_next_sizes, o_eov, o_thr
     const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&s_mbar);
     if (smem_doubles != 0) {
         if (threadIdx.x == 0) {
@@ -926,7 +959,11 @@ abr_step_kernel(EnvView v, const int32_t* __restrict__ action, const double* __r
         }
         const int tr = valid ? w.tr : -1;
         if (smem_doubles == 0) {                 // launch-uniform: no shared-memory row buffer
-            if (valid) { make_sess(v, i, w, s); step_session<false, FAST, LIVE, POL, OT>(ABR_STEP_SESSION_ARGS); }
+            if (valid) {
+                make_sess(v, i, w, s);
+                step_session<false, FAST, LIVE, POL, OT>(v, s, i, q_cur, lk, pol, speed, o_delay, o_sleep, o_buffer, o_rebuf,
+                                                         o_reward, o_eov, o_latency, o_thr, o_next_sizes);
+            }
             continue;
         }
         if (tr_first == tr_last && tr_first != staged) {   // block-uniform: stage another trace's rows
@@ -954,14 +991,15 @@ abr_step_kernel(EnvView v, const int32_t* __restrict__ action, const double* __r
                 ABR_CHECK(row_bytes_of(s.T) <= 8u * (uint32_t)smem_doubles && idx_bytes_of(s.M) <= 2u * (uint32_t)idx_stride(v.T_max),
                           "staged rows fit the shared-memory buffer");
 #endif
-                step_session<true, FAST, LIVE, POL, OT>(ABR_STEP_SESSION_ARGS);
+                step_session<true, FAST, LIVE, POL, OT>(v, s, i, q_cur, lk, pol, speed, o_delay, o_sleep, o_buffer, o_rebuf,
+                                                        o_reward, o_eov, o_latency, o_thr, o_next_sizes);
             } else {
                 make_sess(v, i, w, s);
-                step_session<false, FAST, LIVE, POL, OT>(ABR_STEP_SESSION_ARGS);
+                step_session<false, FAST, LIVE, POL, OT>(v, s, i, q_cur, lk, pol, speed, o_delay, o_sleep, o_buffer, o_rebuf,
+                                                         o_reward, o_eov, o_latency, o_thr, o_next_sizes);
             }
         }
     }
-#undef ABR_STEP_SESSION_ARGS
 }
 
 // Per-session QoE cost of Simulator.calculate_qoe (Simulator.py:83-86) from the accumulators:
@@ -1072,10 +1110,8 @@ __device__ __forceinline__ void stats_finish(const double* __restrict__ partials
 
 template <typename OT>
 struct RolloutOut {
-    OT* __restrict__ delay; OT* __restrict__ sleep; OT* __restrict__ buffer; OT* __restrict__ rebuf;
-    OT* __restrict__ reward; uint8_t* __restrict__ eov; int32_t* __restrict__ actions;
-    OT* __restrict__ latency;                // live mode only (SPEC §7), nullable
-    const double* __restrict__ speed;        // live mode only: playback speed [steps][N], nullable = 1.0
+    StepOutputs<OT> traj;                    // [steps][N]
+    const double* __restrict__ speed;        // live mode only: playback speed [V][N], nullable = 1.0
     // fused reset + episode + session cost (abr_env_run_host): with in_trace_id the kernel resets every session itself
     // (SPEC §2) instead of loading its state, and out_cost receives Simulator.calculate_qoe per session.  Both may
     // be device aliases of page-locked HOST memory: the inputs are then pulled and the result pushed over PCIe by
@@ -1088,6 +1124,30 @@ struct RolloutOut {
     double* __restrict__ out_stats;          // nullable; may alias page-locked host memory
     StatsScratch scratch;
 };
+
+// What the fused episode adds up over one session's steps (the accumulators of SPEC §6), and whether an auto-reset
+// happened (it also clears the robust-MPC predictor state).
+struct EpisodeSums {
+    double rew = 0.0, reb = 0.0, u = 0.0, sm = 0.0, sl = 0.0, dl = 0.0, su = 0.0, lat = 0.0, pl = 0.0;
+    int steps = 0, eps = 0;
+    bool reset_mpc = false;
+};
+
+// Adds one (not inert) step.  COUNT: count it and its end of episode here, note an auto-reset and record the
+// throughput sample in the history ring (hist); without COUNT the caller has all of that in closed form.
+template <bool LIVE, bool COUNT>
+__device__ __forceinline__ void add_step(EpisodeSums& a, const StepRes& r, const EnvView& v, const Sess& s, const int i,
+                                         const bool hist) {
+    a.rew = dadd(a.rew, r.reward); a.reb = dadd(a.reb, r.rebuf); a.u = dadd(a.u, r.u);
+    a.sm = dadd(a.sm, r.smooth); a.sl = dadd(a.sl, r.sleep); a.dl = dadd(a.dl, r.delay);
+    if (LIVE) { a.su = dadd(a.su, r.startup); a.lat = dadd(a.lat, r.area); a.pl = dadd(a.pl, r.played); }
+    if (COUNT) {
+        a.steps += 1;
+        a.eps += r.eov ? 1 : 0;
+        if (r.reset_mpc) a.reset_mpc = true;
+        else if (hist) v.bw_hist[(size_t)((s.hist_len - 1) % v.K) * v.cap + i] = r.thr;
+    }
+}
 
 // `steps` chunk steps of one session with the state in registers (SPEC §3+§4).
 // FAST: the common shape — all six trajectory outputs requested, no action trace, no throughput history,
@@ -1111,23 +1171,14 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     constexpr bool AHEAD = POLICY != ABR_POLICY_BBA && !LIVE;
     // the random policy is keyed by the caller's session index, whatever order the environment keeps the sessions in
     const unsigned long long gsession = (unsigned long long)(v.session_base + (v.perm ? __ldg(v.perm + i) : i));
-    double a_rew = 0.0, a_reb = 0.0, a_u = 0.0, a_sm = 0.0, a_sl = 0.0, a_dl = 0.0, a_su = 0.0, a_lat = 0.0, a_pl = 0.0;
-    int n_steps = 0, n_eps = 0;
+    EpisodeSums sum;
     const int chunk_in = s.chunk;
-    bool flagged = false, reset_mpc = false;
+    bool flagged = false;
     const uint32_t n = (uint32_t)v.n;
     const bool hist = !FAST && v.p.track_history != 0;
     const bool prev_ladder = v.p.smooth_prev_ladder != 0;
     uint32_t packed = 0u;   // random policy: the eight actions of one Philox block, one per nibble
-    if (LIVE) {
-        if (fresh) { s.t_now = 0.0; s.play_time = 0.0; s.play_len = 0.0; s.play_id = 0; s.started = v.p.start_up_length <= 0.0; }
-        else {
-            s.t_now = v.t_now[i]; s.play_time = v.play_time[i]; s.started = v.started[i] != 0;
-            s.play_id = v.play_id[i]; s.play_len = v.play_len[i];
-        }
-        s.speed = o.speed ? o.speed + i : nullptr;   // [V][N] table: the speed of content chunk k is speed[k][i]
-        s.speed_stride = (size_t)n; s.V = v.V; s.bad_speed = false;
-    }
+    if (LIVE) load_live(v, s, i, o.speed, fresh);
     // SPEC §4 action of step t; must be called with increasing t.  FIXED clamps t to the last row so that the
     // calls that run ahead of the final step stay inside the caller's table.
     auto action_at = [&](const int t) -> int {
@@ -1208,31 +1259,10 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             // tail of step t
             ABR_CHECK((unsigned long long)ix < (unsigned long long)steps * n, "trajectory element index");
             const bool moved = step_tail<SMEM, FAST, false>(pl, Vr, s, h, q0, lk0, g, r, hist, inv_q);
-            if (NOOUT) {
-            } else if (FAST) {
-                __stcs(o.delay + ix, (OT)r.delay); __stcs(o.sleep + ix, (OT)r.sleep); __stcs(o.buffer + ix, (OT)r.buffer);
-                __stcs(o.rebuf + ix, (OT)r.rebuf); __stcs(o.reward + ix, (OT)r.reward);
-                o.eov[ix] = r.eov ? 1 : 0;
-            } else {
-                if (o.delay) __stcs(o.delay + ix, (OT)r.delay);
-                if (o.sleep) __stcs(o.sleep + ix, (OT)r.sleep);
-                if (o.buffer) __stcs(o.buffer + ix, (OT)r.buffer);
-                if (o.rebuf) __stcs(o.rebuf + ix, (OT)r.rebuf);
-                if (o.reward) __stcs(o.reward + ix, (OT)r.reward);
-                if (o.eov) o.eov[ix] = r.eov ? 1 : 0;
-                if (o.actions) __stcs(o.actions + ix, q0);
-            }
-            if (FAST || !r.inert) {
-                a_rew = dadd(a_rew, r.reward); a_reb = dadd(a_reb, r.rebuf); a_u = dadd(a_u, r.u);
-                a_sm = dadd(a_sm, r.smooth); a_sl = dadd(a_sl, r.sleep); a_dl = dadd(a_dl, r.delay);
-                if (!FAST) {     // FAST: every step counts and every V-th ends an episode (closed form below)
-                    n_steps += 1;
-                    n_eps += r.eov ? 1 : 0;
-                }
-                if (FAST) {}                         // closed form below
-                else if (r.reset_mpc) reset_mpc = true;   // an auto-reset also clears the robust-MPC predictor state
-                else if (hist) v.bw_hist[(size_t)((s.hist_len - 1) % v.K) * v.cap + i] = r.thr;
-            }
+            store_step<FAST, NOOUT, false>(o.traj, ix, r);
+            if (!FAST && o.traj.actions) __stcs(o.traj.actions + ix, q0);
+            // FAST: every step counts and every V-th ends an episode (closed form below)
+            if (FAST || !r.inert) add_step<false, !FAST>(sum, r, v, s, i, hist);
             calm = !__any_sync(lanes, moved);
             if (moved || !ok1) {   // s.pos: where step t left the session
                 const double raw = dadd(s.pos, lk1.size);
@@ -1253,52 +1283,25 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             ABR_CHECK((unsigned long long)ix < (unsigned long long)steps * n, "trajectory element index");
             step_core<SMEM, FAST, LIVE>(v, s, q, lk, r, hist);
             flagged |= r.walk_error;
-            if (NOOUT) {
-            } else if (FAST) {
-                __stcs(o.delay + ix, (OT)r.delay); __stcs(o.sleep + ix, (OT)r.sleep); __stcs(o.buffer + ix, (OT)r.buffer);
-                __stcs(o.rebuf + ix, (OT)r.rebuf); __stcs(o.reward + ix, (OT)r.reward);
-                o.eov[ix] = r.eov ? 1 : 0;
-            } else {
-                if (o.delay) __stcs(o.delay + ix, (OT)r.delay);
-                if (o.sleep) __stcs(o.sleep + ix, (OT)r.sleep);
-                if (o.buffer) __stcs(o.buffer + ix, (OT)r.buffer);
-                if (o.rebuf) __stcs(o.rebuf + ix, (OT)r.rebuf);
-                if (o.reward) __stcs(o.reward + ix, (OT)r.reward);
-                if (o.eov) o.eov[ix] = r.eov ? 1 : 0;
-                if (LIVE && o.latency) __stcs(o.latency + ix, (OT)r.latency);
-                if (o.actions) __stcs(o.actions + ix, q);
-            }
-            if (FAST || !r.inert) {
-                a_rew = dadd(a_rew, r.reward); a_reb = dadd(a_reb, r.rebuf); a_u = dadd(a_u, r.u);
-                a_sm = dadd(a_sm, r.smooth); a_sl = dadd(a_sl, r.sleep); a_dl = dadd(a_dl, r.delay);
-                if (LIVE) { a_su = dadd(a_su, r.startup); a_lat = dadd(a_lat, r.area); a_pl = dadd(a_pl, r.played); }
-                n_steps += 1;
-                n_eps += r.eov ? 1 : 0;
-                if (r.reset_mpc) reset_mpc = true;   // an auto-reset also clears the robust-MPC predictor state
-                else if (hist) v.bw_hist[(size_t)((s.hist_len - 1) % v.K) * v.cap + i] = r.thr;
-            }
+            store_step<FAST, NOOUT, LIVE>(o.traj, ix, r);
+            if (!FAST && o.traj.actions) __stcs(o.traj.actions + ix, q);
+            if (FAST || !r.inert) add_step<LIVE, true>(sum, r, v, s, i, hist);
             ix += n;
         }
     }
     if (FAST && AHEAD) {   // auto_reset is on: the session ran `steps` steps and wrapped every V chunks
-        n_steps = steps;
-        n_eps = (int)(((long long)chunk_in + steps) / v.V);
-        reset_mpc = n_eps > 0;
+        sum.steps = steps;
+        sum.eps = (int)(((long long)chunk_in + steps) / v.V);
+        sum.reset_mpc = sum.eps > 0;
     }
-    const double a_steps = (double)n_steps, a_eps = (double)n_eps;   // exact: counts below 2^31
     if (flagged || (LIVE && s.bad_speed)) atomicAdd(v.errors, 1ull);
-    v.seg[i] = s.seg; v.chunk[i] = s.chunk; v.last_q[i] = s.last_q; v.phi[i] = s.phi; v.pos[i] = s.pos;
-    v.buffer[i] = s.buffer;
-    if (LIVE) {
-        v.t_now[i] = s.t_now; v.play_time[i] = s.play_time; v.started[i] = s.started ? 1 : 0;
-        v.play_id[i] = s.play_id; v.play_len[i] = s.play_len;
-    }
+    store_state<LIVE>(v, s, i);
     if (hist) v.hist_len[i] = s.hist_len;
-    if (reset_mpc) { v.last_pred[i] = 0.0; v.err_len[i] = 0; }
+    if (sum.reset_mpc) { v.last_pred[i] = 0.0; v.err_len[i] = 0; }
     if (!FAST && s.done) v.done[i] = 1;
     if (fresh) {   // the rest of what abr_reset_kernel writes
         if (!hist) v.hist_len[i] = 0;
-        if (!reset_mpc) { v.last_pred[i] = 0.0; v.err_len[i] = 0; }
+        if (!sum.reset_mpc) { v.last_pred[i] = 0.0; v.err_len[i] = 0; }
         if (FAST || !s.done) v.done[i] = 0;
         if (!LIVE) {
             v.t_now[i] = 0.0; v.play_time[i] = 0.0; v.started[i] = v.p.start_up_length <= 0.0 ? 1 : 0;
@@ -1308,7 +1311,9 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     // accumulator read-modify-write: all loads first (one memory round trip instead of ten dependent ones)
     double* a = v.acc + i;
     const size_t c = v.cap;
-    const double add[ABR_NUM_ACC] = {a_rew, a_reb, a_u, a_sm, a_sl, a_dl, a_steps, a_eps, a_su, a_lat, a_pl};
+    const double add[ABR_NUM_ACC] = {sum.rew, sum.reb, sum.u, sum.sm, sum.sl, sum.dl,
+                                     (double)sum.steps, (double)sum.eps,   // exact: counts below 2^31
+                                     sum.su, sum.lat, sum.pl};
     double old[ABR_NUM_ACC];
 #pragma unroll
     for (int j = 0; j < ABR_NUM_ACC; ++j) old[j] = fresh ? 0.0 : __ldcg(a + j * c);
@@ -1539,17 +1544,15 @@ static cudaError_t allow_smem(Kernel kernel, size_t bytes) {
 }
 
 template <typename OT>
-static cudaError_t launch_step_t(const EnvView& v, const int32_t* d_action, const double* d_speed, OT* d_delay,
-                                 OT* d_sleep, OT* d_buffer, OT* d_rebuf, OT* d_reward, OT* d_latency,
-                                 OT* d_next_sizes, uint8_t* d_eov, OT* d_thr, cudaStream_t st,
-                                 const StepPolicy* policy = nullptr) {
+cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, const StepOutputs<OT>& o,
+                        cudaStream_t st, const StepPolicy* policy) {
     if (v.n == 0) return cudaSuccess;
     const bool live = v.p.live != 0;
     const StepPolicy pol = policy ? *policy : StepPolicy{};
-    const bool fast = !policy && !live && d_delay && d_sleep && d_buffer && d_rebuf && d_reward && d_eov &&
-                      v.p.track_history == 0 && v.p.track_acc == 0 && v.p.auto_reset != 0;
-    // persistent-style grid: one wave of 3 blocks per SM, each walking an equal run of consecutive tiles (at least
-    // kStepTiles, so that small batches still amortise the staging); no tail wave
+    const bool fast = !policy && !live && o.has_core() && v.p.track_history == 0 && v.p.track_acc == 0 &&
+                      v.p.auto_reset != 0;
+    // persistent-style grid: one wave of kTileBlocksPerSM blocks per SM, each walking an equal run of consecutive
+    // tiles (at least kStepTiles, so that small batches still amortise the staging); no tail wave
     static int sm_count = 0;
     if (sm_count == 0) {
         int dev = 0;
@@ -1564,45 +1567,40 @@ static cudaError_t launch_step_t(const EnvView& v, const int32_t* d_action, cons
     int smem_doubles = cum_smem_doubles(v.T_max);
     size_t smem_bytes = (size_t)smem_doubles * sizeof(double) + (size_t)idx_stride(v.T_max) * sizeof(uint16_t);
     if (smem_bytes > kSmemOptInLimit || idx_stride(v.T_max) == 0) { smem_doubles = 0; smem_bytes = 0; }
-    cudaError_t e = cudaSuccess;
-#define ABR_STEP_ARGS v, d_action, d_speed, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_latency, d_next_sizes, d_eov, d_thr, smem_doubles, tiles_per_block, pol
-#define ABR_LAUNCH_STEP(F, L, P)                                                               \
-    do {                                                                                       \
-        e = allow_smem(abr_step_kernel<F, L, P, OT>, smem_bytes);                              \
-        if (e == cudaSuccess) abr_step_kernel<F, L, P, OT><<<grid, kTile, smem_bytes, st>>>(ABR_STEP_ARGS); \
-    } while (0)
+    auto go = [&](auto kernel) {
+        cudaError_t e = allow_smem(kernel, smem_bytes);
+        if (e == cudaSuccess)
+            kernel<<<grid, kTile, smem_bytes, st>>>(v, d_action, d_speed, o.delay, o.sleep, o.buffer, o.rebuf, o.reward,
+                                                    o.latency, o.next_sizes, o.eov, o.thr, smem_doubles, tiles_per_block, pol);
+        return e;
+    };
+    cudaError_t e;
     if (policy) {
-        if constexpr (std::is_same<OT, double>::value) ABR_LAUNCH_STEP(false, false, true);
+        if constexpr (std::is_same<OT, double>::value) e = go(abr_step_kernel<false, false, true, OT>);
         else return cudaErrorInvalidValue;
     }
-    else if (live) ABR_LAUNCH_STEP(false, true, false);
-    else if (fast) ABR_LAUNCH_STEP(true, false, false);
-    else ABR_LAUNCH_STEP(false, false, false);
-#undef ABR_LAUNCH_STEP
-#undef ABR_STEP_ARGS
+    else if (live) e = go(abr_step_kernel<false, true, false, OT>);
+    else if (fast) e = go(abr_step_kernel<true, false, false, OT>);
+    else e = go(abr_step_kernel<false, false, false, OT>);
     if (e != cudaSuccess) return e;
     count_launch();
     return cudaGetLastError();
 }
 
-cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, double* d_delay,
-                        double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward, double* d_latency,
-                        double* d_next_sizes, uint8_t* d_eov, double* d_thr, cudaStream_t st) {
-    return launch_step_t<double>(v, d_action, d_speed, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_latency,
-                                 d_next_sizes, d_eov, d_thr, st);
-}
+template cudaError_t launch_step<double>(const EnvView&, const int32_t*, const double*, const StepOutputs<double>&,
+                                         cudaStream_t, const StepPolicy*);
+template cudaError_t launch_step<float>(const EnvView&, const int32_t*, const double*, const StepOutputs<float>&,
+                                        cudaStream_t, const StepPolicy*);
 
 __global__ void abr_bump_kernel(uint32_t* counter) { *counter += 1u; }
 
 // SPEC §4.1: the step with the action drawn from the caller's logits and the observation written by the same kernel;
 // the draw counter is advanced behind it (same stream: every thread has read it by then), so that a captured graph
 // replays with a new draw every time.
-cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, double* d_delay, double* d_sleep, double* d_buffer,
-                               double* d_rebuf, double* d_reward, uint8_t* d_eov, uint32_t* d_draw_counter,
-                               cudaStream_t st) {
+cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const StepOutputs<double>& o,
+                               uint32_t* d_draw_counter, cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;
-    cudaError_t e = launch_step_t<double>(v, nullptr, nullptr, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, nullptr,
-                                          nullptr, d_eov, nullptr, st, &pol);
+    cudaError_t e = launch_step<double>(v, nullptr, nullptr, o, st, &pol);
     if (e != cudaSuccess) return e;
     if (pol.draw) {
         abr_bump_kernel<<<1, 1, 0, st>>>(d_draw_counter);
@@ -1611,25 +1609,31 @@ cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, double* 
     return cudaGetLastError();
 }
 
-// fp32-output mode: same fp64 arithmetic, every floating-point output rounded once to float on the store
-cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, float* d_delay,
-                        float* d_sleep, float* d_buffer, float* d_rebuf, float* d_reward, float* d_latency,
-                        float* d_next_sizes, uint8_t* d_eov, float* d_thr, cudaStream_t st) {
-    return launch_step_t<float>(v, d_action, d_speed, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_latency,
-                                d_next_sizes, d_eov, d_thr, st);
+// The episode kernel's compile-time form for policy P, launched by go(kernel, outputs).  The carried-utility form
+// (UNI) only exists where it pays: the run-ahead loop (not the buffer-based policy).  NOOUT stores no trajectory, so
+// its output type is never used: the double form serves the fp32 calls too.
+template <int P, typename OT, typename Go>
+static cudaError_t launch_rollout_form(const Go& go, const RolloutOut<OT>& o, const RolloutOut<double>& o_none,
+                                       const bool live, const bool fast, const bool none, const bool uni) {
+    constexpr bool kAhead = P != ABR_POLICY_BBA;
+    if (live) return go(abr_rollout_kernel<P, false, false, true, false, OT>, o);
+    if (fast && uni) return go(abr_rollout_kernel<P, true, false, false, kAhead, OT>, o);
+    if (fast) return go(abr_rollout_kernel<P, true, false, false, false, OT>, o);
+    if (none && uni) return go(abr_rollout_kernel<P, true, true, false, kAhead, double>, o_none);
+    if (none) return go(abr_rollout_kernel<P, true, true, false, false, double>, o_none);
+    return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);
 }
 
 template <typename OT>
-static cudaError_t launch_rollout_t(const EnvView& v, int policy, uint64_t seed, int steps,
-                                    const int32_t* d_actions_in, const double* d_speed, OT* d_delay, OT* d_sleep,
-                                    OT* d_buffer, OT* d_rebuf, OT* d_reward, OT* d_latency, uint8_t* d_eov,
-                                    int32_t* d_actions_out, double* d_block_partials, const RolloutFused& f,
-                                    uint32_t step_base, cudaStream_t st) {
+cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, uint32_t step_base,
+                           const int32_t* d_actions_in, const double* d_speed, const StepOutputs<OT>& out,
+                           double* d_block_partials, const RolloutFused& f, cudaStream_t st) {
     if (v.n == 0 || steps <= 0) return cudaSuccess;
     const dim3 grid((v.n + kRolloutBlock - 1) / kRolloutBlock), block(kRolloutBlock);
     const uint32_t lo = (uint32_t)seed, hi = (uint32_t)(seed >> 32);
-    RolloutOut<OT> o{d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_eov, d_actions_out, d_latency, d_speed,
-                     f.in_trace_id, f.in_offset, f.out_cost, d_block_partials ? f.out_stats : nullptr, f.scratch};
+    double* out_stats = d_block_partials ? f.out_stats : nullptr;
+    const RolloutOut<OT> o{out, d_speed, f.in_trace_id, f.in_offset, f.out_cost, out_stats, f.scratch};
+    const RolloutOut<double> o_none{StepOutputs<double>{}, d_speed, f.in_trace_id, f.in_offset, f.out_cost, out_stats, f.scratch};
     const bool live = v.p.live != 0;
     // shared-memory buffer: the longest C row, the longest index row and the two tables
     int smem_doubles = cum_smem_doubles(v.T_max);
@@ -1638,58 +1642,32 @@ static cudaError_t launch_rollout_t(const EnvView& v, int policy, uint64_t seed,
     // <= 31 KB keeps 7 blocks per SM resident (the 65 536-session shape is then one wave); longer traces opt in to
     // more shared memory and run with fewer blocks per SM, which still beats scattered global probes
     if (smem_bytes > kSmemOptInLimit || idx_stride(v.T_max) == 0) { smem_doubles = 0; smem_bytes = 0; }
-    const bool fast = !live && d_delay && d_sleep && d_buffer && d_rebuf && d_reward && d_eov && !d_actions_out &&
-                      v.p.track_history == 0 && v.p.auto_reset != 0;
-    const bool none = !live && !d_delay && !d_sleep && !d_buffer && !d_rebuf && !d_reward && !d_eov && !d_actions_out &&
-                      v.p.track_history == 0 && v.p.auto_reset != 0;
-    cudaError_t e = cudaSuccess;
-#define ABR_LAUNCH_ROLLOUT_V(P, F, N, L, U)                                                                        \
-    do {                                                                                                           \
-        e = allow_smem(abr_rollout_kernel<P, F, N, L, U, OT>, smem_bytes);                                         \
-        if (e == cudaSuccess)                                                                                      \
-            abr_rollout_kernel<P, F, N, L, U, OT><<<grid, block, smem_bytes, st>>>(v, lo, hi, steps, step_base,     \
-                                                                                   d_actions_in, o, smem_doubles,  \
-                                                                                   d_block_partials);              \
-    } while (0)
-    // the carried-utility form only exists where it pays: the run-ahead loop (not the buffer-based policy)
-#define ABR_LAUNCH_ROLLOUT(P)                                                                                      \
-    do {                                                                                                           \
-        constexpr bool kAhead = P != ABR_POLICY_BBA;                                                               \
-        if (live) ABR_LAUNCH_ROLLOUT_V(P, false, false, true, false);                                              \
-        else if (fast && kAhead && v.uniform_util) ABR_LAUNCH_ROLLOUT_V(P, true, false, false, kAhead);            \
-        else if (fast) ABR_LAUNCH_ROLLOUT_V(P, true, false, false, false);                                         \
-        else if (none && kAhead && v.uniform_util) ABR_LAUNCH_ROLLOUT_V(P, true, true, false, kAhead);             \
-        else if (none) ABR_LAUNCH_ROLLOUT_V(P, true, true, false, false);                                          \
-        else ABR_LAUNCH_ROLLOUT_V(P, false, false, false, false);                                                  \
-    } while (0)
+    const bool plain = !live && v.p.track_history == 0 && v.p.auto_reset != 0;
+    const bool fast = plain && out.has_core() && !out.actions;
+    const bool none = plain && out.none();
+    const bool uni = v.uniform_util != 0;
+    auto go = [&](auto kernel, const auto& o_k) {
+        cudaError_t e = allow_smem(kernel, smem_bytes);
+        if (e == cudaSuccess)
+            kernel<<<grid, block, smem_bytes, st>>>(v, lo, hi, steps, step_base, d_actions_in, o_k, smem_doubles, d_block_partials);
+        return e;
+    };
+    cudaError_t e;
     switch (policy) {
-        case ABR_POLICY_FIXED: ABR_LAUNCH_ROLLOUT(ABR_POLICY_FIXED); break;
-        case ABR_POLICY_RANDOM: ABR_LAUNCH_ROLLOUT(ABR_POLICY_RANDOM); break;
-        case ABR_POLICY_BBA: ABR_LAUNCH_ROLLOUT(ABR_POLICY_BBA); break;
+        case ABR_POLICY_FIXED: e = launch_rollout_form<ABR_POLICY_FIXED>(go, o, o_none, live, fast, none, uni); break;
+        case ABR_POLICY_RANDOM: e = launch_rollout_form<ABR_POLICY_RANDOM>(go, o, o_none, live, fast, none, uni); break;
+        case ABR_POLICY_BBA: e = launch_rollout_form<ABR_POLICY_BBA>(go, o, o_none, live, fast, none, uni); break;
         default: return cudaErrorInvalidValue;
     }
-#undef ABR_LAUNCH_ROLLOUT
-#undef ABR_LAUNCH_ROLLOUT_V
     if (e != cudaSuccess) return e;
     count_launch();
     return cudaGetLastError();
 }
 
-cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, const int32_t* d_actions_in,
-                           const double* d_speed, double* d_delay, double* d_sleep, double* d_buffer, double* d_rebuf,
-                           double* d_reward, double* d_latency, uint8_t* d_eov, int32_t* d_actions_out,
-                           double* d_block_partials, cudaStream_t st, const RolloutFused& f, uint32_t step_base) {
-    return launch_rollout_t<double>(v, policy, seed, steps, d_actions_in, d_speed, d_delay, d_sleep, d_buffer, d_rebuf,
-                                    d_reward, d_latency, d_eov, d_actions_out, d_block_partials, f, step_base, st);
-}
-
-cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, const int32_t* d_actions_in,
-                           const double* d_speed, float* d_delay, float* d_sleep, float* d_buffer, float* d_rebuf,
-                           float* d_reward, float* d_latency, uint8_t* d_eov, int32_t* d_actions_out,
-                           double* d_block_partials, cudaStream_t st, uint32_t step_base) {
-    return launch_rollout_t<float>(v, policy, seed, steps, d_actions_in, d_speed, d_delay, d_sleep, d_buffer, d_rebuf,
-                                   d_reward, d_latency, d_eov, d_actions_out, d_block_partials, RolloutFused{}, step_base, st);
-}
+template cudaError_t launch_rollout<double>(const EnvView&, int, uint64_t, int, uint32_t, const int32_t*, const double*,
+                                            const StepOutputs<double>&, double*, const RolloutFused&, cudaStream_t);
+template cudaError_t launch_rollout<float>(const EnvView&, int, uint64_t, int, uint32_t, const int32_t*, const double*,
+                                           const StepOutputs<float>&, double*, const RolloutFused&, cudaStream_t);
 
 int stats_num_partials(int n) { return n <= 0 ? 1 : (n + kStatsSessionsPerBlock - 1) / kStatsSessionsPerBlock; }
 
