@@ -12,7 +12,7 @@ from . import _build
 
 NUM_ACC = 11
 NUM_STATS = 11
-POLICY_FIXED, POLICY_RANDOM, POLICY_BBA = 0, 1, 2
+POLICY_FIXED, POLICY_RANDOM, POLICY_BBA, POLICY_RATE, POLICY_BOLA = 0, 1, 2, 3, 4
 MPC_REF, MPC_ROBUST = 0, 1
 MPC_TRUNCATE, MPC_EMPTY_DEFAULT, MPC_PRED_SES, MPC_EXHAUSTIVE = 1, 2, 4, 8
 MPC_MODE_EXHAUSTIVE = 0x100
@@ -41,6 +41,11 @@ class AbrParams(C.Structure):
                                  "track_history", "track_acc", "live", "smooth_prev_ladder")]
 
 
+class AbrPolicyParams(C.Structure):
+    """Parameters of the RATE and BOLA policies (SPEC §4.2, §4.3)."""
+    _fields_ = [(n, C.c_double) for n in ("rb_safety", "bola_min_buffer", "bola_target_buffer")]
+
+
 class AbrObsSpec(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
 
@@ -50,7 +55,7 @@ SYMBOLS = ("abr_version", "abr_last_error", "abr_launch_count", "abr_device_info
            "abr_env_create", "abr_env_destroy", "abr_env_num_sessions", "abr_sort_by_trace", "abr_env_set_order", "abr_env_reset", "abr_env_reset_sorted", "abr_env_get_order", "abr_env_reset_host",
            "abr_env_step", "abr_env_step_live", "abr_env_step_f32", "abr_env_step_policy", "abr_env_qoe_cost", "abr_env_rollout_fused",
            "abr_env_rollout_fused_live", "abr_env_rollout_fused_f32", "abr_env_run", "abr_env_mpc_decide", "abr_stats_partial",
-           "abr_env_state_ptr",
+           "abr_env_state_ptr", "abr_policy_params_default", "abr_env_set_policy_params", "abr_env_policy_decide",
            "abr_env_error_count", "abr_env_run_host", "abr_mpc_decide", "abr_mpc_decide_host", "abr_mpc_decide_startup",
            "abr_mpc_decide_startup_host", "abr_mpc_score_host",
            "abr_fp64_probe")

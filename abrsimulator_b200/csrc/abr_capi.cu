@@ -59,6 +59,7 @@ struct AbrEnv {
     size_t d_actions_cap = 0;
     double* d_reward_traj = nullptr;
     size_t d_reward_cap = 0;
+    double bola_vmax = 0.0;   // max over the log table of SPEC §4.3 (when every size is > 0, i.e. v.pol.bola_v is set)
 
     ~AbrEnv() {
         for (void* p : allocs) cudaFree(p);
@@ -133,6 +134,29 @@ static void utility_table(const double* bitrates, int V, int A, const AbrParams*
         }
 }
 
+void abr_policy_params_default(AbrPolicyParams* p) {
+    if (!p) return;
+    p->rb_safety = 1.0; p->bola_min_buffer = 10.0; p->bola_target_buffer = 30.0;
+}
+
+static int check_policy_params(const AbrPolicyParams* pp) {
+    if (!pp) return fail(ABR_ERR_INVALID, "policy params is NULL");
+    if (!(pp->rb_safety > 0.0) || !std::isfinite(pp->rb_safety)) return fail(ABR_ERR_INVALID, "rb_safety must be finite and > 0");
+    if (!(pp->bola_min_buffer > 0.0) || !std::isfinite(pp->bola_min_buffer) || !std::isfinite(pp->bola_target_buffer) ||
+        !(pp->bola_min_buffer < pp->bola_target_buffer))
+        return fail(ABR_ERR_INVALID, "need 0 < bola_min_buffer < bola_target_buffer, both finite");
+    return ABR_OK;
+}
+
+// SPEC §4.2 / §4.3 parameters (already validated): BOLA's (Vp, gp) derived from the buffer range as dash.js does
+static void install_policy_params(AbrEnv* env, const AbrPolicyParams* pp) {
+    EnvView::Policy& pol = env->v.pol;
+    pol.rb_safety = pp->rb_safety;
+    pol.bola_vmax = env->bola_vmax;
+    pol.bola_gp = env->bola_vmax / (pp->bola_target_buffer / pp->bola_min_buffer - 1.0);
+    pol.bola_Vp = pp->bola_min_buffer / pol.bola_gp;
+}
+
 static int check_tables(const double* sizes, const double* bitrates, int V, int A) {
     if (!sizes || !bitrates) return fail(ABR_ERR_INVALID, "sizes/bitrates is NULL");
     if (V < 1 || A < 1 || A > 16) return fail(ABR_ERR_RANGE, "need V >= 1 and 1 <= A <= 16 (got V=%d A=%d)", V, A);
@@ -203,6 +227,29 @@ int abr_env_create(const double* h_trace_bw, const int32_t* h_trace_len, const d
         CUDA_TRY(e->alloc(&d_tab, tab.size()));
         CUDA_TRY(cudaMemcpy(d_tab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice));
         v.tab = reinterpret_cast<const double2*>(d_tab);
+    }
+    {   // BOLA's utilities v[k][a] = log(sizes[k][a] / sizes[k][0]) (SPEC §4.3), with the C library's log like the
+        // utility table; only when every size is > 0 (else BOLA calls fail and the table is not needed)
+        bool positive = true;
+        for (size_t i = 0; i < (size_t)V * A && positive; ++i) positive = h_sizes[i] > 0.0;
+        if (positive) {
+            std::vector<double> lv((size_t)V * A);
+            double vmax = -INFINITY;
+            for (int k = 0; k < V; ++k)
+                for (int a = 0; a < A; ++a) {
+                    const double x = std::log(h_sizes[(size_t)k * A + a] / h_sizes[(size_t)k * A]);
+                    lv[(size_t)k * A + a] = x;
+                    if (x > vmax) vmax = x;
+                }
+            double* d_v;
+            CUDA_TRY(e->alloc(&d_v, lv.size()));
+            CUDA_TRY(cudaMemcpy(d_v, lv.data(), sizeof(double) * lv.size(), cudaMemcpyHostToDevice));
+            v.pol.bola_v = d_v;
+            e->bola_vmax = vmax;
+        }
+        AbrPolicyParams pp;
+        abr_policy_params_default(&pp);
+        install_policy_params(e, &pp);
     }
     // per-trace tables of SPEC §3.1 (cumulative capacity, search widths), built on the device
     // (+4 doubles of slack: the step reads C[j .. j+4] and discards what lies past its candidates)
@@ -311,6 +358,34 @@ static void begin_batch(AbrEnv* env, int n_sessions, long long session_base) {
     env->fresh_partials = 0;
     env->was_reset = true;
     env->step_base = 0;
+}
+
+// A built-in policy id the environment can run: RATE reads the history ring, BOLA the log table of positive sizes.
+static int check_policy(const AbrEnv* env, int policy) {
+    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BOLA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
+    if (policy == ABR_POLICY_RATE && !env->v.p.track_history)
+        return fail(ABR_ERR_STATE, "ABR_POLICY_RATE needs the throughput history: create the environment with track_history = 1");
+    if (policy == ABR_POLICY_BOLA && !env->v.pol.bola_v) return fail(ABR_ERR_INVALID, "BOLA needs positive chunk sizes");
+    return ABR_OK;
+}
+
+int abr_env_set_policy_params(AbrEnv* env, const AbrPolicyParams* params) {
+    if (int rc = check_policy_params(params)) return rc;   // host-side only: bad values are reported without a device
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    install_policy_params(env, params);
+    return ABR_OK;
+}
+
+int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stream) {
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (policy != ABR_POLICY_BBA && policy != ABR_POLICY_RATE && policy != ABR_POLICY_BOLA)
+        return fail(ABR_ERR_INVALID, "abr_env_policy_decide takes ABR_POLICY_BBA, _RATE or _BOLA (got %d)", policy);
+    if (int rc = check_policy(env, policy)) return rc;
+    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+    if (env->v.n == 0) return ABR_OK;
+    if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
+    CUDA_TRY(launch_policy_decide(env->v, policy, d_action, (cudaStream_t)stream));
+    return ABR_OK;
 }
 
 int abr_env_set_order(AbrEnv* env, const int32_t* d_perm, int n_sessions, void* stream) {
@@ -468,7 +543,7 @@ static int env_rollout_any(AbrEnv* env, int policy, uint64_t seed, int steps, co
     if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
     if (env->v.n == 0) return ABR_OK;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
-    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BBA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
+    if (int rc_p = check_policy(env, policy)) return rc_p;
     if (policy == ABR_POLICY_FIXED && !d_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
     if (!env->v.p.live && (d_speed || d_latency))
         return fail(ABR_ERR_STATE, "speed / latency belong to live mode (SPEC 7): create the environment with live = 1");
@@ -604,7 +679,7 @@ int abr_env_run(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t
     int rc = check_capacity(env, n_sessions);
     if (rc) return rc;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
-    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BBA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
+    if (int rc_p = check_policy(env, policy)) return rc_p;
     if (policy == ABR_POLICY_FIXED && !d_actions_in && n_sessions > 0 && steps > 0)
         return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
     if ((rc = check_batch(env, n_sessions))) return rc;
@@ -647,7 +722,7 @@ int abr_env_run_host(AbrEnv* env, int policy, uint64_t seed, int steps, const in
     if (!h_trace_id && n_sessions > 0) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
     int rc = check_capacity(env, n_sessions);
     if (rc) return rc;
-    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BBA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
+    if (int rc_p = check_policy(env, policy)) return rc_p;
     if (policy == ABR_POLICY_FIXED && !h_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs h_actions_in");
     if ((rc = check_batch(env, n_sessions))) return rc;
     cudaStream_t st = (cudaStream_t)stream;

@@ -122,6 +122,12 @@ struct EnvView {
     int uniform_util;                           // every chunk has the same utility row (the usual case: one bitrate ladder)
     long long session_base;
     AbrParams p;
+    // RATE / BOLA policies (SPEC §4.2, §4.3), derived on the host from AbrPolicyParams; last, so that the fields
+    // above keep their kernel-parameter offsets
+    struct Policy {
+        const double* __restrict__ bola_v;      // [V][A] log(sizes[k][a] / sizes[k][0]); null when a size is not > 0
+        double rb_safety, bola_Vp, bola_gp, bola_vmax;
+    } pol;
 };
 
 // launchers implemented in abr_step.cu / abr_mpc.cu (C++ linkage, internal)
@@ -179,6 +185,8 @@ template <typename OT>
 cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, uint32_t step_base,
                            const int32_t* d_actions_in, const double* d_speed, const StepOutputs<OT>& o,
                            double* d_block_partials, const RolloutFused& f, cudaStream_t st);
+// abr_env_policy_decide: the action of policy BBA / RATE / BOLA for every session from the SoA state
+cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st);
 cudaError_t launch_stats(const EnvView& v, double* d_partials, int n_partials, bool have_partials, double* d_out,
                          const StatsScratch& scratch,
                          cudaStream_t st);

@@ -493,6 +493,44 @@ __device__ __forceinline__ int policy_bba(const EnvView& v, const double b) {
     return q > A - 1 ? A - 1 : q;
 }
 
+// SPEC §4.2, rate-based policy: the highest quality whose size fits rb_safety * (harmonic mean of the last
+// min(hist_len, K) throughput samples) * L.  Session i's ring is column i of bw_hist[K][cap], newest sample at slot
+// (hist_len - 1) mod K; it is read with plain loads (the fused episode writes it as it goes).  size_at(a): the size of
+// quality a of the session's current chunk.
+template <typename SizeAt>
+__device__ __forceinline__ int policy_rate(const EnvView& v, const int i, const int hist_len, const SizeAt& size_at) {
+    const int A = v.A, K = v.K;
+    const int n = hist_len < K ? hist_len : K;
+    if (n == 0) {
+        const int d = v.p.default_quality;
+        return d < 0 ? 0 : (d > A - 1 ? A - 1 : d);
+    }
+    double S = 0.0;
+    for (int j = 0; j < n; ++j) {   // oldest first
+        const int slot = (hist_len - n + j) % K;
+        S = dadd(S, ddiv(1.0, v.bw_hist[(size_t)slot * v.cap + i]));
+    }
+    const double budget = dmul(dmul(v.pol.rb_safety, ddiv((double)n, S)), v.p.chunk_length);
+    int q = 0;
+    for (int a = 0; a < A; ++a)
+        if (size_at(a) <= budget) q = a;   // a NaN budget fits nothing
+    return q;
+}
+
+// SPEC §4.3, BOLA: the first quality of the largest score (Vp * (v[chunk][a] + gp) - buffer) / size[chunk][a] on the
+// pre-step buffer b; v is the host-built log table (bola_v, read-only path).  row: first element of the chunk's row.
+template <typename SizeAt>
+__device__ __forceinline__ int policy_bola(const EnvView& v, const double b, const int row, const SizeAt& size_at) {
+    if (v.pol.bola_vmax <= 0.0) return 0;   // every ladder flat
+    int q = 0;
+    double best = 0.0;
+    for (int a = 0; a < v.A; ++a) {
+        const double sc = ddiv(dsub(dmul(v.pol.bola_Vp, dadd(__ldg(v.pol.bola_v + row + a), v.pol.bola_gp)), b), size_at(a));
+        if (a == 0 || sc > best) { best = sc; q = a; }
+    }
+    return q;
+}
+
 // The per-session words of a step that come straight from the SoA state (coalesced: thread i <-> session i).
 struct RawState { int tr, seg, chunk, last_q; double phi, pos, buffer; };
 
@@ -1168,7 +1206,7 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
                                                 const uint32_t seed_hi, const int steps, const uint32_t step_base,
                                                 const int32_t* __restrict__ actions_in, const RolloutOut<OT>& o,
                                                 double (&acc_new)[ABR_NUM_ACC], const bool fresh) {
-    constexpr bool AHEAD = POLICY != ABR_POLICY_BBA && !LIVE;
+    constexpr bool AHEAD = (POLICY == ABR_POLICY_FIXED || POLICY == ABR_POLICY_RANDOM) && !LIVE;
     // the random policy is keyed by the caller's session index, whatever order the environment keeps the sessions in
     const unsigned long long gsession = (unsigned long long)(v.session_base + (v.perm ? __ldg(v.perm + i) : i));
     EpisodeSums sum;
@@ -1202,6 +1240,17 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
                 packed = two(r.x) | (two(r.y) << 8) | (two(r.z) << 16) | (two(r.w) << 24);
             }
             return (int)((packed >> (4 * (tg & 7u))) & 0xfu);
+        }
+        if (POLICY == ABR_POLICY_RATE || POLICY == ABR_POLICY_BOLA) {
+            if (!FAST && s.done) return 0;   // chunk == V: no sizes row (the step is inert)
+            const int row = s.chunk * v.A;
+            ABR_CHECK(s.chunk >= 0 && s.chunk < v.V, "policy row");
+            // the chunk's sizes from the staged {size, utility} table or the global one
+            auto size_at = [&](const int a) -> double {
+                return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
+            };
+            if (POLICY == ABR_POLICY_RATE) return policy_rate(v, i, s.hist_len, size_at);
+            return policy_bola(v, s.buffer, row, size_at);
         }
         return policy_bba(v, s.buffer);
     };
@@ -1516,7 +1565,43 @@ abr_qoe_cost_kernel(EnvView v, double* __restrict__ out) {
                           v.acc[ABR_ACC_STARTUP * c + i], v.acc[ABR_ACC_LATENCY * c + i]);
 }
 
+// abr_env_policy_decide: one thread per session, the same policy functions as the fused episode's action_at, on the
+// state the next step starts from (in live mode the buffer before the pause gate, as in the episode).
+template <int POLICY>
+__global__ void __launch_bounds__(kStepBlock)
+abr_policy_decide_kernel(EnvView v, int32_t* __restrict__ action) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= v.n) return;
+    const double b = v.buffer[i];
+    int q;
+    if (POLICY == ABR_POLICY_BBA) {
+        q = policy_bba(v, b);
+    } else if (!v.p.auto_reset && v.done[i]) {
+        q = 0;   // chunk == V: no sizes row
+    } else {
+        const int chunk = v.chunk[i];
+        ABR_CHECK(chunk >= 0 && chunk < v.V, "policy row");
+        const int row = chunk * v.A;
+        auto size_at = [&](const int a) -> double { return __ldg(v.sizes + row + a); };
+        q = POLICY == ABR_POLICY_RATE ? policy_rate(v, i, v.hist_len[i], size_at) : policy_bola(v, b, row, size_at);
+    }
+    action[i] = q;
+}
+
 }  // namespace
+
+cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st) {
+    if (v.n == 0) return cudaSuccess;
+    const unsigned grid = (v.n + kStepBlock - 1) / kStepBlock;
+    switch (policy) {
+        case ABR_POLICY_BBA: abr_policy_decide_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+        case ABR_POLICY_RATE: abr_policy_decide_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+        case ABR_POLICY_BOLA: abr_policy_decide_kernel<ABR_POLICY_BOLA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+        default: return cudaErrorInvalidValue;
+    }
+    count_launch();
+    return cudaGetLastError();
+}
 
 cudaError_t launch_trace_table(const EnvView& v, double* d_cum, uint16_t* d_idx, int32_t* d_ok, TraceMeta* d_meta,
                                cudaStream_t st) {
@@ -1615,13 +1700,18 @@ cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const St
 template <int P, typename OT, typename Go>
 static cudaError_t launch_rollout_form(const Go& go, const RolloutOut<OT>& o, const RolloutOut<double>& o_none,
                                        const bool live, const bool fast, const bool none, const bool uni) {
-    constexpr bool kAhead = P != ABR_POLICY_BBA;
+    constexpr bool kAhead = P == ABR_POLICY_FIXED || P == ABR_POLICY_RANDOM;
     if (live) return go(abr_rollout_kernel<P, false, false, true, false, OT>, o);
-    if (fast && uni) return go(abr_rollout_kernel<P, true, false, false, kAhead, OT>, o);
-    if (fast) return go(abr_rollout_kernel<P, true, false, false, false, OT>, o);
-    if (none && uni) return go(abr_rollout_kernel<P, true, true, false, kAhead, double>, o_none);
-    if (none) return go(abr_rollout_kernel<P, true, true, false, false, double>, o_none);
-    return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);
+    if constexpr (P == ABR_POLICY_RATE) {   // reads the history ring: track_history = 1, never a FAST / NOOUT form
+        if (fast || none) return cudaErrorInvalidValue;
+        return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);
+    } else {
+        if (fast && uni) return go(abr_rollout_kernel<P, true, false, false, kAhead, OT>, o);
+        if (fast) return go(abr_rollout_kernel<P, true, false, false, false, OT>, o);
+        if (none && uni) return go(abr_rollout_kernel<P, true, true, false, kAhead, double>, o_none);
+        if (none) return go(abr_rollout_kernel<P, true, true, false, false, double>, o_none);
+        return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);
+    }
 }
 
 template <typename OT>
@@ -1657,6 +1747,8 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
         case ABR_POLICY_FIXED: e = launch_rollout_form<ABR_POLICY_FIXED>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_RANDOM: e = launch_rollout_form<ABR_POLICY_RANDOM>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_BBA: e = launch_rollout_form<ABR_POLICY_BBA>(go, o, o_none, live, fast, none, uni); break;
+        case ABR_POLICY_RATE: e = launch_rollout_form<ABR_POLICY_RATE>(go, o, o_none, live, fast, none, uni); break;
+        case ABR_POLICY_BOLA: e = launch_rollout_form<ABR_POLICY_BOLA>(go, o, o_none, live, fast, none, uni); break;
         default: return cudaErrorInvalidValue;
     }
     if (e != cudaSuccess) return e;

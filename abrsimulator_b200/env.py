@@ -15,14 +15,15 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (AbrError, MPC_REF, MPC_ROBUST, NUM_ACC, NUM_STATS, POLICY_BBA, POLICY_FIXED,  # noqa: F401
-                   POLICY_RANDOM)
+from ._lib import (AbrError, MPC_REF, MPC_ROBUST, NUM_ACC, NUM_STATS, POLICY_BBA, POLICY_BOLA,  # noqa: F401
+                   POLICY_FIXED, POLICY_RANDOM, POLICY_RATE)
 from .datamodel import MPD, NetworkInfo, QOEMetric, pack_traces
 
 StepResult = namedtuple("StepResult", "delay sleep buffer rebuffer reward next_sizes end_of_video throughput latency",
                         defaults=(None,))
 
-_POLICIES = {"fixed": POLICY_FIXED, "random": POLICY_RANDOM, "bba": POLICY_BBA, "buffer": POLICY_BBA}
+_POLICIES = {"fixed": POLICY_FIXED, "random": POLICY_RANDOM, "bba": POLICY_BBA, "buffer": POLICY_BBA,
+             "rate": POLICY_RATE, "rb": POLICY_RATE, "bola": POLICY_BOLA}
 _MODES = {"reference": MPC_REF, "ref": MPC_REF, "robust": MPC_ROBUST}
 
 
@@ -450,6 +451,31 @@ class BatchedABREnv:
         self.n = n
         self.session_base = int(session_base)
         return out, qoe_cost, stats
+
+    # -- SPEC §4.2 / §4.3 --
+    def set_policy_params(self, rb_safety=None, bola_min_buffer=None, bola_target_buffer=None):
+        """Parameters of the "rate" and "bola" policies (SPEC §4.2, §4.3) for the following calls; arguments left at
+        None keep their current value (defaults: 1.0, 10 s, 30 s).  Invalid values raise before anything changes."""
+        cur = getattr(self, "_policy_params", None)
+        if cur is None:
+            cur = _lib.AbrPolicyParams()
+            self._lib.abr_policy_params_default(C.byref(cur))
+        pp = _lib.AbrPolicyParams(cur.rb_safety if rb_safety is None else float(rb_safety),
+                                  cur.bola_min_buffer if bola_min_buffer is None else float(bola_min_buffer),
+                                  cur.bola_target_buffer if bola_target_buffer is None else float(bola_target_buffer))
+        _lib.check(self._lib.abr_env_set_policy_params(self._h, C.byref(pp)))
+        self._policy_params = pp
+
+    def policy_decide(self, policy, out=None) -> torch.Tensor:
+        """The action of a state-dependent built-in policy ("bba", "rate" or "bola") for every session, from the
+        environment's own state (int32 [N] on the device); ``step`` with it is one step of the fused episode."""
+        pid = _policy_id(policy)
+        act = self._empty(self.n, dtype=torch.int32) if out is None else out
+        if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:
+            raise TypeError(f"out must be a contiguous int32 tensor of {self.n} elements on {self.device}")
+        with self._on:
+            _lib.check(self._lib.abr_env_policy_decide(self._h, C.c_int(pid), _ptr(act), _stream()))
+        return act
 
     # -- SPEC §5 --
     def mpc_decide(self, horizon=5, mode="robust", want_score=False, out=None, exhaustive=False):

@@ -20,8 +20,9 @@ Controllers
 -----------
 * any object with ``get_next_bitrate(chunk_id, previous_bitrates, previous_bandwidths, buffer_level) -> int``
   (the protocol ``Simulator.run`` calls, ``Simulator.py:155``) is driven chunk by chunk through the step kernel;
-* the markers ``RandomPolicy(seed)`` / ``BufferBasedPolicy()`` / ``FixedPolicy(actions)`` and this package's
-  ``MPCBitrateController`` run fully on the device (fused episode kernel, or decide+step kernels for MPC).
+* the markers ``RandomPolicy(seed)`` / ``BufferBasedPolicy()`` / ``RateBasedPolicy()`` / ``BolaPolicy()`` /
+  ``FixedPolicy(actions)`` and this package's ``MPCBitrateController`` run fully on the device (fused episode kernel,
+  or decide+step kernels for MPC).
 """
 from __future__ import annotations
 
@@ -42,6 +43,20 @@ class RandomPolicy:
 class BufferBasedPolicy:
     def __init__(self, reservoir=5.0, cushion=10.0):
         self.reservoir, self.cushion = float(reservoir), float(cushion)
+
+
+class RateBasedPolicy:
+    """Rate-based bitrate choice (SPEC §4.2): the highest bitrate whose chunk fits ``safety`` times the harmonic mean of
+    the last ``hist_k`` throughputs times the chunk length."""
+    def __init__(self, safety=1.0):
+        self.safety = float(safety)
+
+
+class BolaPolicy:
+    """BOLA (SPEC §4.3): the Lyapunov buffer rule with its (V, gamma*p) derived from the buffer range
+    [min_buffer, target_buffer] in seconds."""
+    def __init__(self, min_buffer=10.0, target_buffer=30.0):
+        self.min_buffer, self.target_buffer = float(min_buffer), float(target_buffer)
 
 
 class FixedPolicy:
@@ -101,6 +116,27 @@ class Simulator:
                 q.startup_weight * start_up_time + getattr(q, "latency_weight", 0.0) * average_latency)
 
     # -- environment --
+    _MARKERS = (RandomPolicy, BufferBasedPolicy, RateBasedPolicy, BolaPolicy, FixedPolicy)
+
+    @staticmethod
+    def _marker_policy(ctrl):
+        """The fused-episode policy name of a built-in policy marker (None: buffer-based)."""
+        return ("random" if isinstance(ctrl, RandomPolicy) else "fixed" if isinstance(ctrl, FixedPolicy) else
+                "rate" if isinstance(ctrl, RateBasedPolicy) else "bola" if isinstance(ctrl, BolaPolicy) else "bba")
+
+    def _marker_env(self, ctrl, n_sessions, **extra):
+        """The environment of a built-in policy marker, with the marker's parameters installed."""
+        if isinstance(ctrl, BufferBasedPolicy):
+            extra.update(bba_reservoir=ctrl.reservoir, bba_cushion=ctrl.cushion)
+        if isinstance(ctrl, RateBasedPolicy):
+            extra.update(track_history=1)             # the rate-based rule reads the throughput history
+        env = self._make_env(n_sessions, **extra)
+        if isinstance(ctrl, RateBasedPolicy):
+            env.set_policy_params(rb_safety=ctrl.safety)
+        elif isinstance(ctrl, BolaPolicy):
+            env.set_policy_params(bola_min_buffer=ctrl.min_buffer, bola_target_buffer=ctrl.target_buffer)
+        return env
+
     def _make_env(self, n_sessions, **extra):
         if self.mpd is None or self.network_info is None or self.qoe_metric is None:
             raise RuntimeError("set_qoe_metric, set_network_info and set_mpd must be called before run()")
@@ -131,14 +167,10 @@ class Simulator:
         q = self.qoe_metric
         if self._live():
             return self._run_live(n_sessions, tid, start_offset, session_base)
-        if isinstance(ctrl, (RandomPolicy, BufferBasedPolicy, FixedPolicy)) or ctrl is None:
-            extra = {}
-            if isinstance(ctrl, BufferBasedPolicy):
-                extra = dict(bba_reservoir=ctrl.reservoir, bba_cushion=ctrl.cushion)
-            env = self._make_env(n_sessions, **extra)
-            policy = "random" if isinstance(ctrl, RandomPolicy) else "fixed" if isinstance(ctrl, FixedPolicy) else "bba"
-            out = env.run_host(policy, V, tid, start_offset, seed=getattr(ctrl, "seed", 0), session_base=session_base,
-                               actions=getattr(ctrl, "actions", None), want_qoe_cost=True)
+        if isinstance(ctrl, self._MARKERS) or ctrl is None:
+            env = self._marker_env(ctrl, n_sessions)
+            out = env.run_host(self._marker_policy(ctrl), V, tid, start_offset, seed=getattr(ctrl, "seed", 0),
+                               session_base=session_base, actions=getattr(ctrl, "actions", None), want_qoe_cost=True)
             acc = out["acc"]
             self.last_run = dict(zip(ACC_NAMES, acc))
             return out["qoe_cost"]          # rw*rebuffer + vw*smooth, computed on the device
@@ -167,16 +199,13 @@ class Simulator:
             for _ in range(V):
                 act = env.mpc_decide(ctrl.horizon, mode)
                 env.step(act, want_next_sizes=False, speed=speed)
-        elif isinstance(ctrl, (RandomPolicy, BufferBasedPolicy, FixedPolicy)) or ctrl is None:
+        elif isinstance(ctrl, self._MARKERS) or ctrl is None:
             # built-in policies: one fused live episode (abr_env_rollout_fused_live), speed table from the controller
-            if isinstance(ctrl, BufferBasedPolicy):
-                extra.update(bba_reservoir=ctrl.reservoir, bba_cushion=ctrl.cushion)
-            env = self._make_env(n_sessions, **extra)
+            env = self._marker_env(ctrl, n_sessions, **extra)
             env.reset(tid, start_offset, session_base)
             speed = self._speed_table(n_sessions, V)
-            policy = "random" if isinstance(ctrl, RandomPolicy) else "fixed" if isinstance(ctrl, FixedPolicy) else "bba"
-            env.rollout(policy, V, seed=getattr(ctrl, "seed", 0), actions=getattr(ctrl, "actions", None), speed=speed,
-                        want=())
+            env.rollout(self._marker_policy(ctrl), V, seed=getattr(ctrl, "seed", 0), actions=getattr(ctrl, "actions", None),
+                        speed=speed, want=())
         else:
             env = self._make_env(n_sessions, **extra)
             self._run_callback(env, n_sessions, tid, start_offset, session_base)

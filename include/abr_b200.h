@@ -31,8 +31,9 @@ extern "C" {
 
 enum { ABR_OK = 0, ABR_ERR_INVALID = 1, ABR_ERR_CUDA = 2, ABR_ERR_RANGE = 3, ABR_ERR_STATE = 4 };
 
-/* built-in policies of the fused episode (SPEC §4) */
-enum { ABR_POLICY_FIXED = 0, ABR_POLICY_RANDOM = 1, ABR_POLICY_BBA = 2 };
+/* built-in policies of the fused episode (SPEC §4): RATE is the rate-based rule (§4.2, needs track_history = 1),
+ * BOLA the Lyapunov buffer rule (§4.3, needs every chunk size > 0) */
+enum { ABR_POLICY_FIXED = 0, ABR_POLICY_RANDOM = 1, ABR_POLICY_BBA = 2, ABR_POLICY_RATE = 3, ABR_POLICY_BOLA = 4 };
 /* MPC modes (SPEC §5): 0 = reference-exact mpc.py, 1 = robust MPC */
 enum { ABR_MPC_REF = 0, ABR_MPC_ROBUST = 1 };
 /* abr_mpc_decide flags */
@@ -193,6 +194,19 @@ int abr_env_rollout_fused_f32(AbrEnv* env, int policy, uint64_t seed, int steps,
                               const double* d_speed, float* d_delay, float* d_sleep, float* d_buffer, float* d_rebuf,
                               float* d_reward, float* d_latency, uint8_t* d_end_of_video, int32_t* d_actions_out,
                               void* stream);
+/* Parameters of the RATE and BOLA policies (SPEC §4.2, §4.3), kept apart from AbrParams so that its layout stays put.
+ * rb_safety: the budget is rb_safety * harmonic mean * chunk_length [1.0].  bola_min_buffer / bola_target_buffer: the
+ * buffer below which BOLA picks the lowest quality and at which the highest quality's score reaches zero [10, 30 s];
+ * the paper's (V, gamma*p) are V = min / gp and gp = v_max / (target / min - 1). */
+typedef struct AbrPolicyParams { double rb_safety, bola_min_buffer, bola_target_buffer; } AbrPolicyParams;
+void abr_policy_params_default(AbrPolicyParams* p);
+/* Validates (rb_safety finite and > 0, 0 < bola_min_buffer < bola_target_buffer, both finite; ABR_ERR_INVALID
+ * otherwise, before any device work) and installs them for the following calls.  abr_env_create installs the defaults. */
+int abr_env_set_policy_params(AbrEnv* env, const AbrPolicyParams* params);
+/* The action of a built-in state-dependent policy (ABR_POLICY_BBA, _RATE or _BOLA) for every session, from the
+ * environment's own state: the per-step counterpart of the fused episode's policies, to be followed by abr_env_step,
+ * abr_env_step_live or abr_env_step_f32.  d_action[N] receives them.  FIXED, RANDOM and unknown ids: ABR_ERR_INVALID. */
+int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stream);
 /* MPC decision for every session from the env's own state and history ring (SPEC §5);
  * never flags errors (implies ABR_MPC_TRUNCATE | ABR_MPC_EMPTY_DEFAULT). */
 int abr_env_mpc_decide(AbrEnv* env, int horizon, int mode, int32_t* d_action, double* d_best_j /*nullable*/,
