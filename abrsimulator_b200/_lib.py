@@ -50,15 +50,53 @@ class AbrObsSpec(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
 
 
-# every symbol include/abr_b200.h declares (tests check that the .so exports all of them)
-SYMBOLS = ("abr_version", "abr_last_error", "abr_launch_count", "abr_device_info", "abr_params_default",
-           "abr_env_create", "abr_env_destroy", "abr_env_num_sessions", "abr_sort_by_trace", "abr_env_set_order", "abr_env_reset", "abr_env_reset_sorted", "abr_env_get_order", "abr_env_reset_host",
-           "abr_env_step", "abr_env_step_live", "abr_env_step_f32", "abr_env_step_policy", "abr_env_qoe_cost", "abr_env_rollout_fused",
-           "abr_env_rollout_fused_live", "abr_env_rollout_fused_f32", "abr_env_run", "abr_env_mpc_decide", "abr_stats_partial",
-           "abr_env_state_ptr", "abr_policy_params_default", "abr_env_set_policy_params", "abr_env_policy_decide",
-           "abr_env_error_count", "abr_env_run_host", "abr_mpc_decide", "abr_mpc_decide_host", "abr_mpc_decide_startup",
-           "abr_mpc_decide_startup_host", "abr_mpc_score_host",
-           "abr_fp64_probe")
+# The signature of every symbol include/abr_b200.h declares, in the header's order: (restype, argtypes).  Buffers,
+# streams and the AbrEnv handle are c_void_p; tests check the table against the header and the .so's exports.
+_P, _I, _LL, _U64, _D = C.c_void_p, C.c_int, C.c_longlong, C.c_uint64, C.c_double
+_PARAMS, _POLICY_PARAMS, _OBS_SPEC = C.POINTER(AbrParams), C.POINTER(AbrPolicyParams), C.POINTER(AbrObsSpec)
+_RUN = [_P, _I, _U64, _I, _P, _P, _I, _LL, _P]                   # env, policy, seed, steps, trace ids, offsets, N, base, actions
+_MPC = [_P, _P, _I, _I, _PARAMS, _I] + [_P] * 5 + [_I] + [_P] * 3 + [_I] * 3   # tables .. robust state, horizon, mode, flags
+_STARTUP = [_P, _I, _D]                                            # startup, n_ts, ts_step
+SIGNATURES = {
+    "abr_version": (_I, []),
+    "abr_last_error": (C.c_char_p, []),
+    "abr_launch_count": (_LL, []),
+    "abr_device_info": (_I, [_P] * 4),
+    "abr_params_default": (None, [_PARAMS]),
+    "abr_env_create": (_I, [_P, _P, _P, _I, _I, _P, _P, _I, _I, _PARAMS, _I, _P]),
+    "abr_env_destroy": (None, [_P]),
+    "abr_env_num_sessions": (_I, [_P]),
+    "abr_sort_by_trace": (_I, [_P, _I, _I, _P, _P]),
+    "abr_env_set_order": (_I, [_P, _P, _I, _P]),
+    "abr_env_reset": (_I, [_P, _P, _P, _I, _LL, _P]),
+    "abr_env_reset_sorted": (_I, [_P, _P, _P, _I, _LL, _P]),
+    "abr_env_get_order": (_I, [_P, _P, _I, _P]),
+    "abr_env_reset_host": (_I, [_P, _P, _P, _I, _LL, _P]),
+    "abr_env_step": (_I, [_P] * 11),
+    "abr_env_step_policy": (_I, [_P, _P, _I, _U64, _OBS_SPEC] + [_P] * 10),
+    "abr_env_step_live": (_I, [_P] * 13),
+    "abr_env_rollout_fused": (_I, [_P, _I, _U64, _I] + [_P] * 9),
+    "abr_env_rollout_fused_live": (_I, [_P, _I, _U64, _I] + [_P] * 11),
+    "abr_env_run": (_I, _RUN + [_P] * 10),
+    "abr_env_step_f32": (_I, [_P] * 13),
+    "abr_env_rollout_fused_f32": (_I, [_P, _I, _U64, _I] + [_P] * 11),
+    "abr_policy_params_default": (None, [_POLICY_PARAMS]),
+    "abr_env_set_policy_params": (_I, [_P, _POLICY_PARAMS]),
+    "abr_env_policy_decide": (_I, [_P, _I, _P, _P]),
+    "abr_env_mpc_decide": (_I, [_P, _I, _I, _P, _P, _P]),
+    "abr_env_qoe_cost": (_I, [_P, _P, _P]),
+    "abr_stats_partial": (_I, [_P, _P, _P]),
+    "abr_env_state_ptr": (_I, [_P, _I, _P]),
+    "abr_env_error_count": (_I, [_P, _P, _P]),
+    "abr_env_run_host": (_I, _RUN + [_P] * 5),
+    "abr_mpc_decide": (_I, _MPC + [_P] * 6),
+    "abr_mpc_decide_startup": (_I, _MPC + _STARTUP + [_P] * 7),
+    "abr_mpc_decide_startup_host": (_I, _MPC + _STARTUP + [_P] * 6),
+    "abr_mpc_decide_host": (_I, _MPC + [_P] * 5),
+    "abr_mpc_score_host": (_I, [_P, _P, _I, _I, _PARAMS, _I, _I, _D, _P, _I, _I, _I, _D, _P, _I, _P]),
+    "abr_fp64_probe": (_I, [_I, _I, _P, _P, _P]),
+}
+SYMBOLS = tuple(SIGNATURES)
 
 _lib = None
 
@@ -78,17 +116,18 @@ def load():
         # under a file lock: concurrent ranks build once, the rest wait and load the finished file
         _build.build_library()
     lib = C.CDLL(path)
-    lib.abr_last_error.restype = C.c_char_p
-    lib.abr_launch_count.restype = C.c_longlong
-    lib.abr_version.restype = C.c_int
-    # argtypes for the host-buffer entry point: plain Python ints / None convert without per-call ctypes objects
-    vp = C.c_void_p
-    lib.abr_env_run_host.argtypes = [vp, C.c_int, C.c_uint64, C.c_int, vp, vp, C.c_int, C.c_longlong, vp, vp, vp, vp, vp, vp]
-    lib.abr_env_run_host.restype = C.c_int
-    lib.abr_env_step_policy.argtypes = [vp, vp, C.c_int, C.c_uint64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
-    lib.abr_env_step_policy.restype = C.c_int
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
+
+
+def _addr(x):
+    """The address of a buffer for a c_void_p argument: None, a torch tensor or a numpy array."""
+    if x is None:
+        return None
+    return x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data
 
 
 def check(rc: int):
@@ -98,7 +137,7 @@ def check(rc: int):
 
 def default_params(**kw) -> AbrParams:
     p = AbrParams()
-    load().abr_params_default(C.byref(p))
+    load().abr_params_default(p)
     for k, v in kw.items():
         if not hasattr(p, k):
             raise TypeError(f"unknown ABR parameter {k!r}")

@@ -5,7 +5,6 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -36,6 +35,34 @@ static int fail(int code, const char* fmt, ...) {
                                            __FILE__, __LINE__);                                        \
     } while (0)
 
+// Grow-only device memory on the current device.  Growing (or moving to another device) first waits for the device,
+// since work already launched may still use the old block; it then allocates half again what was asked for.
+struct DeviceBuffer {
+    void* p = nullptr;
+    size_t bytes = 0;
+    int device = -1;
+    DeviceBuffer() = default;
+    DeviceBuffer(const DeviceBuffer&) = delete;
+    DeviceBuffer& operator=(const DeviceBuffer&) = delete;
+    ~DeviceBuffer() { if (p) cudaFree(p); }
+    // at least `want` bytes; *fresh (nullable) tells whether this call allocated a new block
+    cudaError_t reserve(size_t want, bool* fresh = nullptr) {
+        if (fresh) *fresh = false;
+        int dev = 0;
+        cudaError_t e = cudaGetDevice(&dev);
+        if (e != cudaSuccess || (p && dev == device && want <= bytes)) return e;
+        if (p) { cudaDeviceSynchronize(); cudaFree(p); p = nullptr; bytes = 0; }
+        const size_t n = want + want / 2 > 256 ? want + want / 2 : 256;
+        e = cudaMalloc(&p, n);
+        if (e != cudaSuccess) { p = nullptr; return e; }
+        bytes = n; device = dev;
+        if (fresh) *fresh = true;
+        return cudaSuccess;
+    }
+    template <typename T>
+    T* as() const { return static_cast<T*>(p); }
+};
+
 struct AbrEnv {
     EnvView v{};
     int device = 0;
@@ -46,8 +73,8 @@ struct AbrEnv {
     uint32_t step_base = 0;   // fused-episode steps since the last reset: offsets the random policy's counter (SPEC §4)
     int32_t* d_perm = nullptr;   // session order installed by abr_env_set_order (capacity entries), v.perm points here when set
     int n_order = 0;
-    int32_t* d_sort_hist = nullptr;   // (trace, run) cells of abr_env_reset_sorted's counting sort, grow-only
-    size_t sort_hist_cap = 0, sort_scan_bytes = 0;
+    DeviceBuffer sort_hist;   // (trace, run) cells of abr_env_reset_sorted's counting sort, zero between calls
+    DeviceBuffer sort_scan;   // the scan's scratch of that sort
     int fresh_partials = 0;   // > 0: d_stats_partials holds that many block sums of the current accumulators
     double* d_stats_out = nullptr;
     uint32_t* d_draw_counter = nullptr;       // draws of abr_env_step_policy since the last reset
@@ -55,17 +82,11 @@ struct AbrEnv {
     // scratch for the *_host entry points
     int32_t* d_trace_id = nullptr;
     double* d_offset = nullptr;
-    int32_t* d_actions = nullptr;
-    size_t d_actions_cap = 0;
-    double* d_reward_traj = nullptr;
-    size_t d_reward_cap = 0;
+    DeviceBuffer actions, reward_traj;        // abr_env_run_host's [steps][N] actions in and reward trajectory out
     double bola_vmax = 0.0;   // max over the log table of SPEC §4.3 (when every size is > 0, i.e. v.pol.bola_v is set)
 
     ~AbrEnv() {
         for (void* p : allocs) cudaFree(p);
-        if (d_actions) cudaFree(d_actions);
-        if (d_reward_traj) cudaFree(d_reward_traj);
-        if (d_sort_hist) cudaFree(d_sort_hist);
     }
     template <typename T>
     cudaError_t alloc(T** out, size_t count) {
@@ -75,6 +96,16 @@ struct AbrEnv {
         return e;
     }
 };
+
+// The calls that take host tables validate them first, so that bad arguments are reported without a device.
+static int require_device() {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(ABR_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
+    }
+    return ABR_OK;
+}
 
 extern "C" {
 
@@ -189,11 +220,7 @@ int abr_env_create(const double* h_trace_bw, const int32_t* h_trace_len, const d
                 return fail(ABR_ERR_INVALID, "trace %d segment %d: bandwidth %g must be finite and > 0", t, i, b);
         }
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(ABR_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
-    }
+    if (int rc = require_device()) return rc;
     AbrEnv* e = new (std::nothrow) AbrEnv();
     if (!e) return fail(ABR_ERR_INVALID, "out of host memory");
     struct Guard { AbrEnv* e; ~Guard() { delete e; } } guard{e};
@@ -318,22 +345,19 @@ int abr_sort_by_trace(const int32_t* d_trace_id, int n_sessions, int n_traces, i
     // per call: the default pool hands its memory back to the driver at every synchronisation.)  An event orders the
     // buffer's reuse when consecutive calls come in on different streams.
     struct Scratch {
-        void* p = nullptr; size_t cap = 0; int device = -1; cudaEvent_t last = nullptr;
-        ~Scratch() { if (p) cudaFree(p); if (last) cudaEventDestroy(last); }
+        DeviceBuffer buf; cudaEvent_t last = nullptr;
+        ~Scratch() { if (last) cudaEventDestroy(last); }
     };
     thread_local Scratch sc;
-    int dev = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    if (dev != sc.device || bytes > sc.cap) {
-        if (sc.p) { cudaDeviceSynchronize(); cudaFree(sc.p); sc.p = nullptr; sc.cap = 0; }
+    bool fresh = false;
+    CUDA_TRY(sc.buf.reserve(bytes, &fresh));
+    if (fresh) {   // a new block, on the current device: so is the event
         if (sc.last) { cudaEventDestroy(sc.last); sc.last = nullptr; }
-        CUDA_TRY(cudaMalloc(&sc.p, bytes + bytes / 2));
-        sc.cap = bytes + bytes / 2; sc.device = dev;
         CUDA_TRY(cudaEventCreateWithFlags(&sc.last, cudaEventDisableTiming));
     } else {
         CUDA_TRY(cudaStreamWaitEvent(st, sc.last, 0));
     }
-    CUDA_TRY(launch_sort_by_trace(d_trace_id, n_sessions, n_traces, d_perm, sc.p, &bytes, st));
+    CUDA_TRY(launch_sort_by_trace(d_trace_id, n_sessions, n_traces, d_perm, sc.buf.p, &bytes, st));
     CUDA_TRY(cudaEventRecord(sc.last, st));
     return ABR_OK;
 }
@@ -343,11 +367,17 @@ static int check_capacity(const AbrEnv* env, int n_sessions) {
     return ABR_OK;
 }
 
-// A batch of n_sessions fits the environment and the session order installed for it, if any.
-static int check_batch(const AbrEnv* env, int n_sessions) {
-    if (int rc = check_capacity(env, n_sessions)) return rc;
+// A batch of n_sessions fits the session order installed for it, if any.
+static int check_order(const AbrEnv* env, int n_sessions) {
     if (env->v.perm && env->n_order != n_sessions)
         return fail(ABR_ERR_STATE, "the installed session order has %d entries, the batch %d (abr_env_set_order)", env->n_order, n_sessions);
+    return ABR_OK;
+}
+
+// The start of every call on the current batch (an empty batch then makes the call a no-op).
+static int check_reset(const AbrEnv* env) {
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
     return ABR_OK;
 }
 
@@ -381,7 +411,7 @@ int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stre
     if (policy != ABR_POLICY_BBA && policy != ABR_POLICY_RATE && policy != ABR_POLICY_BOLA)
         return fail(ABR_ERR_INVALID, "abr_env_policy_decide takes ABR_POLICY_BBA, _RATE or _BOLA (got %d)", policy);
     if (int rc = check_policy(env, policy)) return rc;
-    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+    if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
     CUDA_TRY(launch_policy_decide(env->v, policy, d_action, (cudaStream_t)stream));
@@ -402,7 +432,8 @@ int abr_env_set_order(AbrEnv* env, const int32_t* d_perm, int n_sessions, void* 
 int abr_env_reset(AbrEnv* env, const int32_t* d_trace_id, const double* d_start_offset, int n_sessions,
                   long long session_base, void* stream) {
     if (!env || (!d_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    if (int rc = check_batch(env, n_sessions)) return rc;
+    if (int rc = check_capacity(env, n_sessions)) return rc;
+    if (int rc = check_order(env, n_sessions)) return rc;
     begin_batch(env, n_sessions, session_base);
     CUDA_TRY(launch_reset(env->v, d_trace_id, d_start_offset, env->d_draw_counter, (cudaStream_t)stream));
     return ABR_OK;
@@ -430,16 +461,12 @@ int abr_env_reset_sorted(AbrEnv* env, const int32_t* d_trace_id, const double* d
         if (n_blocks > 0) {
             const size_t cells = (((size_t)env->v.n_traces * n_blocks) + 63) & ~(size_t)63;
             const size_t scan_bytes = sort_scan_tmp_bytes((int)cells);
-            if (cells > env->sort_hist_cap) {
-                if (env->d_sort_hist) { cudaDeviceSynchronize(); cudaFree(env->d_sort_hist); env->d_sort_hist = nullptr; env->sort_hist_cap = 0; }
-                CUDA_TRY(cudaMalloc(&env->d_sort_hist, sizeof(int32_t) * cells + scan_bytes));
-                CUDA_TRY(cudaMemset(env->d_sort_hist, 0, sizeof(int32_t) * cells));   // the sort leaves it zero
-                env->sort_hist_cap = cells;
-                env->sort_scan_bytes = scan_bytes;
-            }
-            // the scan's scratch sits behind the capacity's cells (its size grows with the cell count)
-            CUDA_TRY(launch_sort_gather(d_trace_id, d_start_offset, n_sessions, env->v.n_traces, S, n_blocks, env->d_sort_hist,
-                                        env->d_sort_hist + env->sort_hist_cap, env->sort_scan_bytes,
+            bool fresh = false;
+            CUDA_TRY(env->sort_hist.reserve(sizeof(int32_t) * cells, &fresh));
+            if (fresh) CUDA_TRY(cudaMemset(env->sort_hist.p, 0, env->sort_hist.bytes));   // the sort leaves it zero
+            CUDA_TRY(env->sort_scan.reserve(scan_bytes));
+            CUDA_TRY(launch_sort_gather(d_trace_id, d_start_offset, n_sessions, env->v.n_traces, S, n_blocks,
+                                        env->sort_hist.as<int32_t>(), env->sort_scan.p, scan_bytes,
                                         env->d_perm, env->d_trace_id, env->d_offset, st));
         } else {   // shapes the counting sort does not take: CUB's radix sort, then one gather
             int rc = abr_sort_by_trace(d_trace_id, n_sessions, env->v.n_traces, env->d_perm, stream);
@@ -468,8 +495,7 @@ template <typename OT>
 static int env_step_any(AbrEnv* env, const int32_t* d_action, const double* d_speed, OT* d_delay, OT* d_sleep,
                         OT* d_buffer, OT* d_rebuf, OT* d_reward, OT* d_latency, OT* d_next_sizes,
                         uint8_t* d_end_of_video, OT* d_throughput, void* stream) {
-    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
-    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+    if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
     env->fresh_partials = 0;
@@ -491,8 +517,7 @@ int abr_env_step_live(AbrEnv* env, const int32_t* d_action, const double* d_spee
 int abr_env_step_policy(AbrEnv* env, const float* d_logits, int sample, uint64_t seed, const AbrObsSpec* spec,
                         float* d_obs, int32_t* d_action_out, double* d_reward_sum, double* d_delay, double* d_sleep,
                         double* d_buffer, double* d_rebuf, double* d_reward, uint8_t* d_end_of_video, void* stream) {
-    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
-    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+    if (int rc = check_reset(env)) return rc;
     if (env->v.p.live) return fail(ABR_ERR_STATE, "abr_env_step_policy is not available in live mode (SPEC 7)");
     if (env->v.n == 0) return ABR_OK;
     if (!d_logits) return fail(ABR_ERR_INVALID, "logits is NULL");
@@ -534,31 +559,36 @@ int abr_env_qoe_cost(AbrEnv* env, double* d_out, void* stream) {
 }
 
 extern "C++" {
+// A fused episode of the current batch, whose other arguments have passed the caller's checks.
+template <typename OT>
+static int episode(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t* d_actions_in, const double* d_speed,
+                   const StepOutputs<OT>& o, cudaStream_t st, const RolloutFused& fused = RolloutFused{}) {
+    // the kernel indexes the [steps][N] outputs with 32 bits (4 Gi elements of one array are 32 GB)
+    if ((unsigned long long)steps * (unsigned long long)env->v.n > 0xffffffffull)
+        return fail(ABR_ERR_RANGE, "steps * sessions = %llu exceeds 2^32 - 1: split the episode into several calls",
+                    (unsigned long long)steps * (unsigned long long)env->v.n);
+    CUDA_TRY(launch_rollout(env->v, policy, seed, steps, env->step_base, d_actions_in, d_speed, o, env->d_stats_partials,
+                            fused, st));
+    env->step_base += (uint32_t)steps;
+    env->fresh_partials = steps > 0 ? rollout_num_blocks(env->v.n) : 0;
+    return ABR_OK;
+}
+
 template <typename OT>
 static int env_rollout_any(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t* d_actions_in,
                            const double* d_speed, OT* d_delay, OT* d_sleep, OT* d_buffer, OT* d_rebuf, OT* d_reward,
-                           OT* d_latency, uint8_t* d_end_of_video, int32_t* d_actions_out, void* stream,
-                           const RolloutFused& fused = RolloutFused{}) {
-    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
-    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+                           OT* d_latency, uint8_t* d_end_of_video, int32_t* d_actions_out, void* stream) {
+    if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
     if (int rc_p = check_policy(env, policy)) return rc_p;
     if (policy == ABR_POLICY_FIXED && !d_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
     if (!env->v.p.live && (d_speed || d_latency))
         return fail(ABR_ERR_STATE, "speed / latency belong to live mode (SPEC 7): create the environment with live = 1");
-    // the kernel indexes the [steps][N] outputs with 32 bits (4 Gi elements of one array are 32 GB)
-    if ((unsigned long long)steps * (unsigned long long)env->v.n > 0xffffffffull)
-        return fail(ABR_ERR_RANGE, "steps * sessions = %llu exceeds 2^32 - 1: split the episode into several calls",
-                    (unsigned long long)steps * (unsigned long long)env->v.n);
     StepOutputs<OT> o;
     o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
     o.eov = d_end_of_video; o.actions = d_actions_out; o.latency = d_latency;
-    CUDA_TRY(launch_rollout(env->v, policy, seed, steps, env->step_base, d_actions_in, d_speed, o, env->d_stats_partials,
-                            fused, (cudaStream_t)stream));
-    env->step_base += (uint32_t)steps;
-    env->fresh_partials = steps > 0 ? rollout_num_blocks(env->v.n) : 0;
-    return ABR_OK;
+    return episode(env, policy, seed, steps, d_actions_in, d_speed, o, (cudaStream_t)stream);
 }
 }  // extern "C++"
 
@@ -595,8 +625,7 @@ static int check_mpc_shape(int A, int H) {
 }
 
 int abr_env_mpc_decide(AbrEnv* env, int horizon, int mode, int32_t* d_action, double* d_best_j, void* stream) {
-    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
-    if (!env->was_reset) return fail(ABR_ERR_STATE, "abr_env_reset has not been called");
+    if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
     const bool exhaustive = (mode & ABR_MPC_MODE_EXHAUSTIVE) != 0;
@@ -671,44 +700,48 @@ int abr_env_error_count(AbrEnv* env, long long* out, void* stream) {
     return ABR_OK;
 }
 
+// abr_env_run and abr_env_run_host on device pointers, after their checks: with sessions and steps, one episode kernel
+// that resets the sessions itself (no state round trip through HBM) and writes the session cost and the statistics;
+// otherwise the reset, the cost and the statistics of the reset state.
+static int run_batch(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t* d_trace_id,
+                     const double* d_start_offset, int n_sessions, long long session_base, const int32_t* d_actions_in,
+                     const StepOutputs<double>& o, double* d_qoe_cost, double* d_stats, cudaStream_t st) {
+    begin_batch(env, n_sessions, session_base);
+    if (n_sessions > 0 && steps > 0) {
+        RolloutFused fused;
+        fused.in_trace_id = d_trace_id; fused.in_offset = d_start_offset; fused.out_cost = d_qoe_cost;
+        fused.out_stats = d_stats; fused.scratch = env->stats_scratch;   // statistics by the kernel's own blocks
+        return episode(env, policy, seed, steps, d_actions_in, nullptr, o, st, fused);
+    }
+    CUDA_TRY(launch_reset(env->v, d_trace_id, d_start_offset, env->d_draw_counter, st));
+    if (d_qoe_cost) CUDA_TRY(launch_qoe_cost(env->v, d_qoe_cost, st));
+    return d_stats ? abr_stats_partial(env, d_stats, st) : ABR_OK;
+}
+
 int abr_env_run(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t* d_trace_id,
                 const double* d_start_offset, int n_sessions, long long session_base, const int32_t* d_actions_in,
                 double* d_delay, double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward,
                 uint8_t* d_end_of_video, int32_t* d_actions_out, double* d_qoe_cost, double* d_stats, void* stream) {
     if (!env || (!d_trace_id && n_sessions > 0)) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    int rc = check_capacity(env, n_sessions);
-    if (rc) return rc;
+    if (int rc = check_capacity(env, n_sessions)) return rc;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
-    if (int rc_p = check_policy(env, policy)) return rc_p;
+    if (int rc = check_policy(env, policy)) return rc;
     if (policy == ABR_POLICY_FIXED && !d_actions_in && n_sessions > 0 && steps > 0)
         return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
-    if ((rc = check_batch(env, n_sessions))) return rc;
-    if (n_sessions > 0 && steps > 0) {   // the episode kernel resets the sessions itself and writes the session cost
-        begin_batch(env, n_sessions, session_base);
-        RolloutFused fused;
-        fused.in_trace_id = d_trace_id; fused.in_offset = d_start_offset; fused.out_cost = d_qoe_cost;
-        fused.out_stats = d_stats; fused.scratch = env->stats_scratch;   // statistics by the kernel's own blocks
-        rc = env_rollout_any<double>(env, policy, seed, steps, d_actions_in, nullptr, d_delay, d_sleep, d_buffer, d_rebuf,
-                                     d_reward, nullptr, d_end_of_video, d_actions_out, stream, fused);
-        return rc;
-    } else {
-        rc = abr_env_reset(env, d_trace_id, d_start_offset, n_sessions, session_base, stream);
-        if (rc) return rc;
-        if (d_qoe_cost) CUDA_TRY(launch_qoe_cost(env->v, d_qoe_cost, (cudaStream_t)stream));
-    }
-    return d_stats ? abr_stats_partial(env, d_stats, stream) : ABR_OK;
+    if (int rc = check_order(env, n_sessions)) return rc;
+    StepOutputs<double> o;
+    o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
+    o.eov = d_end_of_video; o.actions = d_actions_out;
+    return run_batch(env, policy, seed, steps, d_trace_id, d_start_offset, n_sessions, session_base, d_actions_in, o,
+                     d_qoe_cost, d_stats, (cudaStream_t)stream);
 }
 
 // Zero-copy: a host pointer inside page-locked memory (cudaHostAlloc / cudaHostRegister, e.g. a pinned torch tensor)
 // has a device alias under unified addressing; the kernels then read the inputs and write the results over PCIe
 // themselves, which removes the copy launches and overlaps the transfers with the kernels' other work.  Returns
-// nullptr for pageable memory (the staged cudaMemcpyAsync path is used).  ABR_ZERO_COPY=0 disables it (A/B timing).
+// nullptr for pageable memory (the staged cudaMemcpyAsync path is used).
 static void* device_alias(const void* h) {
-    static const bool enabled = [] {
-        const char* e = getenv("ABR_ZERO_COPY");
-        return !(e && e[0] == '0');
-    }();
-    if (!h || !enabled) return nullptr;
+    if (!h) return nullptr;
     cudaPointerAttributes a{};
     if (cudaPointerGetAttributes(&a, h) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
@@ -720,125 +753,78 @@ int abr_env_run_host(AbrEnv* env, int policy, uint64_t seed, int steps, const in
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
     if (!h_trace_id && n_sessions > 0) return fail(ABR_ERR_INVALID, "env or trace_id is NULL");
-    int rc = check_capacity(env, n_sessions);
-    if (rc) return rc;
-    if (int rc_p = check_policy(env, policy)) return rc_p;
+    if (int rc = check_capacity(env, n_sessions)) return rc;
+    if (int rc = check_policy(env, policy)) return rc;
     if (policy == ABR_POLICY_FIXED && !h_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs h_actions_in");
-    if ((rc = check_batch(env, n_sessions))) return rc;
+    if (int rc = check_order(env, n_sessions)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    // inputs: device aliases of page-locked buffers (read over PCIe by the kernel), else staged copies
+    // inputs: device aliases of page-locked buffers (read over PCIe by the kernels), else copies into the scratch
     const int32_t* tid = (const int32_t*)device_alias(h_trace_id);
-    if (!tid && n_sessions > 0) {
-        CUDA_TRY(cudaMemcpyAsync(env->d_trace_id, h_trace_id, sizeof(int32_t) * n_sessions, cudaMemcpyHostToDevice, st));
+    if (!tid) {
+        if (n_sessions > 0)
+            CUDA_TRY(cudaMemcpyAsync(env->d_trace_id, h_trace_id, sizeof(int32_t) * n_sessions, cudaMemcpyHostToDevice, st));
         tid = env->d_trace_id;
     }
-    if (!tid) tid = env->d_trace_id;   // empty batch
-    const double* off = nullptr;
-    if (h_start_offset) {
-        off = (const double*)device_alias(h_start_offset);
-        if (!off) {
-            CUDA_TRY(cudaMemcpyAsync(env->d_offset, h_start_offset, sizeof(double) * n_sessions, cudaMemcpyHostToDevice, st));
-            off = env->d_offset;
-        }
-    }
-    // The episode kernel resets the sessions itself (one launch, no state round trip through HBM) unless there is
-    // no episode to run; the per-session cost goes straight to a page-locked h_qoe_cost from the same kernel.
-    const bool fuse = n_sessions > 0 && steps > 0;
-    double* z_cost = fuse ? (double*)device_alias(h_qoe_cost) : nullptr;
-    if (fuse) {
-        begin_batch(env, n_sessions, session_base);
-    } else {
-        rc = abr_env_reset(env, tid, off, n_sessions, session_base, stream);
-        if (rc) return rc;
+    const double* off = (const double*)device_alias(h_start_offset);
+    if (h_start_offset && !off) {
+        CUDA_TRY(cudaMemcpyAsync(env->d_offset, h_start_offset, sizeof(double) * n_sessions, cudaMemcpyHostToDevice, st));
+        off = env->d_offset;
     }
     const size_t traj = (size_t)steps * n_sessions;
+    const int32_t* d_actions = nullptr;
     if (policy == ABR_POLICY_FIXED) {
-        if (traj > env->d_actions_cap) {
-            if (env->d_actions) cudaFree(env->d_actions);
-            env->d_actions = nullptr; env->d_actions_cap = 0;
-            CUDA_TRY(cudaMalloc(&env->d_actions, sizeof(int32_t) * (traj ? traj : 1)));
-            env->d_actions_cap = traj;
-        }
-        CUDA_TRY(cudaMemcpyAsync(env->d_actions, h_actions_in, sizeof(int32_t) * traj, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(env->actions.reserve(sizeof(int32_t) * traj));
+        d_actions = env->actions.as<int32_t>();
+        CUDA_TRY(cudaMemcpyAsync(env->actions.p, h_actions_in, sizeof(int32_t) * traj, cudaMemcpyHostToDevice, st));
     }
-    if (h_reward_traj && traj > env->d_reward_cap) {
-        if (env->d_reward_traj) cudaFree(env->d_reward_traj);
-        env->d_reward_traj = nullptr; env->d_reward_cap = 0;
-        CUDA_TRY(cudaMalloc(&env->d_reward_traj, sizeof(double) * (traj ? traj : 1)));
-        env->d_reward_cap = traj;
+    StepOutputs<double> o;
+    if (h_reward_traj) {
+        CUDA_TRY(env->reward_traj.reserve(sizeof(double) * traj));
+        o.reward = env->reward_traj.as<double>();
     }
-    RolloutFused fused;
-    double* z_stats = h_stats ? (double*)device_alias(h_stats) : nullptr;
-    if (fuse) {
-        fused.in_trace_id = tid; fused.in_offset = off; fused.out_cost = z_cost;
-        if (h_stats) { fused.out_stats = z_stats ? z_stats : env->d_stats_out; fused.scratch = env->stats_scratch; }
-    }
-    rc = env_rollout_any<double>(env, policy, seed, steps, policy == ABR_POLICY_FIXED ? env->d_actions : nullptr, nullptr,
-                                 nullptr, nullptr, nullptr, nullptr, h_reward_traj ? env->d_reward_traj : nullptr,
-                                 nullptr, nullptr, nullptr, stream, fused);
-    if (rc) return rc;
-    if (h_stats) {
-        if (!fuse) {   // no episode ran: the statistics of the reset state
-            rc = abr_stats_partial(env, z_stats ? z_stats : env->d_stats_out, stream);
-            if (rc) return rc;
-        }
-        if (!z_stats)
-            CUDA_TRY(cudaMemcpyAsync(h_stats, env->d_stats_out, sizeof(double) * ABR_NUM_STATS, cudaMemcpyDeviceToHost, st));
-    }
+    // outputs: page-locked ones are written by the kernels through their aliases; pageable statistics go through
+    // d_stats_out, a pageable cost through d_offset (free again once the sessions are reset) by a launch of its own
+    double* z_cost = (double*)device_alias(h_qoe_cost);
+    double* z_stats = (double*)device_alias(h_stats);
+    if (int rc = run_batch(env, policy, seed, steps, tid, off, n_sessions, session_base, d_actions, o, z_cost,
+                           h_stats && !z_stats ? env->d_stats_out : z_stats, st))
+        return rc;
+    if (h_stats && !z_stats)
+        CUDA_TRY(cudaMemcpyAsync(h_stats, env->d_stats_out, sizeof(double) * ABR_NUM_STATS, cudaMemcpyDeviceToHost, st));
     if (h_acc) {
         // acc rows are strided by the capacity on the device; the host table is dense [ABR_NUM_ACC][N]
         CUDA_TRY(cudaMemcpy2DAsync(h_acc, sizeof(double) * n_sessions, env->v.acc, sizeof(double) * env->v.cap,
                                    sizeof(double) * n_sessions, ABR_NUM_ACC, cudaMemcpyDeviceToHost, st));
     }
     if (h_reward_traj)
-        CUDA_TRY(cudaMemcpyAsync(h_reward_traj, env->d_reward_traj, sizeof(double) * traj, cudaMemcpyDeviceToHost, st));
-    if (h_qoe_cost) {
-        double* z_alias = z_cost ? nullptr : (double*)device_alias(h_qoe_cost);
-        if (z_cost) {                                                // already written by the episode kernel
-        } else if (z_alias) {
-            CUDA_TRY(launch_qoe_cost(env->v, z_alias, st));          // written to host memory by the kernel
-        } else {                                                     // d_offset is free again after the reset
-            CUDA_TRY(launch_qoe_cost(env->v, env->d_offset, st));
-            CUDA_TRY(cudaMemcpyAsync(h_qoe_cost, env->d_offset, sizeof(double) * n_sessions, cudaMemcpyDeviceToHost, st));
-        }
+        CUDA_TRY(cudaMemcpyAsync(h_reward_traj, o.reward, sizeof(double) * traj, cudaMemcpyDeviceToHost, st));
+    if (h_qoe_cost && !z_cost) {
+        CUDA_TRY(launch_qoe_cost(env->v, env->d_offset, st));
+        CUDA_TRY(cudaMemcpyAsync(h_qoe_cost, env->d_offset, sizeof(double) * n_sessions, cudaMemcpyDeviceToHost, st));
     }
     CUDA_TRY(cudaStreamSynchronize(st));
     return ABR_OK;
 }
 
-static int mpc_decide_impl(const double* d_sizes, const double* d_utility, int V, int A, const AbrParams* params, int N,
-                           const int32_t* d_chunk_idx, const int32_t* d_prev_q, const double* d_buffer,
-                           const double* d_bw_hist, const int32_t* d_hist_len, int K, double* d_last_pred,
-                           double* d_err_ring, int32_t* d_err_len, int horizon, int mode, int flags,
-                           const uint8_t* d_startup, int n_ts, double ts_step, int32_t* d_action,
-                           double* d_startup_delay, double* d_best_j, int32_t* d_best_seq, double* d_preds,
-                           int32_t* d_error_count, void* stream) {
-    if (!d_sizes || !d_utility || !d_chunk_idx || !d_prev_q || !d_buffer || !d_bw_hist || !d_hist_len || !d_action)
+// The standalone decision of abr_mpc_decide*: checks the arguments `a` names, completes it and launches.
+static int mpc_decide(MpcArgs a, const AbrParams* params, cudaStream_t st) {
+    if (!a.sizes || !a.util || !a.chunk_idx || !a.prev_q || !a.buffer || !a.bw_hist || !a.hist_len || !a.action)
         return fail(ABR_ERR_INVALID, "a required pointer is NULL");
     if (!params) return fail(ABR_ERR_INVALID, "params is NULL");
-    if (N < 0 || V < 1) return fail(ABR_ERR_RANGE, "N must be >= 0 and V >= 1");
-    if (K < 1) return fail(ABR_ERR_RANGE, "K must be >= 1");
-    if (mode != ABR_MPC_REF && mode != ABR_MPC_ROBUST) return fail(ABR_ERR_INVALID, "unknown MPC mode %d", mode);
-    if ((flags & ABR_MPC_PRED_SES) && mode != ABR_MPC_REF)
+    if (a.N < 0 || a.V < 1) return fail(ABR_ERR_RANGE, "N must be >= 0 and V >= 1");
+    if (a.K < 1) return fail(ABR_ERR_RANGE, "K must be >= 1");
+    if (a.mode != ABR_MPC_REF && a.mode != ABR_MPC_ROBUST) return fail(ABR_ERR_INVALID, "unknown MPC mode %d", a.mode);
+    if ((a.flags & ABR_MPC_PRED_SES) && a.mode != ABR_MPC_REF)
         return fail(ABR_ERR_INVALID, "ABR_MPC_PRED_SES (mpc.py:72-79) replaces the predictor of mode 0; the robust mode defines its own");
-    if ((d_last_pred || d_err_ring || d_err_len) && !(d_last_pred && d_err_ring && d_err_len))
+    if ((a.last_pred || a.err_ring || a.err_len) && !(a.last_pred && a.err_ring && a.err_len))
         return fail(ABR_ERR_INVALID, "last_pred, err_ring and err_len must be given together");
-    if (n_ts < 1 || n_ts > 4096) return fail(ABR_ERR_RANGE, "n_ts must be in [1, 4096] (got %d)", n_ts);
-    if (n_ts > 1 && !(ts_step > 0.0 && std::isfinite(ts_step))) return fail(ABR_ERR_RANGE, "ts_step must be finite and > 0");
-    if (n_ts > 1 && !std::isfinite(params->startup_penalty)) return fail(ABR_ERR_INVALID, "startup_penalty must be finite");
-    int rc = check_mpc_shape(A, horizon);
-    if (rc) return rc;
-    MpcArgs a{};
-    a.sizes = d_sizes; a.util = d_utility; a.V = V; a.A = A; a.p = *params; a.N = N;
-    a.chunk_idx = d_chunk_idx; a.prev_q = d_prev_q; a.buffer = d_buffer; a.done = nullptr;
-    a.bw_hist = d_bw_hist; a.hist_len = d_hist_len; a.K = K;
-    a.hist_session_stride = K; a.hist_slot_stride = 1;        // standalone rings are [N][K]
-    a.last_pred = d_last_pred; a.err_ring = d_err_ring; a.err_len = d_err_len;
-    a.H = horizon; a.mode = mode; a.flags = flags;
-    a.action = d_action; a.best_j = d_best_j; a.best_seq = d_best_seq; a.preds = d_preds;
-    a.error_count64 = nullptr; a.error_count32 = d_error_count;
-    a.startup = d_startup; a.n_ts = n_ts; a.ts_step = ts_step; a.startup_delay = d_startup_delay;
-    CUDA_TRY(launch_mpc(a, (cudaStream_t)stream));
+    if (a.n_ts < 1 || a.n_ts > 4096) return fail(ABR_ERR_RANGE, "n_ts must be in [1, 4096] (got %d)", a.n_ts);
+    if (a.n_ts > 1 && !(a.ts_step > 0.0 && std::isfinite(a.ts_step))) return fail(ABR_ERR_RANGE, "ts_step must be finite and > 0");
+    if (a.n_ts > 1 && !std::isfinite(params->startup_penalty)) return fail(ABR_ERR_INVALID, "startup_penalty must be finite");
+    if (int rc = check_mpc_shape(a.A, a.H)) return rc;
+    a.p = *params;
+    a.hist_session_stride = a.K; a.hist_slot_stride = 1;        // standalone rings are [N][K]
+    CUDA_TRY(launch_mpc(a, st));
     return ABR_OK;
 }
 
@@ -847,9 +833,12 @@ int abr_mpc_decide(const double* d_sizes, const double* d_utility, int V, int A,
                    const int32_t* d_hist_len, int K, double* d_last_pred, double* d_err_ring, int32_t* d_err_len,
                    int horizon, int mode, int flags, int32_t* d_action, double* d_best_j, int32_t* d_best_seq,
                    double* d_preds, int32_t* d_error_count, void* stream) {
-    return mpc_decide_impl(d_sizes, d_utility, V, A, params, N, d_chunk_idx, d_prev_q, d_buffer, d_bw_hist, d_hist_len, K,
-                           d_last_pred, d_err_ring, d_err_len, horizon, mode, flags, nullptr, 1, 0.0, d_action, nullptr,
-                           d_best_j, d_best_seq, d_preds, d_error_count, stream);
+    MpcArgs a{};
+    a.sizes = d_sizes; a.util = d_utility; a.V = V; a.A = A; a.N = N; a.K = K; a.H = horizon; a.mode = mode; a.flags = flags;
+    a.chunk_idx = d_chunk_idx; a.prev_q = d_prev_q; a.buffer = d_buffer; a.bw_hist = d_bw_hist; a.hist_len = d_hist_len;
+    a.last_pred = d_last_pred; a.err_ring = d_err_ring; a.err_len = d_err_len;
+    a.action = d_action; a.best_j = d_best_j; a.best_seq = d_best_seq; a.preds = d_preds; a.error_count32 = d_error_count;
+    return mpc_decide(a, params, (cudaStream_t)stream);
 }
 
 int abr_mpc_decide_startup(const double* d_sizes, const double* d_utility, int V, int A, const AbrParams* params, int N,
@@ -860,65 +849,60 @@ int abr_mpc_decide_startup(const double* d_sizes, const double* d_utility, int V
                            double* d_startup_delay, double* d_best_j, int32_t* d_best_seq, double* d_preds,
                            int32_t* d_error_count, void* stream) {
     if (!d_startup_delay) return fail(ABR_ERR_INVALID, "startup_delay is NULL");
-    return mpc_decide_impl(d_sizes, d_utility, V, A, params, N, d_chunk_idx, d_prev_q, d_buffer, d_bw_hist, d_hist_len, K,
-                           d_last_pred, d_err_ring, d_err_len, horizon, mode, flags, d_startup, n_ts, ts_step, d_action,
-                           d_startup_delay, d_best_j, d_best_seq, d_preds, d_error_count, stream);
+    MpcArgs a{};
+    a.sizes = d_sizes; a.util = d_utility; a.V = V; a.A = A; a.N = N; a.K = K; a.H = horizon; a.mode = mode; a.flags = flags;
+    a.chunk_idx = d_chunk_idx; a.prev_q = d_prev_q; a.buffer = d_buffer; a.bw_hist = d_bw_hist; a.hist_len = d_hist_len;
+    a.last_pred = d_last_pred; a.err_ring = d_err_ring; a.err_len = d_err_len;
+    a.action = d_action; a.best_j = d_best_j; a.best_seq = d_best_seq; a.preds = d_preds; a.error_count32 = d_error_count;
+    a.startup = d_startup; a.n_ts = n_ts; a.ts_step = ts_step; a.startup_delay = d_startup_delay;
+    return mpc_decide(a, params, (cudaStream_t)stream);
+}
+
+// The host tables and parameters of abr_mpc_decide*_host and abr_mpc_score_host.
+static int check_host_tables(const double* h_sizes, const double* h_bitrates, int V, int A, const AbrParams* params) {
+    if (int rc = check_tables(h_sizes, h_bitrates, V, A)) return rc;
+    return params ? ABR_OK : fail(ABR_ERR_INVALID, "params is NULL");
 }
 
 // ---- host-buffer decisions: one staging arena per host thread (grow-only, released at thread exit), so that a
 //      decision is one host->device copy, one kernel and one device->host copy — no allocation on the call path ----
 namespace {
 struct HostArena {
-    char* dev = nullptr; char* pin = nullptr; size_t cap = 0; int device = -1;
-    ~HostArena() { release(); }
-    void release() {
-        if (dev) cudaFree(dev);
-        if (pin) cudaFreeHost(pin);
-        dev = pin = nullptr; cap = 0;
-    }
+    DeviceBuffer dev;
+    char* pin = nullptr;   // as large as dev
+    ~HostArena() { if (pin) cudaFreeHost(pin); }
     cudaError_t reserve(size_t bytes) {
-        int cur = 0;
-        cudaError_t e = cudaGetDevice(&cur);
-        if (e != cudaSuccess) return e;
-        if (cur == device && bytes <= cap) return cudaSuccess;
-        release();
-        size_t want = bytes < (64u << 10) ? (64u << 10) : bytes + bytes / 2;
-        e = cudaMalloc((void**)&dev, want);
-        if (e != cudaSuccess) { dev = nullptr; return e; }
-        e = cudaHostAlloc((void**)&pin, want, cudaHostAllocDefault);
-        if (e != cudaSuccess) { cudaFree(dev); dev = pin = nullptr; return e; }
-        cap = want; device = cur;
-        return cudaSuccess;
+        bool fresh = false;
+        cudaError_t e = dev.reserve(bytes < (64u << 10) ? (64u << 10) : bytes, &fresh);
+        if (e != cudaSuccess || (pin && !fresh)) return e;
+        if (pin) cudaFreeHost(pin);
+        e = cudaHostAlloc((void**)&pin, dev.bytes, cudaHostAllocDefault);
+        if (e != cudaSuccess) pin = nullptr;
+        return e;
     }
 };
 thread_local HostArena t_arena;
 inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+extern "C++" template <typename T>
+void point(T*& field, char* base, size_t off) { field = reinterpret_cast<T*>(base + off); }
 }  // namespace
 
-static int mpc_decide_host_impl(const double* h_sizes, const double* h_bitrates, int V, int A, const AbrParams* params,
-                                int N, const int32_t* h_chunk_idx, const int32_t* h_prev_q, const double* h_buffer,
-                                const double* h_bw_hist, const int32_t* h_hist_len, int K, double* h_last_pred,
-                                double* h_err_ring, int32_t* h_err_len, int horizon, int mode, int flags,
-                                const uint8_t* h_startup, int n_ts, double ts_step, int32_t* h_action,
-                                double* h_startup_delay, double* h_best_j, int32_t* h_best_seq, double* h_preds,
-                                int32_t* h_error_count) {
-    if (!h_chunk_idx || !h_prev_q || !h_buffer || !h_bw_hist || !h_hist_len || !h_action)
+// `a` names the caller's host buffers (sizes: the size table; util: unused, the utilities are computed from
+// h_bitrates).  They are packed into the arena and copied to the device in one piece, `a` is re-pointed at the device
+// copies for mpc_decide, and the outputs come back the same way.  A partial robust state counts as none.
+static int mpc_decide_host(MpcArgs a, const double* h_bitrates, const AbrParams* params) {
+    if (!a.chunk_idx || !a.prev_q || !a.buffer || !a.bw_hist || !a.hist_len || !a.action)
         return fail(ABR_ERR_INVALID, "a required pointer is NULL");
-    int rc = check_tables(h_sizes, h_bitrates, V, A);
-    if (rc) return rc;
-    if (!params) return fail(ABR_ERR_INVALID, "params is NULL");
-    if (N < 0 || K < 1) return fail(ABR_ERR_RANGE, "N must be >= 0 and K >= 1");
-    rc = check_mpc_shape(A, horizon);
-    if (rc) return rc;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(ABR_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
-    }
+    if (int rc = check_host_tables(a.sizes, h_bitrates, a.V, a.A, params)) return rc;
+    if (a.N < 0 || a.K < 1) return fail(ABR_ERR_RANGE, "N must be >= 0 and K >= 1");
+    if (int rc = check_mpc_shape(a.A, a.H)) return rc;
+    if (int rc = require_device()) return rc;
     std::vector<double> util;
-    utility_table(h_bitrates, V, A, params, util);
-    const size_t n = (size_t)(N > 0 ? N : 1), H = (size_t)horizon, VA = (size_t)V * A;
-    const bool robust_state = h_last_pred && h_err_ring && h_err_len;
+    utility_table(h_bitrates, a.V, a.A, params, util);
+    a.util = util.data();
+    if (!(a.last_pred && a.err_ring && a.err_len)) { a.last_pred = a.err_ring = nullptr; a.err_len = nullptr; }
+    const MpcArgs h = a;
+    const size_t N = (size_t)a.N, n = N > 0 ? N : 1, K = (size_t)a.K, H = (size_t)a.H, VA = (size_t)a.V * a.A;
     // arena layout: [inputs, copied host->device in one piece | outputs, copied back in one piece]
     size_t off = 0;
     auto take = [&off](size_t bytes) { const size_t o = off; off = align16(off + bytes); return o; };
@@ -931,45 +915,27 @@ static int mpc_decide_host_impl(const double* h_sizes, const double* h_bitrates,
     const size_t total = off;
     CUDA_TRY(t_arena.reserve(total));
     char* hp = t_arena.pin;
-    char* dp = t_arena.dev;
-    memcpy(hp + o_sizes, h_sizes, 8 * VA);
-    memcpy(hp + o_util, util.data(), 8 * VA);
-    memcpy(hp + o_buffer, h_buffer, 8 * (size_t)N);
-    memcpy(hp + o_hist, h_bw_hist, 8 * (size_t)N * K);
-    memcpy(hp + o_chunk, h_chunk_idx, 4 * (size_t)N);
-    memcpy(hp + o_pq, h_prev_q, 4 * (size_t)N);
-    memcpy(hp + o_hl, h_hist_len, 4 * (size_t)N);
-    if (h_startup) memcpy(hp + o_su, h_startup, (size_t)N);
-    if (robust_state) {
-        memcpy(hp + o_lp, h_last_pred, 8 * (size_t)N);
-        memcpy(hp + o_er, h_err_ring, 8 * (size_t)N * K);
-        memcpy(hp + o_el, h_err_len, 4 * (size_t)N);
-    }
+    char* dp = t_arena.dev.as<char>();
+    auto in = [&](auto*& field, size_t o, size_t bytes) {   // an input: packed, then read from its device copy
+        if (!field) return;
+        memcpy(hp + o, field, bytes);
+        point(field, dp, o);
+    };
+    in(a.sizes, o_sizes, 8 * VA); in(a.util, o_util, 8 * VA); in(a.buffer, o_buffer, 8 * N); in(a.bw_hist, o_hist, 8 * N * K);
+    in(a.chunk_idx, o_chunk, 4 * N); in(a.prev_q, o_pq, 4 * N); in(a.hist_len, o_hl, 4 * N); in(a.startup, o_su, N);
+    in(a.last_pred, o_lp, 8 * N); in(a.err_ring, o_er, 8 * N * K); in(a.err_len, o_el, 4 * N);
     memset(hp + o_ec, 0, 16);
+    point(a.action, dp, o_act); point(a.startup_delay, dp, o_ts); point(a.best_j, dp, o_bj); point(a.best_seq, dp, o_seq);
+    point(a.preds, dp, o_pr); point(a.error_count32, dp, o_ec);
     cudaStream_t st = 0;
     CUDA_TRY(cudaMemcpyAsync(dp, hp, in_bytes, cudaMemcpyHostToDevice, st));
-    rc = mpc_decide_impl((const double*)(dp + o_sizes), (const double*)(dp + o_util), V, A, params, N,
-                         (const int32_t*)(dp + o_chunk), (const int32_t*)(dp + o_pq), (const double*)(dp + o_buffer),
-                         (const double*)(dp + o_hist), (const int32_t*)(dp + o_hl), K,
-                         robust_state ? (double*)(dp + o_lp) : nullptr, robust_state ? (double*)(dp + o_er) : nullptr,
-                         robust_state ? (int32_t*)(dp + o_el) : nullptr, horizon, mode, flags,
-                         h_startup ? (const uint8_t*)(dp + o_su) : nullptr, n_ts, ts_step, (int32_t*)(dp + o_act),
-                         (double*)(dp + o_ts), (double*)(dp + o_bj), (int32_t*)(dp + o_seq), (double*)(dp + o_pr),
-                         (int32_t*)(dp + o_ec), st);
-    if (rc) return rc;
+    if (int rc = mpc_decide(a, params, st)) return rc;
     CUDA_TRY(cudaMemcpyAsync(hp + o_out, dp + o_out, total - o_out, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    memcpy(h_action, hp + o_act, 4 * (size_t)N);
-    if (h_startup_delay) memcpy(h_startup_delay, hp + o_ts, 8 * (size_t)N);
-    if (h_best_j) memcpy(h_best_j, hp + o_bj, 8 * (size_t)N);
-    if (h_best_seq) memcpy(h_best_seq, hp + o_seq, 4 * (size_t)N * H);
-    if (h_preds) memcpy(h_preds, hp + o_pr, 8 * (size_t)N * H);
-    if (h_error_count) memcpy(h_error_count, hp + o_ec, 4);
-    if (robust_state) {
-        memcpy(h_last_pred, hp + o_lp, 8 * (size_t)N);
-        memcpy(h_err_ring, hp + o_er, 8 * (size_t)N * K);
-        memcpy(h_err_len, hp + o_el, 4 * (size_t)N);
-    }
+    auto out = [hp](void* dst, size_t o, size_t bytes) { if (dst) memcpy(dst, hp + o, bytes); };
+    out(h.action, o_act, 4 * N); out(h.startup_delay, o_ts, 8 * N); out(h.best_j, o_bj, 8 * N);
+    out(h.best_seq, o_seq, 4 * N * H); out(h.preds, o_pr, 8 * N * H); out(h.error_count32, o_ec, 4);
+    out(h.last_pred, o_lp, 8 * N); out(h.err_ring, o_er, 8 * N * K); out(h.err_len, o_el, 4 * N);
     return ABR_OK;
 }
 
@@ -978,9 +944,12 @@ int abr_mpc_decide_host(const double* h_sizes, const double* h_bitrates, int V, 
                         const double* h_bw_hist, const int32_t* h_hist_len, int K, double* h_last_pred,
                         double* h_err_ring, int32_t* h_err_len, int horizon, int mode, int flags, int32_t* h_action,
                         double* h_best_j, int32_t* h_best_seq, double* h_preds, int32_t* h_error_count) {
-    return mpc_decide_host_impl(h_sizes, h_bitrates, V, A, params, N, h_chunk_idx, h_prev_q, h_buffer, h_bw_hist,
-                                h_hist_len, K, h_last_pred, h_err_ring, h_err_len, horizon, mode, flags, nullptr, 1, 0.0,
-                                h_action, nullptr, h_best_j, h_best_seq, h_preds, h_error_count);
+    MpcArgs a{};
+    a.sizes = h_sizes; a.V = V; a.A = A; a.N = N; a.K = K; a.H = horizon; a.mode = mode; a.flags = flags;
+    a.chunk_idx = h_chunk_idx; a.prev_q = h_prev_q; a.buffer = h_buffer; a.bw_hist = h_bw_hist; a.hist_len = h_hist_len;
+    a.last_pred = h_last_pred; a.err_ring = h_err_ring; a.err_len = h_err_len;
+    a.action = h_action; a.best_j = h_best_j; a.best_seq = h_best_seq; a.preds = h_preds; a.error_count32 = h_error_count;
+    return mpc_decide_host(a, h_bitrates, params);
 }
 
 int abr_mpc_decide_startup_host(const double* h_sizes, const double* h_bitrates, int V, int A, const AbrParams* params,
@@ -991,20 +960,21 @@ int abr_mpc_decide_startup_host(const double* h_sizes, const double* h_bitrates,
                                 double* h_startup_delay, double* h_best_j, int32_t* h_best_seq, double* h_preds,
                                 int32_t* h_error_count) {
     if (!h_startup_delay) return fail(ABR_ERR_INVALID, "startup_delay is NULL");
-    return mpc_decide_host_impl(h_sizes, h_bitrates, V, A, params, N, h_chunk_idx, h_prev_q, h_buffer, h_bw_hist,
-                                h_hist_len, K, h_last_pred, h_err_ring, h_err_len, horizon, mode, flags, h_startup, n_ts,
-                                ts_step, h_action, h_startup_delay, h_best_j, h_best_seq, h_preds, h_error_count);
+    MpcArgs a{};
+    a.sizes = h_sizes; a.V = V; a.A = A; a.N = N; a.K = K; a.H = horizon; a.mode = mode; a.flags = flags;
+    a.chunk_idx = h_chunk_idx; a.prev_q = h_prev_q; a.buffer = h_buffer; a.bw_hist = h_bw_hist; a.hist_len = h_hist_len;
+    a.last_pred = h_last_pred; a.err_ring = h_err_ring; a.err_len = h_err_len;
+    a.action = h_action; a.best_j = h_best_j; a.best_seq = h_best_seq; a.preds = h_preds; a.error_count32 = h_error_count;
+    a.startup = h_startup; a.n_ts = n_ts; a.ts_step = ts_step; a.startup_delay = h_startup_delay;
+    return mpc_decide_host(a, h_bitrates, params);
 }
 
 int abr_mpc_score_host(const double* h_sizes, const double* h_bitrates, int V, int A, const AbrParams* params,
                        int chunk_idx, int prev_q, double buffer, const double* h_history, int n_history, int horizon,
                        int mode, double max_err, const int32_t* h_sequences, int M, double* h_scores) {
     if (!h_history || !h_sequences || !h_scores) return fail(ABR_ERR_INVALID, "a required pointer is NULL");
-    int rc = check_tables(h_sizes, h_bitrates, V, A);
-    if (rc) return rc;
-    if (!params) return fail(ABR_ERR_INVALID, "params is NULL");
-    rc = check_mpc_shape(A, horizon);
-    if (rc) return rc;
+    if (int rc = check_host_tables(h_sizes, h_bitrates, V, A, params)) return rc;
+    if (int rc = check_mpc_shape(A, horizon)) return rc;
     if (mode != ABR_MPC_REF && mode != ABR_MPC_ROBUST) return fail(ABR_ERR_INVALID, "unknown MPC mode %d", mode);
     if (M < 0) return fail(ABR_ERR_RANGE, "M must be >= 0");
     if (n_history < 1) return fail(ABR_ERR_RANGE, "empty throughput history (ZeroDivisionError in mpc.py:90)");
@@ -1014,11 +984,7 @@ int abr_mpc_score_host(const double* h_sizes, const double* h_bitrates, int V, i
     if (prev_q >= A) return fail(ABR_ERR_RANGE, "prev_q out of range");
     for (size_t i = 0; i < (size_t)M * horizon; ++i)
         if (h_sequences[i] < 0 || h_sequences[i] >= A) return fail(ABR_ERR_RANGE, "sequence entry %zu out of range", i);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return fail(ABR_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
-    }
+    if (int rc = require_device()) return rc;
     std::vector<double> util;
     utility_table(h_bitrates, V, A, params, util);
     const size_t m = (size_t)(M > 0 ? M : 1);

@@ -8,7 +8,6 @@ used only for device memory and streams.  There is no CPU fallback.
 """
 from __future__ import annotations
 
-import ctypes as C
 from collections import namedtuple
 
 import numpy as np
@@ -16,7 +15,7 @@ import torch
 
 from . import _lib
 from ._lib import (AbrError, MPC_REF, MPC_ROBUST, NUM_ACC, NUM_STATS, POLICY_BBA, POLICY_BOLA,  # noqa: F401
-                   POLICY_FIXED, POLICY_RANDOM, POLICY_RATE)
+                   POLICY_FIXED, POLICY_RANDOM, POLICY_RATE, _addr)
 from .datamodel import MPD, NetworkInfo, QOEMetric, pack_traces
 
 StepResult = namedtuple("StepResult", "delay sleep buffer rebuffer reward next_sizes end_of_video throughput latency",
@@ -51,14 +50,8 @@ _TYPESTR = {"int32": "<i4", "uint8": "|u1", "float64": "<f8"}
 _ITEMSIZE = {"int32": 4, "uint8": 1, "float64": 8}
 
 
-def _ptr(t):
-    if t is None:
-        return None
-    return C.c_void_p(t.data_ptr())
-
-
 def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    return torch.cuda.current_stream().cuda_stream
 
 
 class _OnDevice:
@@ -131,16 +124,6 @@ def _check_host_out(a, size, name):
         raise TypeError(f"output {name!r} must be a contiguous host float64 buffer of {size} elements")
 
 
-def _hptr(a):
-    if a is None:
-        return None
-    return a.data_ptr() if isinstance(a, torch.Tensor) else a.ctypes.data
-
-
-def _hptr_dev(t):
-    return None if t is None else t.data_ptr()
-
-
 def _out_dtype(t, dtype):
     """float64 or float32: the dtype of a caller-given output tensor, else the requested one."""
     d = dtype if t is None else t.dtype
@@ -188,13 +171,12 @@ class BatchedABREnv:
         self.n = 0
         self.perm = None          # installed session order (set_order), environment position -> caller's index
         self._inv_perm = None
-        self._h = C.c_void_p()
+        self._h = None
+        h = np.zeros(1, np.uintp)
         with self._on:
-            _lib.check(self._lib.abr_env_create(
-                bw.ctypes.data_as(C.c_void_p), tl.ctypes.data_as(C.c_void_p), ti.ctypes.data_as(C.c_void_p),
-                C.c_int(self.n_traces), C.c_int(self.T_max), sz.ctypes.data_as(C.c_void_p),
-                br.ctypes.data_as(C.c_void_p), C.c_int(self.V), C.c_int(self.A), C.byref(self.params),
-                C.c_int(self.capacity), C.byref(self._h)))
+            _lib.check(self._lib.abr_env_create(_addr(bw), _addr(tl), _addr(ti), self.n_traces, self.T_max, _addr(sz),
+                                                _addr(br), self.V, self.A, self.params, self.capacity, _addr(h)))
+        self._h = int(h[0])
         self._stats = torch.empty(NUM_STATS, dtype=torch.float64, device=self.device)
 
     # -- construction from the reference's objects (Simulator.set_network_info / set_mpd / set_qoe_metric) --
@@ -247,8 +229,7 @@ class BatchedABREnv:
         tid = self._dev(trace_id, torch.int32)
         perm = self._empty(tid.numel(), dtype=torch.int32)
         with self._on:
-            _lib.check(self._lib.abr_sort_by_trace(_ptr(tid), C.c_int(tid.numel()), C.c_int(self.n_traces), _ptr(perm),
-                                                   _stream()))
+            _lib.check(self._lib.abr_sort_by_trace(_addr(tid), tid.numel(), self.n_traces, _addr(perm), _stream()))
         return perm
 
     def set_order(self, perm):
@@ -258,8 +239,8 @@ class BatchedABREnv:
         self.perm = None if perm is None else self._dev(perm, torch.int32)
         self._inv_perm = None
         with self._on:
-            _lib.check(self._lib.abr_env_set_order(self._h, _ptr(self.perm),
-                                                   C.c_int(0 if self.perm is None else self.perm.numel()), _stream()))
+            _lib.check(self._lib.abr_env_set_order(self._h, _addr(self.perm),
+                                                   0 if self.perm is None else self.perm.numel(), _stream()))
 
     def to_env_order(self, x):
         """Caller-order array(s) [..., N] -> environment order (identity without an installed order)."""
@@ -286,15 +267,13 @@ class BatchedABREnv:
             raise ValueError("start_offset must have one entry per session")
         if sort_by_trace:      # one call: counting sort by trace + gather of the inputs + reset (abr_env_reset_sorted)
             with self._on:
-                _lib.check(self._lib.abr_env_reset_sorted(self._h, _ptr(tid), _ptr(off), C.c_int(n),
-                                                          C.c_longlong(session_base), _stream()))
+                _lib.check(self._lib.abr_env_reset_sorted(self._h, _addr(tid), _addr(off), n, session_base, _stream()))
             self.n = n
             self.session_base = int(session_base)
             self.perm, self._inv_perm = self.state("order"), None    # a view of the environment's own copy
             return
         with self._on:
-            _lib.check(self._lib.abr_env_reset(self._h, _ptr(tid), _ptr(off), C.c_int(n), C.c_longlong(session_base),
-                                               _stream()))
+            _lib.check(self._lib.abr_env_reset(self._h, _addr(tid), _addr(off), n, session_base, _stream()))
         self.n = n
         self.session_base = int(session_base)
 
@@ -328,9 +307,9 @@ class BatchedABREnv:
         fn = self._lib.abr_env_step_live if _out_dtype(out.delay, dtype) == torch.float64 else self._lib.abr_env_step_f32
         with self._on:
             _lib.check(fn(
-                self._h, _ptr(a), _ptr(v), _ptr(out.delay), _ptr(out.sleep), _ptr(out.buffer), _ptr(out.rebuffer),
-                _ptr(out.reward), _ptr(out.latency), _ptr(out.next_sizes), _ptr(out.end_of_video),
-                _ptr(out.throughput), _stream()))
+                self._h, _addr(a), _addr(v), _addr(out.delay), _addr(out.sleep), _addr(out.buffer), _addr(out.rebuffer),
+                _addr(out.reward), _addr(out.latency), _addr(out.next_sizes), _addr(out.end_of_video),
+                _addr(out.throughput), _stream()))
         return out
 
     # -- SPEC §4.1: policy in the loop (RL harness) --
@@ -363,12 +342,12 @@ class BatchedABREnv:
             chk(getattr(o, name), torch.float64, n, name)
         if o is not None:
             chk(o.end_of_video, torch.uint8, n, "end_of_video")
-        g = (lambda name: _hptr_dev(getattr(o, name))) if o is not None else (lambda name: None)
+        g = (lambda name: _addr(getattr(o, name))) if o is not None else (lambda name: None)
         with self._on:
             _lib.check(self._lib.abr_env_step_policy(
-                self._h, logits.data_ptr(), int(bool(sample)), int(seed), C.addressof(spec), _hptr_dev(obs),
-                _hptr_dev(action_out), _hptr_dev(reward_sum), g("delay"), g("sleep"), g("buffer"), g("rebuffer"),
-                g("reward"), g("end_of_video"), torch.cuda.current_stream().cuda_stream))
+                self._h, _addr(logits), int(bool(sample)), int(seed), spec, _addr(obs),
+                _addr(action_out), _addr(reward_sum), g("delay"), g("sleep"), g("buffer"), g("rebuffer"),
+                g("reward"), g("end_of_video"), _stream()))
         return obs
 
     # -- SPEC §3+§4 --
@@ -405,9 +384,9 @@ class BatchedABREnv:
         fn = self._lib.abr_env_rollout_fused_f32 if f32 else self._lib.abr_env_rollout_fused_live
         with self._on:
             _lib.check(fn(
-                self._h, C.c_int(pid), C.c_uint64(seed), C.c_int(steps), _ptr(a_in), _ptr(v), _ptr(out.get("delay")),
-                _ptr(out.get("sleep")), _ptr(out.get("buffer")), _ptr(out.get("rebuffer")), _ptr(out.get("reward")),
-                _ptr(out.get("latency")), _ptr(out.get("end_of_video")), _ptr(out.get("actions")), _stream()))
+                self._h, pid, seed, steps, _addr(a_in), _addr(v), _addr(out.get("delay")), _addr(out.get("sleep")),
+                _addr(out.get("buffer")), _addr(out.get("rebuffer")), _addr(out.get("reward")), _addr(out.get("latency")),
+                _addr(out.get("end_of_video")), _addr(out.get("actions")), _stream()))
         return out
 
     # -- SPEC §2+§3+§4+§6 in one launch --
@@ -444,10 +423,9 @@ class BatchedABREnv:
         g = out.get
         with self._on:
             _lib.check(self._lib.abr_env_run(
-                self._h, C.c_int(pid), C.c_uint64(seed), C.c_int(steps), _ptr(tid), _ptr(off), C.c_int(n),
-                C.c_longlong(session_base), _ptr(a_in), _ptr(g("delay")), _ptr(g("sleep")), _ptr(g("buffer")),
-                _ptr(g("rebuffer")), _ptr(g("reward")), _ptr(g("end_of_video")), _ptr(g("actions")), _ptr(qoe_cost),
-                _ptr(stats), _stream()))
+                self._h, pid, seed, steps, _addr(tid), _addr(off), n, session_base, _addr(a_in), _addr(g("delay")),
+                _addr(g("sleep")), _addr(g("buffer")), _addr(g("rebuffer")), _addr(g("reward")),
+                _addr(g("end_of_video")), _addr(g("actions")), _addr(qoe_cost), _addr(stats), _stream()))
         self.n = n
         self.session_base = int(session_base)
         return out, qoe_cost, stats
@@ -459,11 +437,11 @@ class BatchedABREnv:
         cur = getattr(self, "_policy_params", None)
         if cur is None:
             cur = _lib.AbrPolicyParams()
-            self._lib.abr_policy_params_default(C.byref(cur))
+            self._lib.abr_policy_params_default(cur)
         pp = _lib.AbrPolicyParams(cur.rb_safety if rb_safety is None else float(rb_safety),
                                   cur.bola_min_buffer if bola_min_buffer is None else float(bola_min_buffer),
                                   cur.bola_target_buffer if bola_target_buffer is None else float(bola_target_buffer))
-        _lib.check(self._lib.abr_env_set_policy_params(self._h, C.byref(pp)))
+        _lib.check(self._lib.abr_env_set_policy_params(self._h, pp))
         self._policy_params = pp
 
     def policy_decide(self, policy, out=None) -> torch.Tensor:
@@ -474,7 +452,7 @@ class BatchedABREnv:
         if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:
             raise TypeError(f"out must be a contiguous int32 tensor of {self.n} elements on {self.device}")
         with self._on:
-            _lib.check(self._lib.abr_env_policy_decide(self._h, C.c_int(pid), _ptr(act), _stream()))
+            _lib.check(self._lib.abr_env_policy_decide(self._h, pid, _addr(act), _stream()))
         return act
 
     # -- SPEC §5 --
@@ -486,8 +464,7 @@ class BatchedABREnv:
         bj = self._empty(self.n) if want_score else None
         mode_id = _mode_id(mode) | (_lib.MPC_MODE_EXHAUSTIVE if exhaustive else 0)
         with self._on:
-            _lib.check(self._lib.abr_env_mpc_decide(self._h, C.c_int(horizon), C.c_int(mode_id), _ptr(act),
-                                                    _ptr(bj), _stream()))
+            _lib.check(self._lib.abr_env_mpc_decide(self._h, horizon, mode_id, _addr(act), _addr(bj), _stream()))
         return (act, bj) if want_score else act
 
     def mpc_episode(self, steps, horizon=5, mode="robust", exhaustive=False):
@@ -496,7 +473,7 @@ class BatchedABREnv:
         for _ in range(steps):
             self.mpc_decide(horizon, mode, out=act, exhaustive=exhaustive)
             with self._on:
-                _lib.check(self._lib.abr_env_step(self._h, _ptr(act), None, None, None, None, None, None, None, None,
+                _lib.check(self._lib.abr_env_step(self._h, _addr(act), None, None, None, None, None, None, None, None,
                                                   _stream()))   # live mode: speed 1.0
         return act
 
@@ -506,14 +483,14 @@ class BatchedABREnv:
         Σcontent played] (the last three are live-mode sums, SPEC §7)."""
         out = torch.empty(NUM_STATS, dtype=torch.float64, device=self.device)
         with self._on:
-            _lib.check(self._lib.abr_stats_partial(self._h, _ptr(out), _stream()))
+            _lib.check(self._lib.abr_stats_partial(self._h, _addr(out), _stream()))
         return out
 
     def state(self, name) -> torch.Tensor:
         """Zero-copy view of a state field (library-owned device memory)."""
         fid, dt = _lib.FIELDS[name]
-        p = C.c_void_p()
-        _lib.check(self._lib.abr_env_state_ptr(self._h, C.c_int(fid), C.byref(p)))
+        p = np.zeros(1, np.uintp)
+        _lib.check(self._lib.abr_env_state_ptr(self._h, fid, _addr(p)))
         cap = self.capacity
         if name in ("bw_hist", "err_ring"):
             shape = (self.K, cap)
@@ -525,7 +502,7 @@ class BatchedABREnv:
             shape = (self.n_traces, self.T_max)
         else:
             shape = (cap,)
-        t = torch.as_tensor(_DevPtr(p.value, shape, _TYPESTR[dt]), device=self.device)
+        t = torch.as_tensor(_DevPtr(p[0], shape, _TYPESTR[dt]), device=self.device)
         if name in ("bw_hist", "err_ring", "acc"):
             return t[:, :self.n]
         if name in ("sizes", "utility", "trace_bw"):
@@ -541,14 +518,14 @@ class BatchedABREnv:
         """Per-session cost of ``Simulator.calculate_qoe`` (Simulator.py:83-86) from the accumulators, on the device."""
         out = self._empty(self.n)
         with self._on:
-            _lib.check(self._lib.abr_env_qoe_cost(self._h, _ptr(out), _stream()))
+            _lib.check(self._lib.abr_env_qoe_cost(self._h, _addr(out), _stream()))
         return out
 
     def error_count(self) -> int:
-        out = C.c_longlong(0)
+        out = np.zeros(1, np.int64)
         with self._on:
-            _lib.check(self._lib.abr_env_error_count(self._h, C.byref(out), _stream()))
-        return int(out.value)
+            _lib.check(self._lib.abr_env_error_count(self._h, _addr(out), _stream()))
+        return int(out[0])
 
     # -- host-buffer path (what Simulator.run() uses; e2e benchmark leg) --
     def run_host(self, policy, steps, trace_id, start_offset=None, seed=0, session_base=0, actions=None,
@@ -583,11 +560,11 @@ class BatchedABREnv:
         g = out.get
         for k, size in (("acc", NUM_ACC * n), ("stats", NUM_STATS), ("reward", steps * n), ("qoe_cost", n)):
             _check_host_out(g(k), size, k)
-        args = [self._h, pid, seed, steps, _hptr(tid), _hptr(off), n, session_base, _hptr(a_in),
-                _hptr(g("acc")), _hptr(g("stats")), _hptr(g("reward")), _hptr(g("qoe_cost")), None]
+        args = [self._h, pid, seed, steps, _addr(tid), _addr(off), n, session_base, _addr(a_in),
+                _addr(g("acc")), _addr(g("stats")), _addr(g("reward")), _addr(g("qoe_cost")), None]
         if _prepare:
             return HostRun(self, args, out, (tid, off, a_in))
-        args[13] = torch.cuda.current_stream().cuda_stream
+        args[13] = _stream()
         with self._on:
             rc = self._run_host(*args)
         if rc:

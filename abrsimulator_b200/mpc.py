@@ -17,17 +17,12 @@ Every decision runs on the GPU; there is no CPU fallback.
 """
 from __future__ import annotations
 
-import ctypes as C
 import itertools
 
 import numpy as np
 
 from . import _lib
-from ._lib import MPC_REF, MPC_ROBUST, MPC_PRED_SES
-
-
-def _hp(a):
-    return None if a is None else a.ctypes.data_as(C.c_void_p)
+from ._lib import MPC_REF, MPC_ROBUST, MPC_PRED_SES, _addr
 
 
 class MPCBitrateController:
@@ -126,18 +121,19 @@ class MPCBitrateController:
         nerr = np.zeros(1, np.int32)
         robust = self.mode == MPC_ROBUST
         flags = MPC_PRED_SES if ses else 0
-        head = (_hp(sizes), _hp(bitrates), C.c_int(V), C.c_int(A), C.byref(p), C.c_int(1),
-                _hp(np.array([chunk], np.int32)), _hp(np.array([prev_q], np.int32)),
-                _hp(np.array([buffer_level], np.float64)), _hp(ring), _hp(np.array([hl], np.int32)), C.c_int(K),
-                _hp(self._last_pred) if robust else None, _hp(self._err_ring) if robust else None,
-                _hp(self._err_len) if robust else None, C.c_int(horizon), C.c_int(self.mode), C.c_int(flags))
+        # named: only their addresses are passed, so they must outlive the call
+        chunk_a, prev_a = np.array([chunk], np.int32), np.array([prev_q], np.int32)
+        buffer_a, hl_a = np.array([buffer_level], np.float64), np.array([hl], np.int32)
+        head = (_addr(sizes), _addr(bitrates), V, A, p, 1, _addr(chunk_a), _addr(prev_a), _addr(buffer_a), _addr(ring),
+                _addr(hl_a), K, _addr(self._last_pred) if robust else None, _addr(self._err_ring) if robust else None,
+                _addr(self._err_len) if robust else None, horizon, self.mode, flags)
         ts = np.zeros(1)
         if startup_grid is None:
-            _lib.check(lib.abr_mpc_decide_host(*head, _hp(act), _hp(bj), _hp(seq), _hp(preds), _hp(nerr)))
+            _lib.check(lib.abr_mpc_decide_host(*head, _addr(act), _addr(bj), _addr(seq), _addr(preds), _addr(nerr)))
         else:
             n_ts, ts_step = startup_grid
-            _lib.check(lib.abr_mpc_decide_startup_host(*head, None, C.c_int(int(n_ts)), C.c_double(float(ts_step)),
-                                                       _hp(act), _hp(ts), _hp(bj), _hp(seq), _hp(preds), _hp(nerr)))
+            _lib.check(lib.abr_mpc_decide_startup_host(*head, None, int(n_ts), float(ts_step), _addr(act), _addr(ts),
+                                                       _addr(bj), _addr(seq), _addr(preds), _addr(nerr)))
         if nerr[0] != 0 or act[0] < 0:
             raise ValueError("invalid MPC input (previous bitrate index out of range, or a non-positive prediction?)")
         if startup_grid is not None:
@@ -296,11 +292,9 @@ class MPCBitrateController:
             prev = chunk_info.previous_bitrates[-1]
         scores = np.empty(M)
         p = self._params()
-        _lib.check(lib.abr_mpc_score_host(_hp(sizes), _hp(bitrates), C.c_int(V), C.c_int(A), C.byref(p),
-                                          C.c_int(int(chunk)), C.c_int(int(prev)),
-                                          C.c_double(float(chunk_info.buffer_level)), _hp(hist), C.c_int(hist.size),
-                                          C.c_int(H), C.c_int(self.mode), C.c_double(0.0), _hp(seqs), C.c_int(M),
-                                          _hp(scores)))
+        _lib.check(lib.abr_mpc_score_host(_addr(sizes), _addr(bitrates), V, A, p, int(chunk), int(prev),
+                                          float(chunk_info.buffer_level), _addr(hist), hist.size, H, self.mode, 0.0,
+                                          _addr(seqs), M, _addr(scores)))
         return scores
 
     def score_grid(self, chunk_info):
@@ -321,7 +315,7 @@ def decide_batch(sizes, utility, chunk_idx, prev_q, buffer, bw_hist, hist_len, h
     sessions with ``startup`` != 0 ([N] uint8, None = all); the result then carries ``startup_delay`` [N].
     """
     import torch
-    from .env import _ptr, _stream, _mode_id
+    from .env import _stream, _mode_id
     lib = _lib.load()
     V, A = sizes.shape
     N, K = bw_hist.shape
@@ -338,17 +332,16 @@ def decide_batch(sizes, utility, chunk_idx, prev_q, buffer, bw_hist, hist_len, h
     for t in (sizes, utility, chunk_idx, prev_q, buffer, bw_hist, hist_len):
         if not t.is_contiguous():
             raise ValueError("tensors must be contiguous")
-    head = (_ptr(sizes), _ptr(utility), C.c_int(V), C.c_int(A), C.byref(p), C.c_int(N), _ptr(chunk_idx), _ptr(prev_q),
-            _ptr(buffer), _ptr(bw_hist), _ptr(hist_len), C.c_int(K), _ptr(last_pred), _ptr(err_ring), _ptr(err_len),
-            C.c_int(horizon), C.c_int(_mode_id(mode)), C.c_int(flags))
-    tail = (_ptr(out.get("best_j")), _ptr(out.get("best_seq")), _ptr(out.get("preds")), _ptr(out["errors"]), _stream())
+    head = (_addr(sizes), _addr(utility), V, A, p, N, _addr(chunk_idx), _addr(prev_q), _addr(buffer), _addr(bw_hist),
+            _addr(hist_len), K, _addr(last_pred), _addr(err_ring), _addr(err_len), horizon, _mode_id(mode), flags)
+    tail = (_addr(out.get("best_j")), _addr(out.get("best_seq")), _addr(out.get("preds")), _addr(out["errors"]), _stream())
     with torch.cuda.device(dev):
         if n_ts > 1:
             out["startup_delay"] = torch.empty(N, dtype=torch.float64, device=dev)
             if startup is not None and (startup.dtype != torch.uint8 or not startup.is_contiguous() or startup.numel() != N):
                 raise ValueError("startup must be a contiguous uint8 tensor [N]")
-            _lib.check(lib.abr_mpc_decide_startup(*head, _ptr(startup), C.c_int(int(n_ts)), C.c_double(float(ts_step)),
-                                                  _ptr(out["action"]), _ptr(out["startup_delay"]), *tail))
+            _lib.check(lib.abr_mpc_decide_startup(*head, _addr(startup), int(n_ts), float(ts_step), _addr(out["action"]),
+                                                  _addr(out["startup_delay"]), *tail))
         else:
-            _lib.check(lib.abr_mpc_decide(*head, _ptr(out["action"]), *tail))
+            _lib.check(lib.abr_mpc_decide(*head, _addr(out["action"]), *tail))
     return out
