@@ -97,6 +97,10 @@ SIGNATURES = {
     "abr_fp64_probe": (_I, [_I, _I, _P, _P, _P]),
 }
 SYMBOLS = tuple(SIGNATURES)
+# Entry points declared in the companion headers of abr_b200.h (include/abr_b200_lookahead.h), bound the same way.
+EXTRA_SIGNATURES = {
+    "abr_env_lookahead_decide": (_I, [_P, _I, _P, _P, _P, _P]),
+}
 
 _lib = None
 
@@ -116,7 +120,7 @@ def load():
         # under a file lock: concurrent ranks build once, the rest wait and load the finished file
         _build.build_library()
     lib = C.CDLL(path)
-    for name, (restype, argtypes) in SIGNATURES.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "abr_common.cuh"
+#include "../../include/abr_b200_lookahead.h"
 
 namespace abr {
 static std::atomic<long long> g_launches{0};
@@ -646,6 +647,21 @@ int abr_env_mpc_decide(AbrEnv* env, int horizon, int mode, int32_t* d_action, do
     a.action = d_action; a.best_j = d_best_j; a.best_seq = nullptr; a.preds = nullptr;
     a.error_count64 = v.errors; a.error_count32 = nullptr;
     CUDA_TRY(launch_mpc(a, (cudaStream_t)stream));
+    return ABR_OK;
+}
+
+int abr_env_lookahead_decide(AbrEnv* env, int horizon, int32_t* d_action, double* d_best_value, int32_t* d_best_seq,
+                             void* stream) {
+    if (int rc = check_reset(env)) return rc;
+    if (env->v.p.live) return fail(ABR_ERR_STATE, "abr_env_lookahead_decide is not available in live mode (SPEC 7)");
+    if (env->v.n == 0) return ABR_OK;
+    if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
+    if (horizon < 1 || horizon > 8) return fail(ABR_ERR_RANGE, "horizon must be in [1, 8] (got %d)", horizon);
+    double combos = 1;
+    for (int i = 0; i < horizon; ++i) combos *= env->v.A;
+    if (combos > 1048576.0)
+        return fail(ABR_ERR_RANGE, "A^horizon = %g sequences exceed the lookahead limit of 2^20 = 1048576", combos);
+    CUDA_TRY(launch_lookahead(env->v, horizon, d_action, d_best_value, d_best_seq, (cudaStream_t)stream));
     return ABR_OK;
 }
 

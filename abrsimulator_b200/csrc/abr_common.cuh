@@ -187,6 +187,11 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
                            double* d_block_partials, const RolloutFused& f, cudaStream_t st);
 // abr_env_policy_decide: the action of policy BBA / RATE / BOLA for every session from the SoA state
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st);
+// abr_env_lookahead_decide (SPEC §4.4): the clairvoyant best sequence over the next min(H, V - chunk) chunks against
+// every session's own trace, H in [1, 8]; d_best_value [N] and d_best_seq [N][H] nullable.  Writes nothing else but
+// the error counter.
+cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double* d_best_value, int32_t* d_best_seq,
+                             cudaStream_t st);
 cudaError_t launch_stats(const EnvView& v, double* d_partials, int n_partials, bool have_partials, double* d_out,
                          const StatsScratch& scratch,
                          cudaStream_t st);

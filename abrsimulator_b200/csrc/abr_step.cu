@@ -1588,7 +1588,111 @@ abr_policy_decide_kernel(EnvView v, int32_t* __restrict__ action) {
     action[i] = q;
 }
 
+// ---- SPEC §4.4: clairvoyant lookahead (abr_env_lookahead_decide) ----
+// One thread per (session, first action a0); the A threads of a session sit in consecutive lanes of one warp
+// (32 / A sessions per warp, the remaining lanes idle).  A thread walks the A^(h-1) completions of its a0 depth first
+// in C order, stepping a register copy of the session with the per-step kernel's own step_core; the states before
+// steps 1 .. h-1 and the partial sums wait on a per-thread stack, so every node of the tree is stepped once.  The
+// lane of a0 = 0 then scans the A lane results in a0 order with the same strict > as each lane's own scan, which is
+// the first maximum of SPEC §4.4 over the whole tree.
+constexpr int kLookaheadBlock = 128;
+constexpr int kLookaheadMaxH = 8;
+
+struct LookNode { double phi, pos, buffer, J; int seg; };   // a session's state before a step, and the sum so far
+
+// FAST: auto_reset is on, so that no session is inert (the step drops the done bookkeeping)
+template <bool FAST>
+__global__ void __launch_bounds__(kLookaheadBlock)
+abr_lookahead_kernel(EnvView v, const int H, int32_t* __restrict__ action, double* __restrict__ best_value,
+                     int32_t* __restrict__ best_seq) {
+    __shared__ double s_val[kLookaheadBlock];
+    __shared__ int s_leaf[kLookaheadBlock];
+    __shared__ int s_err[kLookaheadBlock];
+    const int A = v.A;
+    const int per_warp = 32 / A;
+    const int lane = threadIdx.x & 31;
+    const int g = lane / A, a0 = lane - g * A;
+    const int i = (int)((blockIdx.x * (kLookaheadBlock / 32) + (threadIdx.x >> 5)) * per_warp) + g;
+    const bool active = g < per_warp && i < v.n;
+    double best = 0.0;
+    int best_leaf = 0, h = 0, n_leaves = 1;
+    bool err = false;
+    if (active) {
+        Sess s;
+        load_sess(v, i, s);
+        h = s.done ? 0 : min(H, v.V - s.chunk);
+        ABR_CHECK(h <= kLookaheadMaxH && s.chunk >= 0, "lookahead depth");
+        for (int d = 1; d < h; ++d) n_leaves *= A;
+        if (h > 0) {
+            const bool prev_ladder = v.p.smooth_prev_ladder != 0;
+            const int chunk0 = s.chunk, hist0 = s.hist_len;
+            LookNode st[kLookaheadMaxH];   // st[d]: the state before step d (d >= 1)
+            int dig[kLookaheadMaxH];       // the sequence of the current leaf
+            dig[0] = a0;
+            for (int d = 1; d < h; ++d) dig[d] = 0;
+            int k = 0, leaf = 0;
+            double J = 0.0;
+            for (;;) {
+                for (int d = k; d < h; ++d) {
+                    const int q = dig[d];
+                    const Lookup lk = lookup_tables<false>(s, A, v.V, s.chunk, q, s.last_q, prev_ladder);
+                    StepRes r;
+                    step_core<false, FAST, false>(v, s, q, lk, r, false);
+                    err |= r.walk_error;
+                    J = dadd(J, r.reward);
+                    if (d + 1 < h) {
+                        LookNode& nd = st[d + 1];
+                        nd.phi = s.phi; nd.pos = s.pos; nd.buffer = s.buffer; nd.J = J; nd.seg = s.seg;
+                    }
+                }
+                if (leaf == 0 || J > best) { best = J; best_leaf = leaf; }
+                int d = h - 1;   // the next leaf in C order: the deepest digit that can still grow
+                while (d >= 1 && dig[d] == A - 1) dig[d--] = 0;
+                if (d < 1) break;
+                ++dig[d];
+                ++leaf;
+                k = d;
+                const LookNode& nd = st[k];
+                s.phi = nd.phi; s.pos = nd.pos; s.buffer = nd.buffer; J = nd.J; s.seg = nd.seg;
+                s.chunk = chunk0 + k; s.last_q = dig[k - 1]; s.hist_len = hist0 + k; s.done = false;
+            }
+        }
+    }
+    s_val[threadIdx.x] = best;
+    s_leaf[threadIdx.x] = a0 * n_leaves + best_leaf;
+    s_err[threadIdx.x] = err ? 1 : 0;
+    __syncwarp();
+    if (!active || a0 != 0) return;
+    int idx = s_leaf[threadIdx.x], flagged = s_err[threadIdx.x];
+    for (int a = 1; a < A; ++a) {
+        const double x = s_val[threadIdx.x + a];
+        if (x > best) { best = x; idx = s_leaf[threadIdx.x + a]; }
+        flagged |= s_err[threadIdx.x + a];
+    }
+    if (flagged) atomicAdd(v.errors, 1ull);
+    if (h == 0) best = 0.0;
+    action[i] = h > 0 ? idx / n_leaves : 0;
+    if (best_value) best_value[i] = best;
+    if (best_seq) {
+        int32_t* row = best_seq + (size_t)i * H;
+        for (int d = H - 1; d >= h; --d) row[d] = -1;
+        for (int d = h - 1; d >= 0; --d) { row[d] = idx % A; idx /= A; }
+    }
+}
+
 }  // namespace
+
+cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double* d_best_value, int32_t* d_best_seq,
+                             cudaStream_t st) {
+    if (v.n == 0) return cudaSuccess;
+    if (H < 1 || H > kLookaheadMaxH || v.A < 1 || v.A > 32) return cudaErrorInvalidValue;
+    const int per_block = (kLookaheadBlock / 32) * (32 / v.A);
+    const unsigned grid = (unsigned)((v.n + per_block - 1) / per_block);
+    if (v.p.auto_reset) abr_lookahead_kernel<true><<<grid, kLookaheadBlock, 0, st>>>(v, H, d_action, d_best_value, d_best_seq);
+    else abr_lookahead_kernel<false><<<grid, kLookaheadBlock, 0, st>>>(v, H, d_action, d_best_value, d_best_seq);
+    count_launch();
+    return cudaGetLastError();
+}
 
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;

@@ -477,6 +477,35 @@ class BatchedABREnv:
                                                   _stream()))   # live mode: speed 1.0
         return act
 
+    # -- SPEC §4.4 --
+    def lookahead_decide(self, horizon=5, want_value=False, want_seq=False, out=None):
+        """Clairvoyant lookahead (SPEC §4.4): for every session, the first action of the bitrate sequence over the next
+        min(horizon, V - chunk) chunks with the largest sum of the environment's own rewards against the session's
+        actual future trace.  An upper reference that sees the future, not a deployable controller; the state does
+        not change.  Returns the int32 [N] actions, or a tuple with the float64 [N] best values and / or the int32
+        [N, horizon] best sequences (-1 past the end of the video).  Not available in live mode."""
+        act = self._empty(self.n, dtype=torch.int32) if out is None else out
+        if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:
+            raise TypeError(f"out must be a contiguous int32 tensor of {self.n} elements on {self.device}")
+        val = self._empty(self.n) if want_value else None
+        seq = self._empty(self.n, int(horizon), dtype=torch.int32) if want_seq else None
+        with self._on:
+            _lib.check(self._lib.abr_env_lookahead_decide(self._h, horizon, _addr(act), _addr(val), _addr(seq),
+                                                          _stream()))
+        if not (want_value or want_seq):
+            return act
+        return (act,) + ((val,) if want_value else ()) + ((seq,) if want_seq else ())
+
+    def lookahead_episode(self, steps, horizon=5):
+        """lookahead_decide -> step for `steps` chunks (track_acc=1 for the per-session sums)."""
+        act = self._empty(self.n, dtype=torch.int32)
+        for _ in range(steps):
+            self.lookahead_decide(horizon, out=act)
+            with self._on:
+                _lib.check(self._lib.abr_env_step(self._h, _addr(act), None, None, None, None, None, None, None, None,
+                                                  _stream()))
+        return act
+
     # -- SPEC §6 --
     def stats(self) -> torch.Tensor:
         """[Σreward, Σrebuffer, Σutility, Σsmooth, Σsleep, Σdelay, steps, episodes, Σstartup, Σlatency integral,

@@ -22,7 +22,8 @@ Controllers
   (the protocol ``Simulator.run`` calls, ``Simulator.py:155``) is driven chunk by chunk through the step kernel;
 * the markers ``RandomPolicy(seed)`` / ``BufferBasedPolicy()`` / ``RateBasedPolicy()`` / ``BolaPolicy()`` /
   ``FixedPolicy(actions)`` and this package's ``MPCBitrateController`` run fully on the device (fused episode kernel,
-  or decide+step kernels for MPC).
+  or decide+step kernels for MPC);
+* ``LookaheadPolicy(horizon)`` is the clairvoyant reference of SPEC §4.4 (decide+step kernels, on-demand mode only).
 """
 from __future__ import annotations
 
@@ -57,6 +58,14 @@ class BolaPolicy:
     [min_buffer, target_buffer] in seconds."""
     def __init__(self, min_buffer=10.0, target_buffer=30.0):
         self.min_buffer, self.target_buffer = float(min_buffer), float(target_buffer)
+
+
+class LookaheadPolicy:
+    """Clairvoyant lookahead (SPEC §4.4): at every chunk, the first bitrate of the sequence over the next ``horizon``
+    chunks with the largest sum of rewards against the session's actual future trace.  It sees the future: an upper
+    reference to compare controllers against, not a controller a player could run.  Not available in live mode."""
+    def __init__(self, horizon=5):
+        self.horizon = int(horizon)
 
 
 class FixedPolicy:
@@ -165,6 +174,9 @@ class Simulator:
             if trace_id is None else np.asarray(trace_id, np.int32)
         ctrl = self.abr_controller
         q = self.qoe_metric
+        if isinstance(ctrl, LookaheadPolicy) and self._live():
+            raise ValueError("LookaheadPolicy is not available in live mode (SPEC §7): its objective has no playback "
+                             "speeds and no latency term")
         if self._live():
             return self._run_live(n_sessions, tid, start_offset, session_base)
         if isinstance(ctrl, self._MARKERS) or ctrl is None:
@@ -178,6 +190,11 @@ class Simulator:
             env = self._make_env(n_sessions, track_history=1, track_acc=1, **ctrl.extra_params)
             env.reset(tid, start_offset, session_base)
             env.mpc_episode(V, horizon=ctrl.horizon, mode="robust" if ctrl.mode == MPC_ROBUST else "reference")
+            acc = env.session_acc().cpu().numpy()
+        elif isinstance(ctrl, LookaheadPolicy):
+            env = self._make_env(n_sessions, track_acc=1)
+            env.reset(tid, start_offset, session_base)
+            env.lookahead_episode(V, horizon=ctrl.horizon)
             acc = env.session_acc().cpu().numpy()
         else:
             acc = self._run_callback(self._make_env(n_sessions, track_acc=1), n_sessions, tid, start_offset)
