@@ -101,6 +101,10 @@ SYMBOLS = tuple(SIGNATURES)
 EXTRA_SIGNATURES = {
     "abr_env_lookahead_decide": (_I, [_P, _I, _P, _P, _P, _P]),
 }
+# include/abr_b200_mpc_pred.h: MPC over caller-supplied throughput predictions (SPEC §5.6).
+MPC_PRED_SIGNATURES = {
+    "abr_env_mpc_decide_pred": (_I, [_P, _I, _I, _P, _P, _P, _P, _P]),
+}
 
 _lib = None
 
@@ -120,7 +124,7 @@ def load():
         # under a file lock: concurrent ranks build once, the rest wait and load the finished file
         _build.build_library()
     lib = C.CDLL(path)
-    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES}.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -11,6 +11,7 @@
 
 #include "abr_common.cuh"
 #include "../../include/abr_b200_lookahead.h"
+#include "../../include/abr_b200_mpc_pred.h"
 
 namespace abr {
 static std::atomic<long long> g_launches{0};
@@ -646,6 +647,28 @@ int abr_env_mpc_decide(AbrEnv* env, int horizon, int mode, int32_t* d_action, do
     a.H = horizon; a.mode = mode; a.flags = ABR_MPC_TRUNCATE | ABR_MPC_EMPTY_DEFAULT | (exhaustive ? ABR_MPC_EXHAUSTIVE : 0);
     a.action = d_action; a.best_j = d_best_j; a.best_seq = nullptr; a.preds = nullptr;
     a.error_count64 = v.errors; a.error_count32 = nullptr;
+    CUDA_TRY(launch_mpc(a, (cudaStream_t)stream));
+    return ABR_OK;
+}
+
+int abr_env_mpc_decide_pred(AbrEnv* env, int horizon, int flags, const double* d_pred, int32_t* d_action,
+                            double* d_best_j, int32_t* d_best_seq, void* stream) {
+    if (int rc = check_reset(env)) return rc;
+    if (env->v.n == 0) return ABR_OK;
+    if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
+    if (!d_pred) return fail(ABR_ERR_INVALID, "pred is NULL");
+    if (flags != 0 && flags != ABR_MPC_EXHAUSTIVE)
+        return fail(ABR_ERR_INVALID, "flags must be 0 or ABR_MPC_EXHAUSTIVE (got %d)", flags);
+    if (int rc = check_mpc_shape(env->v.A, horizon)) return rc;
+    const EnvView& v = env->v;
+    MpcArgs a{};   // no history ring and no robust state: the kernel reads neither (SPEC §5.6)
+    a.sizes = v.sizes; a.util = v.util; a.V = v.V; a.A = v.A; a.p = v.p; a.N = v.n;
+    a.chunk_idx = v.chunk; a.prev_q = v.last_q; a.buffer = v.buffer; a.done = v.p.auto_reset ? nullptr : v.done;
+    a.K = v.K;
+    a.H = horizon; a.mode = ABR_MPC_ROBUST; a.flags = flags;
+    a.action = d_action; a.best_j = d_best_j; a.best_seq = d_best_seq;
+    a.error_count64 = v.errors;
+    a.pred = d_pred;
     CUDA_TRY(launch_mpc(a, (cudaStream_t)stream));
     return ABR_OK;
 }

@@ -222,6 +222,9 @@ struct MpcArgs {
     unsigned long long* error_count64; int32_t* error_count32; // either may be null
     // start-up phase (SPEC §5.3): sessions with startup[s] != 0 also choose a start-up delay on the grid jt * ts_step
     const uint8_t* startup = nullptr; int n_ts = 1; double ts_step = 0.0; double* startup_delay = nullptr;
+    // caller-supplied predictions (SPEC §5.6): [N][H], p_i of session s at s*H + i; non-null selects the EXT kernels,
+    // which read neither the history ring nor the robust state.  Last, so that every other field keeps its offset.
+    const double* pred = nullptr;
 };
 cudaError_t launch_mpc(const MpcArgs& a, cudaStream_t st);
 cudaError_t launch_mpc_score(const double* d_sizes, const double* d_util, int V, int A, const AbrParams& p, int k,

@@ -462,12 +462,16 @@ struct LiveLists {
 // that each gets its own register allocation.
 // PRUNE (with CLAMP): branch and bound (search / search_compact); decided by the host (robust mode, non-negative
 // penalties, no ABR_MPC_EXHAUSTIVE).  A template parameter so that the enumerating kernel carries none of it.
+// EXT (with CLAMP, SPEC §5.6): the step-i tables divide by the caller's prediction a.pred[s][i] instead of the robust
+// prediction; the history ring and the robust state are neither read nor written.  Everything from the tables on is
+// the robust search: it reads only the per-step tables, and the bounds of branch and bound only U.
 #ifndef ABR_MPC_PRUNE_BLOCKS
 #define ABR_MPC_PRUNE_BLOCKS 5
 #endif
-template <int WPS, int AT, bool CLAMP, bool PRUNE>
+template <int WPS, int AT, bool CLAMP, bool PRUNE, bool EXT = false>
 __global__ void __launch_bounds__(32 * kMpcWarpsPerBlock, PRUNE ? ABR_MPC_PRUNE_BLOCKS : 5)   // <= 96 registers: 20 warps per SM (A/B-tested: 4 -> 5 +3 %, 6 -3 %)
 abr_mpc_kernel(const MpcArgs a) {
+    static_assert(!EXT || CLAMP, "caller predictions use the robust objective");
     constexpr int SPB = kMpcWarpsPerBlock / WPS;
     __shared__ SessShared sh[SPB];
     __shared__ LiveLists<PRUNE> live[SPB];
@@ -488,7 +492,7 @@ abr_mpc_kernel(const MpcArgs a) {
         const int k = a.chunk_idx[s];
         const int prev_q = a.prev_q[s];
         const double buf0 = a.buffer[s];
-        const int hlen = a.hist_len[s];
+        const int hlen = EXT ? 0 : a.hist_len[s];   // EXT: no history (the call works without track_history)
         const int n = hlen < K ? hlen : K;
         const int start = hlen <= K ? 0 : hlen % K;
         const bool inert = a.done && a.done[s];
@@ -497,7 +501,7 @@ abr_mpc_kernel(const MpcArgs a) {
         int act = -1;
         if (inert) { status = 1; act = 0; }
         else if (k < 0 || prev_q >= A) status = 2;
-        else if (n <= 0) {
+        else if (!EXT && n <= 0) {
             if (a.mode == ABR_MPC_ROBUST || (a.flags & ABR_MPC_EMPTY_DEFAULT)) { status = 1; act = p.default_quality > 0 ? p.default_quality : 0; }
             else status = 2;                                               // ZeroDivisionError, mpc.py:90
         }
@@ -508,8 +512,27 @@ abr_mpc_kernel(const MpcArgs a) {
                 if (status == 0 && h <= 0) { status = 1; act = 0; }
             }
         }
+        if constexpr (EXT) {
+            if (status == 0) {
+                // ---- caller predictions (SPEC §5.6): lane i < h reads p_i; one that is not finite and > 0 is an input
+                //      error.  Every warp of the session reads them, so status stays uniform across the session. ----
+                double pv = 1.0;
+                if (lane < h) pv = a.pred[s * H + lane];
+                if (__ballot_sync(0xffffffffu, lane < h && !(pv > 0.0 && pv < __longlong_as_double(0x7ff0000000000000ll))) != 0u)
+                    status = 2;
+                else {
+                    for (int e = tid; e < h * A; e += NT) {   // the robust branch's fill, with p_i for c_rob
+                        ABR_CHECK(e < kMaxH * kMaxA && (k + e / A) < a.V, "lookahead table entry");
+                        const int i = e / A, aa = e - i * A;
+                        const double dl = ddiv(a.sizes[(k + i) * A + aa], a.pred[s * H + i]);
+                        S.RB[e] = dl; S.DL[e] = dl;
+                        S.U[e] = a.util[(k + i) * A + aa];
+                    }
+                }
+            }
+        }
         double c_rob = 0.0;
-        if (status == 0) {
+        if (!EXT && status == 0) {
             // ---- predictor: S = sum of 1/x oldest first (mpc.py:84-88) ----
             double Ssum = 0.0;
             bool bad = false;
@@ -844,15 +867,20 @@ cudaError_t launch_mpc(const MpcArgs& a, cudaStream_t st) {
     const bool clamp = a.mode == ABR_MPC_ROBUST;
     // branch and bound (SPEC §5.5): robust mode, non-negative penalties, unless the caller asks for the enumeration
     const bool prune = clamp && !(a.flags & ABR_MPC_EXHAUSTIVE) && a.p.smooth_penalty >= 0.0 && a.p.rebuf_penalty >= 0.0;
+    const bool ext = a.pred != nullptr;   // caller predictions (SPEC §5.6): robust mode only, checked by the C-ABI
     const unsigned g = (unsigned)blocks, t = 32 * kMpcWarpsPerBlock;
 #define ABR_MPC_LAUNCH(AT_)                                                                        \
     do {                                                                                           \
         if (wps == 1) {                                                                            \
-            if (prune) abr_mpc_kernel<1, AT_, true, true><<<g, t, 0, st>>>(a);                     \
+            if (ext && prune) abr_mpc_kernel<1, AT_, true, true, true><<<g, t, 0, st>>>(a);        \
+            else if (ext) abr_mpc_kernel<1, AT_, true, false, true><<<g, t, 0, st>>>(a);           \
+            else if (prune) abr_mpc_kernel<1, AT_, true, true><<<g, t, 0, st>>>(a);                \
             else if (clamp) abr_mpc_kernel<1, AT_, true, false><<<g, t, 0, st>>>(a);               \
             else abr_mpc_kernel<1, AT_, false, false><<<g, t, 0, st>>>(a);                         \
         } else {                                                                                   \
-            if (prune) abr_mpc_kernel<kMpcWarpsPerBlock, AT_, true, true><<<g, t, 0, st>>>(a);     \
+            if (ext && prune) abr_mpc_kernel<kMpcWarpsPerBlock, AT_, true, true, true><<<g, t, 0, st>>>(a); \
+            else if (ext) abr_mpc_kernel<kMpcWarpsPerBlock, AT_, true, false, true><<<g, t, 0, st>>>(a); \
+            else if (prune) abr_mpc_kernel<kMpcWarpsPerBlock, AT_, true, true><<<g, t, 0, st>>>(a);     \
             else if (clamp) abr_mpc_kernel<kMpcWarpsPerBlock, AT_, true, false><<<g, t, 0, st>>>(a); \
             else abr_mpc_kernel<kMpcWarpsPerBlock, AT_, false, false><<<g, t, 0, st>>>(a);         \
         }                                                                                          \

@@ -477,6 +477,65 @@ class BatchedABREnv:
                                                   _stream()))   # live mode: speed 1.0
         return act
 
+    # -- SPEC §5.6 --
+    def mpc_decide_pred(self, predictions, horizon=5, want_score=False, want_seq=False, out=None, exhaustive=False):
+        """Robust MPC decision (SPEC §5.6) over the caller's throughput predictions instead of the built-in predictor:
+        ``predictions`` is a device tensor [N] (one throughput for every step) or [N, horizon] (step i of session s at
+        [s, i]), float64 or float32 (widened exactly), in environment order.  Only the first min(horizon, V - chunk)
+        entries of a row are read; a session with one that is not finite and > 0 gets action -1 and counts as an
+        error.  Reads no history ring (no track_history needed) and writes no state.  Returns the int32 [N] actions, or
+        a tuple with the float64 [N] objective values J and / or the int32 [N, horizon] best sequences (-1 past the
+        end of the video)."""
+        act = self._empty(self.n, dtype=torch.int32) if out is None else out
+        if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:
+            raise TypeError(f"out must be a contiguous int32 tensor of {self.n} elements on {self.device}")
+        p = predictions
+        if not isinstance(p, torch.Tensor) or p.device != self.device or p.dtype not in (torch.float64, torch.float32):
+            raise TypeError(f"predictions must be a float64 or float32 tensor on {self.device}")
+        H = int(horizon)
+        if p.dim() == 1 and p.shape[0] == self.n:
+            p = p.unsqueeze(1).expand(self.n, H)
+        if tuple(p.shape) != (self.n, H):
+            raise ValueError(f"predictions must be [N] or [N, horizon] = [{self.n}, {H}] (got {tuple(p.shape)})")
+        p = p.to(torch.float64).contiguous()
+        bj = self._empty(self.n) if want_score else None
+        seq = self._empty(self.n, H, dtype=torch.int32) if want_seq else None
+        flags = _lib.MPC_EXHAUSTIVE if exhaustive else 0
+        with self._on:
+            _lib.check(self._lib.abr_env_mpc_decide_pred(self._h, H, flags, _addr(p), _addr(act), _addr(bj),
+                                                         _addr(seq), _stream()))
+        if not (want_score or want_seq):
+            return act
+        return (act,) + ((bj,) if want_score else ()) + ((seq,) if want_seq else ())
+
+    def mpc_episode_pred(self, steps, predictor, horizon=5, exhaustive=False):
+        """``predictor(env)`` -> mpc_decide_pred -> step for `steps` chunks (track_acc=1 for the per-session sums).
+        ``predictor`` returns the [N] or [N, horizon] device predictions for the current state.  Nothing here
+        synchronises with the host, so one chunk can be captured in a CUDA graph when the predictor allows it."""
+        act = self._empty(self.n, dtype=torch.int32)
+        for _ in range(steps):
+            self.mpc_decide_pred(predictor(self), horizon, out=act, exhaustive=exhaustive)
+            with self._on:
+                _lib.check(self._lib.abr_env_step(self._h, _addr(act), None, None, None, None, None, None, None, None,
+                                                  _stream()))   # live mode: speed 1.0
+        return act
+
+    def throughput_history(self):
+        """The throughput samples of every session's history ring, for predictors: ``(x, n)`` with x float64 [N, K]
+        oldest first and NaN past the n[s] = min(hist_len, K) samples a session has (int32 [N]).  Needs
+        track_history=1.  Gathered on the device from the K-major ring, without a host synchronisation."""
+        if not self.params.track_history:
+            raise ValueError("throughput_history needs the throughput history: create the environment with "
+                             "track_history=1")
+        ring, hl = self.state("bw_hist"), self.state("hist_len")      # [K, N] slot-major, [N]
+        K = self.K
+        n = torch.clamp(hl, max=K)
+        start = torch.where(hl <= K, torch.zeros_like(hl), hl % K)  # the oldest sample's slot once the ring wrapped
+        j = torch.arange(K, device=self.device, dtype=hl.dtype)
+        slot = (start[:, None] + j[None, :]) % K
+        x = ring.t().gather(1, slot.long())
+        return torch.where(j[None, :] < n[:, None], x, torch.full_like(x, float("nan"))), n
+
     # -- SPEC §4.4 --
     def lookahead_decide(self, horizon=5, want_value=False, want_seq=False, out=None):
         """Clairvoyant lookahead (SPEC §4.4): for every session, the first action of the bitrate sequence over the next
