@@ -647,7 +647,8 @@ abr_trace_table_kernel(EnvView v, double* __restrict__ cum, uint16_t* __restrict
     }
     for (int j = T + 1; j < cum_stride(v.T_max); ++j) c_row[j] = kInf;
     const bool ok = c > 0.0 && c < kInf && mincap > 0.0;
-    int M = idx_cells(T);
+    // no index rows at all when the longest trace is too long for 16-bit entries: every trace then bisects
+    int M = idx_stride(v.T_max) > 0 ? idx_cells(T) : 0;
     double scale = 0.0;
     if (M > 0 && ok) {
         scale = ddiv((double)M, c);

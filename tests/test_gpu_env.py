@@ -219,7 +219,7 @@ def test_fused_rollout_key_search_with_equal_keys():
 @pytest.mark.parametrize("ragged", [False, True])
 @pytest.mark.parametrize("fast", [False, True])
 def test_step_kernel_shared_memory_trace_path(ragged, fast):
-    """Per-step kernel: a block walks four consecutive tiles of 256 sessions; tiles on one trace use the staged
+    """Per-step kernel: a block walks consecutive tiles of 128 sessions; tiles on one trace use the staged
     capacity row (restaged when the trace changes between tiles), mixed tiles and the partial last tile included."""
     N, steps = 256 * 11 + 100, 30
     bitrates, sizes, bw, tl, ti = small_world(n_traces=9, T=400, ragged=ragged)
