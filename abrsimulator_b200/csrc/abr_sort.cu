@@ -3,8 +3,9 @@
 // follows one trace and takes the shared-memory path whatever order the caller's sessions come in.
 //
 // abr_sort_by_trace builds that order: perm[p] = caller's index of the session at environment position p, a stable
-// (hence deterministic) radix sort of (trace id, session index) pairs.  Set-up code, run once per session->trace
-// assignment; the radix sort itself is CUB's (header-only, part of the CUDA toolkit).
+// (hence deterministic) radix sort of (trace id, session index) pairs, an invalid trace id (< 0 or >= n_traces) keyed
+// as trace 0, the trace the reset puts such a session on.  Set-up code, run once per session->trace assignment; the
+// radix sort itself is CUB's (header-only, part of the CUDA toolkit).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -14,17 +15,23 @@ namespace abr {
 
 namespace {
 
-__global__ void __launch_bounds__(256) abr_iota_kernel(int32_t* __restrict__ out, int n) {
+// The radix sort's pairs: the trace id as the counting sort buckets it (an invalid id as trace 0; the raw id would
+// sort by its low end_bit bits, -1 after every trace) and the session index.
+__global__ void __launch_bounds__(256)
+abr_sort_keys_kernel(const int32_t* __restrict__ tid, int n, int n_traces, int32_t* __restrict__ keys, int32_t* __restrict__ iota) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = i;
+    if (i >= n) return;
+    const int t = tid[i];
+    keys[i] = (t < 0 || t >= n_traces) ? 0 : t;
+    iota[i] = i;
 }
 
 // ---- counting sort by trace, fused with the gather of the reset's inputs (abr_env_reset_sorted) ----
 // The sessions are cut into n_blocks runs of S consecutive sessions.  hist[trace][block] first counts the sessions
 // of each trace in each run, an exclusive scan in that (trace-major) order turns the counts into the first output
 // position of every (trace, run), and one warp per run then walks its sessions in order and places them: stable,
-// hence deterministic — the same order as the radix sort above.  Three small launches instead of CUB's sort, an iota,
-// a copy of the order and two gathers.
+// hence deterministic — the same order as the radix sort above, invalid ids included.  Three small launches instead
+// of CUB's sort, its key pass, a copy of the order and two gathers.
 
 __global__ void __launch_bounds__(256)
 abr_sort_count(const int32_t* __restrict__ tid, int n, int S, int n_traces, int n_blocks, int32_t* __restrict__ hist) {
@@ -174,7 +181,7 @@ cudaError_t launch_sort_gather(const int32_t* d_trace_id, const double* d_off, i
 }
 
 // d_tmp: caller-provided scratch of *tmp_bytes bytes; with d_tmp == nullptr only *tmp_bytes is set (layout:
-// [sorted keys n][iota n][CUB temp storage]).
+// [keys n][sorted keys n][iota n][CUB temp storage]).
 cudaError_t launch_sort_by_trace(const int32_t* d_trace_id, int n, int n_traces, int32_t* d_perm, void* d_tmp,
                                  size_t* tmp_bytes, cudaStream_t st) {
     int end_bit = 1;
@@ -184,13 +191,14 @@ cudaError_t launch_sort_by_trace(const int32_t* d_trace_id, int n, int n_traces,
                                                     (const int32_t*)nullptr, (int32_t*)nullptr, n, 0, end_bit, st);
     if (e != cudaSuccess) return e;
     const size_t arr = ((size_t)n * sizeof(int32_t) + 255) & ~(size_t)255;
-    if (!d_tmp) { *tmp_bytes = 2 * arr + cub_bytes; return cudaSuccess; }
-    int32_t* keys_out = reinterpret_cast<int32_t*>(d_tmp);
-    int32_t* iota = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(d_tmp) + arr);
-    void* cub_tmp = reinterpret_cast<char*>(d_tmp) + 2 * arr;
-    abr_iota_kernel<<<(n + 255) / 256, 256, 0, st>>>(iota, n);
+    if (!d_tmp) { *tmp_bytes = 3 * arr + cub_bytes; return cudaSuccess; }
+    int32_t* keys_in = reinterpret_cast<int32_t*>(d_tmp);
+    int32_t* keys_out = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(d_tmp) + arr);
+    int32_t* iota = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(d_tmp) + 2 * arr);
+    void* cub_tmp = reinterpret_cast<char*>(d_tmp) + 3 * arr;
+    abr_sort_keys_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_trace_id, n, n_traces, keys_in, iota);
     count_launch();
-    e = cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, d_trace_id, keys_out, iota, d_perm, n, 0, end_bit, st);
+    e = cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, keys_in, keys_out, iota, d_perm, n, 0, end_bit, st);
     count_launch(2);
     return e != cudaSuccess ? e : cudaGetLastError();
 }

@@ -113,7 +113,8 @@ int abr_env_num_sessions(const AbrEnv* env);
  * order in which an environment keeps them is free; kept sorted by trace, every thread block of the step kernels follows
  * one trace and stages it in shared memory whatever order the caller's sessions come in.
  * abr_sort_by_trace: d_perm[p] = caller's index of the session at environment position p (stable sort by trace id,
- * deterministic; run once per session->trace assignment).
+ * an invalid id (< 0 or >= n_traces) sorting as trace 0, deterministic; run once per session->trace assignment;
+ * SPEC §8).
  * abr_env_set_order: installs (copies) such an order; NULL removes it.  Every per-session array the caller passes or
  * receives afterwards (trace ids, start offsets, actions, speeds, outputs, state views) is in ENVIRONMENT order, i.e.
  * element p belongs to the caller's session d_perm[p]; the only thing the library does with the order is key the

@@ -1169,7 +1169,7 @@ def test_trace_sorted_order_is_bit_identical_to_the_callers_order():
 @pytest.mark.parametrize("N,n_traces,T", [(70001, 1024, 8), (5000, 13000, 4), (1, 3, 16), (33, 1, 16)])
 def test_reset_sorted_is_the_stable_sort_by_trace(N, n_traces, T):
     """abr_env_reset_sorted (counting sort by trace + gather + reset in one call; CUB's radix sort for the shapes the
-    counting sort does not take: here more than 12 288 traces) installs the order abr_sort_by_trace computes — the
+    counting sort does not take: here more than 11 264 traces) installs the order abr_sort_by_trace computes — the
     stable sort — and resets every session exactly like abr_env_reset on the reordered inputs."""
     bitrates, sizes, bw, tl, ti = small_world(n_traces=n_traces, T=T)
     rng = np.random.default_rng(N)
