@@ -20,7 +20,8 @@ STAMP = LIB + ".srchash"
 SOURCES = ["abr_step.cu", "abr_mpc.cu", "abr_capi.cu", "abr_sort.cu"]
 HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(HERE, "..", "include", "abr_b200.h"),
            os.path.join(HERE, "..", "include", "abr_b200_lookahead.h"),
-           os.path.join(HERE, "..", "include", "abr_b200_mpc_pred.h")]
+           os.path.join(HERE, "..", "include", "abr_b200_mpc_pred.h"),
+           os.path.join(HERE, "..", "include", "abr_b200_obs.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"] + os.environ.get("ABR_EXTRA_NVCC_FLAGS", "").split()

@@ -50,6 +50,12 @@ class AbrObsSpec(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
 
 
+class AbrObsWindowSpec(C.Structure):
+    """The window length and the scales of the windowed observation (SPEC §4.5, include/abr_b200_obs.h)."""
+    _fields_ = [("window", C.c_int32)] + [(n, C.c_double) for n in (
+        "util_scale", "buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
+
+
 # The signature of every symbol include/abr_b200.h declares, in the header's order: (restype, argtypes).  Buffers,
 # streams and the AbrEnv handle are c_void_p; tests check the table against the header and the .so's exports.
 _P, _I, _LL, _U64, _D = C.c_void_p, C.c_int, C.c_longlong, C.c_uint64, C.c_double
@@ -105,6 +111,12 @@ EXTRA_SIGNATURES = {
 MPC_PRED_SIGNATURES = {
     "abr_env_mpc_decide_pred": (_I, [_P, _I, _I, _P, _P, _P, _P, _P]),
 }
+# include/abr_b200_obs.h: the windowed observation of the policy-in-the-loop step (SPEC §4.5).
+_OBS_WINDOW_SPEC = C.POINTER(AbrObsWindowSpec)
+OBS_SIGNATURES = {
+    "abr_env_step_policy_window": (_I, [_P, _P, _I, _U64, _OBS_WINDOW_SPEC] + [_P] * 10),
+    "abr_env_observe_window": (_I, [_P, _OBS_WINDOW_SPEC, _P, _P]),
+}
 
 _lib = None
 
@@ -124,7 +136,7 @@ def load():
         # under a file lock: concurrent ranks build once, the rest wait and load the finished file
         _build.build_library()
     lib = C.CDLL(path)
-    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES}.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -12,6 +12,7 @@
 #include "abr_common.cuh"
 #include "../../include/abr_b200_lookahead.h"
 #include "../../include/abr_b200_mpc_pred.h"
+#include "../../include/abr_b200_obs.h"
 
 namespace abr {
 static std::atomic<long long> g_launches{0};
@@ -516,27 +517,75 @@ int abr_env_step_live(AbrEnv* env, const int32_t* d_action, const double* d_spee
                                 d_next_sizes, d_end_of_video, d_throughput, stream);
 }
 
-int abr_env_step_policy(AbrEnv* env, const float* d_logits, int sample, uint64_t seed, const AbrObsSpec* spec,
-                        float* d_obs, int32_t* d_action_out, double* d_reward_sum, double* d_delay, double* d_sleep,
-                        double* d_buffer, double* d_rebuf, double* d_reward, uint8_t* d_end_of_video, void* stream) {
+// The checks of the windowed observation's spec and buffer (SPEC §4.5), in their order, and its fields of `pol`.
+static int set_obs_window(StepPolicyWindow& pol, const AbrObsWindowSpec* spec, float* d_obs) {
+    if (!spec) return fail(ABR_ERR_INVALID, "spec is NULL");
+    if (!d_obs) return fail(ABR_ERR_INVALID, "obs is NULL");
+    if (spec->window < 1 || spec->window > 32) return fail(ABR_ERR_RANGE, "window must be in [1, 32] (got %d)", spec->window);
+    pol.obs = d_obs; pol.window = spec->window;
+    pol.w_util = spec->util_scale; pol.w_buffer = spec->buffer_scale; pol.w_thr = spec->throughput_scale;
+    pol.w_delay = spec->delay_scale; pol.w_size = spec->size_scale;
+    return ABR_OK;
+}
+
+extern "C++" {
+// The policy-in-the-loop step (SPEC §4.1, §4.5): `name` is the entry point, `observe(pol)` sets its observation
+// fields and returns its own checks' result, after the common ones.
+template <typename Observe>
+static int step_policy_any(AbrEnv* env, const char* name, const float* d_logits, int sample, uint64_t seed,
+                           const Observe& observe, int32_t* d_action_out, double* d_reward_sum, double* d_delay,
+                           double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward,
+                           uint8_t* d_end_of_video, void* stream) {
     if (int rc = check_reset(env)) return rc;
-    if (env->v.p.live) return fail(ABR_ERR_STATE, "abr_env_step_policy is not available in live mode (SPEC 7)");
+    if (env->v.p.live) return fail(ABR_ERR_STATE, "%s is not available in live mode (SPEC 7)", name);
     if (env->v.n == 0) return ABR_OK;
     if (!d_logits) return fail(ABR_ERR_INVALID, "logits is NULL");
-    StepPolicy pol;
+    StepPolicyWindow pol;
+    if (int rc = observe(pol)) return rc;
     pol.logits = d_logits;
     pol.draw = sample ? env->d_draw_counter : nullptr;
     pol.seed_lo = (uint32_t)seed; pol.seed_hi = (uint32_t)(seed >> 32);
-    pol.action_out = d_action_out; pol.obs = d_obs; pol.reward_sum = d_reward_sum;
-    if (spec) {
-        pol.s_buffer = spec->buffer_scale; pol.s_thr = spec->throughput_scale;
-        pol.s_delay = spec->delay_scale; pol.s_size = spec->size_scale;
-    }
+    pol.action_out = d_action_out; pol.reward_sum = d_reward_sum;
     env->fresh_partials = 0;
     StepOutputs<double> o;
     o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
     o.eov = d_end_of_video;
     CUDA_TRY(launch_step_policy(env->v, pol, o, env->d_draw_counter, (cudaStream_t)stream));
+    return ABR_OK;
+}
+}  // extern "C++"
+
+int abr_env_step_policy(AbrEnv* env, const float* d_logits, int sample, uint64_t seed, const AbrObsSpec* spec,
+                        float* d_obs, int32_t* d_action_out, double* d_reward_sum, double* d_delay, double* d_sleep,
+                        double* d_buffer, double* d_rebuf, double* d_reward, uint8_t* d_end_of_video, void* stream) {
+    auto observe = [&](StepPolicyWindow& pol) {
+        pol.obs = d_obs;
+        if (spec) {
+            pol.s_buffer = spec->buffer_scale; pol.s_thr = spec->throughput_scale;
+            pol.s_delay = spec->delay_scale; pol.s_size = spec->size_scale;
+        }
+        return ABR_OK;
+    };
+    return step_policy_any(env, "abr_env_step_policy", d_logits, sample, seed, observe, d_action_out, d_reward_sum,
+                           d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_end_of_video, stream);
+}
+
+int abr_env_step_policy_window(AbrEnv* env, const float* d_logits, int sample, uint64_t seed,
+                               const AbrObsWindowSpec* spec, float* d_obs, int32_t* d_action_out, double* d_reward_sum,
+                               double* d_delay, double* d_sleep, double* d_buffer, double* d_rebuf, double* d_reward,
+                               uint8_t* d_end_of_video, void* stream) {
+    auto observe = [&](StepPolicyWindow& pol) { return set_obs_window(pol, spec, d_obs); };
+    return step_policy_any(env, "abr_env_step_policy_window", d_logits, sample, seed, observe, d_action_out,
+                           d_reward_sum, d_delay, d_sleep, d_buffer, d_rebuf, d_reward, d_end_of_video, stream);
+}
+
+int abr_env_observe_window(AbrEnv* env, const AbrObsWindowSpec* spec, float* d_obs, void* stream) {
+    if (int rc = check_reset(env)) return rc;
+    if (env->v.p.live) return fail(ABR_ERR_STATE, "abr_env_observe_window is not available in live mode (SPEC 7)");
+    if (env->v.n == 0) return ABR_OK;
+    StepPolicyWindow pol;
+    if (int rc = set_obs_window(pol, spec, d_obs)) return rc;
+    CUDA_TRY(launch_observe_window(env->v, pol, (cudaStream_t)stream));
     return ABR_OK;
 }
 

@@ -146,6 +146,14 @@ struct StepPolicy {
     double s_buffer = 1.0, s_thr = 1.0, s_delay = 1.0, s_size = 1.0;   // observation scales
     double* __restrict__ reward_sum = nullptr;     // [N]: += reward, nullable
 };
+// SPEC §4.5 windowed observation (abr_env_step_policy_window, abr_env_observe_window): the StepPolicy fields, then
+// window = W in [1, 32], which selects it (0 = the §4.1 observation), and its scales w_*; obs is then
+// [3 + 2W + A][N] and carries the throughput and download-time windows from one call to the next.  A type of its own
+// rather than fields appended to StepPolicy: a larger StepPolicy parameter changed the code of the live step kernels.
+struct StepPolicyWindow : StepPolicy {
+    int32_t window = 0;
+    double w_util = 1.0, w_buffer = 1.0, w_thr = 1.0, w_delay = 1.0, w_size = 1.0;
+};
 // Per-step outputs of both step launchers: element ix of each array ([N] for a step, [steps][N] for an episode,
 // next_sizes [N][A]); every pointer is nullable.  OT: double, or float for the fp32-output mode (the arithmetic stays
 // fp64, an output is rounded once on the store).
@@ -164,12 +172,14 @@ struct StepOutputs {
         return !delay && !sleep && !buffer && !rebuf && !reward && !eov && !actions && !latency && !thr && !next_sizes;
     }
 };
-cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const StepOutputs<double>& o,
+cudaError_t launch_step_policy(const EnvView& v, const StepPolicyWindow& pol, const StepOutputs<double>& o,
                                uint32_t* d_draw_counter, cudaStream_t st);
+// abr_env_observe_window (SPEC §4.5): the windowed observation of the state, both windows 0; pol.window and pol.obs set
+cudaError_t launch_observe_window(const EnvView& v, const StepPolicyWindow& pol, cudaStream_t st);
 // d_speed (live mode): the playback speed of content chunk k of session i is d_speed[k * N + i]; nullable = 1.0
 template <typename OT>
 cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, const StepOutputs<OT>& o,
-                        cudaStream_t st, const StepPolicy* policy = nullptr);
+                        cudaStream_t st, const StepPolicyWindow* policy = nullptr);
 // Fused reset + episode + session cost (abr_env_run_host): with in_trace_id the episode kernel resets every session
 // itself (SPEC §2) and out_cost receives Simulator.calculate_qoe per session; the pointers may alias pinned host memory.
 // Scratch of the statistics reduction (SPEC §6): one sum per group of block partials, and the counters of finished

@@ -823,14 +823,70 @@ __device__ __forceinline__ void store_step(const StepOutputs<OT>& o, const uint3
     }
 }
 
+// SPEC §4.5: what a windowed observation does with its two windows.
+enum WinMode { kWinZero, kWinRoll, kWinKeep };
+
+// SPEC §4.5: column i of the windowed observation obs[3 + 2W + A][N] from a session's state (chunk, last_q, buffer,
+// done).  kWinRoll: both windows move up one entry (fp32 bits copied; every load of a group of eight is issued before
+// its stores, which only reach entries that are already read) and take (thr, delay) last; kWinZero: both become 0;
+// kWinKeep: neither is touched.  Every other row is one fp64 operation rounded once to fp32.
+__device__ __forceinline__ void write_obs_window(const EnvView& v, const StepPolicyWindow& pol, const int i, const int chunk,
+                                                 const int last_q, const double buffer, const bool done, const WinMode mode,
+                                                 const double thr, const double delay) {
+    const int W = pol.window, A = v.A, V = v.V;
+    ABR_CHECK(i >= 0 && i < v.n && W >= 1 && W <= 32 && chunk >= 0 && (chunk < V || (done && chunk == V)),
+              "windowed observation column / window / chunk");
+    const size_t n = (size_t)v.n;
+    float* __restrict__ ob = pol.obs + i;
+    const int k_prev = chunk > 0 ? chunk - 1 : 0;
+    __stcs(ob, last_q < 0 ? 0.0f : (float)dmul(__ldg(v.util + (size_t)k_prev * A + last_q), pol.w_util));
+    __stcs(ob + n, (float)dmul(buffer, pol.w_buffer));
+    __stcs(ob + 2 * n, (float)ddiv((double)(V - chunk), (double)V));
+    float* __restrict__ wt = ob + 3 * n;                 // throughput window, oldest first
+    float* __restrict__ wd = ob + (size_t)(3 + W) * n;   // download-time window
+    if (mode == kWinRoll) {
+        for (int w0 = 0; w0 < W - 1; w0 += 8) {
+            float xt[8], xd[8];
+#pragma unroll
+            for (int k = 0; k < 8; ++k)
+                if (w0 + k < W - 1) {
+                    xt[k] = __ldcs(wt + (size_t)(w0 + k + 1) * n);
+                    xd[k] = __ldcs(wd + (size_t)(w0 + k + 1) * n);
+                }
+#pragma unroll
+            for (int k = 0; k < 8; ++k)
+                if (w0 + k < W - 1) {
+                    __stcs(wt + (size_t)(w0 + k) * n, xt[k]);
+                    __stcs(wd + (size_t)(w0 + k) * n, xd[k]);
+                }
+        }
+        __stcs(wt + (size_t)(W - 1) * n, (float)dmul(thr, pol.w_thr));
+        __stcs(wd + (size_t)(W - 1) * n, (float)dmul(delay, pol.w_delay));
+    } else if (mode == kWinZero) {
+        for (int w = 0; w < W; ++w) {
+            __stcs(wt + (size_t)w * n, 0.0f);
+            __stcs(wd + (size_t)w * n, 0.0f);
+        }
+    }
+    float* __restrict__ os = ob + (size_t)(3 + 2 * W) * n;
+    for (int a = 0; a < A; ++a)
+        __stcs(os + (size_t)a * n, done ? 0.0f : (float)dmul(__ldg(v.sizes + (size_t)chunk * A + a), pol.w_size));
+}
+
 // `q`: the action, already clamped to [0, A); `lk`: the step's table reads (the caller issues them as soon as it holds
 // the session's state words, next to the read of the trace record, so that the two L2 round trips overlap).
 // The outputs arrive as __restrict__ parameters (of the kernel and of this function), not as StepOutputs: nvcc drops
 // the qualifier on struct members, and without it the per-step kernels lose the no-alias facts their schedule is built
 // on (both forms measured slower on a B200: 0.2-0.3 us of 104 per launch at 4 Mi sessions).
-template <bool SMEM, bool FAST, bool LIVE, bool POL, typename OT>
+// POL: 0 = the action comes from the caller, 1 = from the logits with the §4.1 observation, 2 = from the logits with
+// the §4.5 windowed observation.  PolicyArgs<POL>: the kernel's policy parameter (StepPolicyWindow for POL = 2).
+template <int POL> struct PolicyArg { using type = StepPolicy; };
+template <> struct PolicyArg<2> { using type = StepPolicyWindow; };
+template <int POL> using PolicyArgs = typename PolicyArg<POL>::type;
+
+template <bool SMEM, bool FAST, bool LIVE, int POL, typename OT>
 __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const int i, const int q, const Lookup& lk,
-                                             const StepPolicy& pol, const double* __restrict__ speed,
+                                             const PolicyArgs<POL>& pol, const double* __restrict__ speed,
                                              OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer,
                                              OT* __restrict__ o_rebuf, OT* __restrict__ o_reward, uint8_t* __restrict__ o_eov,
                                              OT* __restrict__ o_latency, OT* __restrict__ o_thr, OT* __restrict__ o_next_sizes) {
@@ -879,7 +935,10 @@ __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const in
     if (POL) {   // SPEC §4.1: the chosen action, the running reward and the next observation, feature-major fp32
         if (pol.action_out) pol.action_out[i] = q;
         if (pol.reward_sum) pol.reward_sum[i] = dadd(pol.reward_sum[i], r.reward);
-        if (pol.obs) {
+        if constexpr (POL == 2) {   // SPEC §4.5: from the state after the step; an end of video with auto_reset restarts the windows
+            write_obs_window(v, pol, i, s.chunk, s.last_q, s.buffer, !FAST && s.done,
+                             r.inert ? kWinKeep : (r.reset_mpc ? kWinZero : kWinRoll), r.thr, r.delay);
+        } else if (pol.obs) {
             ABR_CHECK(i >= 0 && i < v.n && (s.chunk >= 0 && (s.chunk < v.V || s.done)), "observation column / next chunk");
             float* __restrict__ ob = pol.obs + i;
             const size_t n = (size_t)v.n;
@@ -908,13 +967,14 @@ __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const in
 // the following tiles stay on that trace; no barrier is needed while the rows stay — and the probes of the lanes on
 // that trace are LDS.  Every other lane reads the L2-resident tables directly (one index pair + one or two sectors of C).
 // POL: the actions come from the caller's logits (policy_action) instead of `action`, and the kernel also writes the
-// next observation (SPEC §4.1); never with FAST or LIVE.
-template <bool FAST, bool LIVE, bool POL, typename OT>
+// next observation (POL = 1: SPEC §4.1; POL = 2: the windowed observation of §4.5); never with FAST or LIVE.
+template <bool FAST, bool LIVE, int POL, typename OT>
 __global__ void __launch_bounds__(kTile, (LIVE || POL) ? 4 : kTileBlocksPerSM)
 abr_step_kernel(EnvView v, const int32_t* __restrict__ action, const double* __restrict__ speed,
                 OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer, OT* __restrict__ o_rebuf,
                 OT* __restrict__ o_reward, OT* __restrict__ o_latency, OT* __restrict__ o_next_sizes,
-                uint8_t* __restrict__ o_eov, OT* __restrict__ o_thr, int smem_doubles, int tiles_per_block, const StepPolicy pol) {
+                uint8_t* __restrict__ o_eov, OT* __restrict__ o_thr, int smem_doubles, int tiles_per_block,
+                const PolicyArgs<POL> pol) {
     extern __shared__ __align__(16) double2 s_row2[];
     __shared__ __align__(8) unsigned long long s_mbar;
     __shared__ Quad s_meta;                      // the record of the trace whose rows are staged
@@ -1735,10 +1795,10 @@ static cudaError_t allow_smem(Kernel kernel, size_t bytes) {
 
 template <typename OT>
 cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, const StepOutputs<OT>& o,
-                        cudaStream_t st, const StepPolicy* policy) {
+                        cudaStream_t st, const StepPolicyWindow* policy) {
     if (v.n == 0) return cudaSuccess;
     const bool live = v.p.live != 0;
-    const StepPolicy pol = policy ? *policy : StepPolicy{};
+    const StepPolicyWindow pol = policy ? *policy : StepPolicyWindow{};
     const bool fast = !policy && !live && o.has_core() && v.p.track_history == 0 && v.p.track_acc == 0 &&
                       v.p.auto_reset != 0;
     // persistent-style grid: one wave of kTileBlocksPerSM blocks per SM, each walking an equal run of consecutive
@@ -1766,28 +1826,29 @@ cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double*
     };
     cudaError_t e;
     if (policy) {
-        if constexpr (std::is_same<OT, double>::value) e = go(abr_step_kernel<false, false, true, OT>);
+        if constexpr (std::is_same<OT, double>::value)
+            e = pol.window > 0 ? go(abr_step_kernel<false, false, 2, OT>) : go(abr_step_kernel<false, false, 1, OT>);
         else return cudaErrorInvalidValue;
     }
-    else if (live) e = go(abr_step_kernel<false, true, false, OT>);
-    else if (fast) e = go(abr_step_kernel<true, false, false, OT>);
-    else e = go(abr_step_kernel<false, false, false, OT>);
+    else if (live) e = go(abr_step_kernel<false, true, 0, OT>);
+    else if (fast) e = go(abr_step_kernel<true, false, 0, OT>);
+    else e = go(abr_step_kernel<false, false, 0, OT>);
     if (e != cudaSuccess) return e;
     count_launch();
     return cudaGetLastError();
 }
 
 template cudaError_t launch_step<double>(const EnvView&, const int32_t*, const double*, const StepOutputs<double>&,
-                                         cudaStream_t, const StepPolicy*);
+                                         cudaStream_t, const StepPolicyWindow*);
 template cudaError_t launch_step<float>(const EnvView&, const int32_t*, const double*, const StepOutputs<float>&,
-                                        cudaStream_t, const StepPolicy*);
+                                        cudaStream_t, const StepPolicyWindow*);
 
 __global__ void abr_bump_kernel(uint32_t* counter) { *counter += 1u; }
 
 // SPEC §4.1: the step with the action drawn from the caller's logits and the observation written by the same kernel;
 // the draw counter is advanced behind it (same stream: every thread has read it by then), so that a captured graph
 // replays with a new draw every time.
-cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const StepOutputs<double>& o,
+cudaError_t launch_step_policy(const EnvView& v, const StepPolicyWindow& pol, const StepOutputs<double>& o,
                                uint32_t* d_draw_counter, cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;
     cudaError_t e = launch_step<double>(v, nullptr, nullptr, o, st, &pol);
@@ -1796,6 +1857,21 @@ cudaError_t launch_step_policy(const EnvView& v, const StepPolicy& pol, const St
         abr_bump_kernel<<<1, 1, 0, st>>>(d_draw_counter);
         count_launch();
     }
+    return cudaGetLastError();
+}
+
+// SPEC §4.5: the windowed observation of every session's state, both windows 0 (the first observation of an episode).
+__global__ void __launch_bounds__(kStepBlock) abr_observe_window_kernel(EnvView v, const StepPolicyWindow pol) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= v.n) return;
+    const bool done = !v.p.auto_reset && v.done[i] != 0;
+    write_obs_window(v, pol, i, v.chunk[i], v.last_q[i], v.buffer[i], done, kWinZero, 0.0, 0.0);
+}
+
+cudaError_t launch_observe_window(const EnvView& v, const StepPolicyWindow& pol, cudaStream_t st) {
+    if (v.n == 0) return cudaSuccess;
+    abr_observe_window_kernel<<<(v.n + kStepBlock - 1) / kStepBlock, kStepBlock, 0, st>>>(v, pol);
+    count_launch();
     return cudaGetLastError();
 }
 

@@ -350,6 +350,71 @@ class BatchedABREnv:
                 g("reward"), g("end_of_video"), _stream()))
         return obs
 
+    # -- SPEC §4.5: the windowed (Pensieve-style) observation --
+    def _window_spec(self, window, scales):
+        if not 1 <= int(window) <= 32:
+            raise ValueError(f"window must be in [1, 32] (got {window})")
+        if len(scales) != 5:
+            raise ValueError("scales are (util, buffer, throughput, delay, size)")
+        return _lib.AbrObsWindowSpec(int(window), *[float(x) for x in scales])
+
+    def observe_window(self, window=8, scales=(1.0,) * 5, obs=None):
+        """The windowed observation of the current state (float32 [3 + 2W + A, N], feature-major, W = ``window``) with
+        both windows 0: the first observation of an episode, or a restart of the windows.  Rows: the last chunk's
+        utility, the buffer, the chunks left / V, the last W throughputs, the last W download times (oldest first)
+        and the next chunk's sizes, each times its entry of ``scales`` = (util, buffer, throughput, delay, size)
+        (the chunks left are not scaled).  ``obs``: written in place when given."""
+        spec = self._window_spec(window, scales)
+        n, F = self.n, 3 + 2 * int(window) + self.A
+        if obs is None:
+            obs = self._empty(F, n, dtype=torch.float32)
+        self._check_window_obs(obs, F, n)
+        with self._on:
+            _lib.check(self._lib.abr_env_observe_window(self._h, spec, _addr(obs), _stream()))
+        return obs
+
+    def _check_window_obs(self, obs, F, n):
+        if obs.dtype != torch.float32 or obs.device != self.device or not obs.is_contiguous() or \
+                tuple(obs.shape) != (F, n):
+            raise TypeError(f"obs must be a contiguous float32 [3 + 2W + A, N] = [{F}, {n}] tensor on {self.device}")
+
+    def step_policy_window(self, logits, obs, sample=True, seed=0, scales=(1.0,) * 5, action_out=None,
+                           reward_sum=None, out=None):
+        """``step_policy`` with the windowed observation of ``observe_window``: ``obs`` (float32 [3 + 2W + A, N],
+        W = (rows - 3 - A) / 2) holds the two windows from one call to the next and is updated in place: each step
+        moves them up one entry and appends its throughput and download time, a step that ends the video with
+        auto_reset zeroes them, and an inert step (a done session, auto_reset=0) leaves them.  Action, per-step
+        outputs, ``action_out``, ``reward_sum`` and the state are those of ``step_policy``.  All arguments are used in
+        place (graph-capturable); returns ``obs``."""
+        n = self.n
+        if logits.dtype != torch.float32 or logits.device != self.device or not logits.is_contiguous() or \
+                logits.numel() != n * self.A:
+            raise TypeError(f"logits must be a contiguous float32 [N, A] = [{n}, {self.A}] tensor on {self.device}")
+        if obs is None or obs.dim() != 2 or (obs.shape[0] - 3 - self.A) % 2 or obs.shape[0] < 5 + self.A:
+            raise TypeError(f"obs must be a float32 [3 + 2W + A, N] tensor with W in [1, 32] (A = {self.A})")
+        W = (obs.shape[0] - 3 - self.A) // 2
+        spec = self._window_spec(W, scales)
+        self._check_window_obs(obs, obs.shape[0], n)
+
+        def chk(t, dtype, size, name):
+            if t is not None and (t.dtype != dtype or t.device != self.device or not t.is_contiguous() or t.numel() != size):
+                raise TypeError(f"{name} must be a contiguous {dtype} tensor of {size} elements on {self.device}")
+
+        chk(action_out, torch.int32, n, "action_out")
+        chk(reward_sum, torch.float64, n, "reward_sum")
+        o = out
+        for name in ("delay", "sleep", "buffer", "rebuffer", "reward") if o is not None else ():
+            chk(getattr(o, name), torch.float64, n, name)
+        if o is not None:
+            chk(o.end_of_video, torch.uint8, n, "end_of_video")
+        g = (lambda name: _addr(getattr(o, name))) if o is not None else (lambda name: None)
+        with self._on:
+            _lib.check(self._lib.abr_env_step_policy_window(
+                self._h, _addr(logits), int(bool(sample)), int(seed), spec, _addr(obs),
+                _addr(action_out), _addr(reward_sum), g("delay"), g("sleep"), g("buffer"), g("rebuffer"),
+                g("reward"), g("end_of_video"), _stream()))
+        return obs
+
     # -- SPEC §3+§4 --
     def rollout(self, policy, steps, seed=0, actions=None, want=("delay", "sleep", "buffer", "rebuffer", "reward",
                                                                 "end_of_video", "actions"), out=None, speed=None,
