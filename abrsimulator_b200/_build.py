@@ -17,10 +17,12 @@ CSRC = os.path.join(HERE, "csrc")
 _SUFFIX = os.environ.get("ABR_LIB_SUFFIX", "")
 LIB = os.path.join(HERE, "lib", f"libabr_b200{_SUFFIX}.so")
 STAMP = LIB + ".srchash"
-SOURCES = ["abr_step.cu", "abr_mpc.cu", "abr_capi.cu", "abr_sort.cu"]
-HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(HERE, "..", "include", "abr_b200.h"),
+SOURCES = ["abr_step.cu", "abr_mpc.cu", "abr_mpc_scen.cu", "abr_capi.cu", "abr_sort.cu"]
+HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(CSRC, "abr_mpc_search.cuh"),
+           os.path.join(HERE, "..", "include", "abr_b200.h"),
            os.path.join(HERE, "..", "include", "abr_b200_lookahead.h"),
            os.path.join(HERE, "..", "include", "abr_b200_mpc_pred.h"),
+           os.path.join(HERE, "..", "include", "abr_b200_mpc_scen.h"),
            os.path.join(HERE, "..", "include", "abr_b200_obs.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",

@@ -117,6 +117,11 @@ OBS_SIGNATURES = {
     "abr_env_step_policy_window": (_I, [_P, _P, _I, _U64, _OBS_WINDOW_SPEC] + [_P] * 10),
     "abr_env_observe_window": (_I, [_P, _OBS_WINDOW_SPEC, _P, _P]),
 }
+# include/abr_b200_mpc_scen.h: MPC over caller-supplied throughput scenarios (SPEC §5.7).
+MPC_SCEN_MEAN, MPC_SCEN_WORST, MPC_SCEN_MAX = 0, 1, 16
+MPC_SCEN_SIGNATURES = {
+    "abr_env_mpc_decide_scen": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
+}
 
 _lib = None
 
@@ -136,7 +141,8 @@ def load():
         # under a file lock: concurrent ranks build once, the rest wait and load the finished file
         _build.build_library()
     lib = C.CDLL(path)
-    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES}.items():
+    for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES,
+                                   **MPC_SCEN_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -12,6 +12,7 @@
 #include "abr_common.cuh"
 #include "../../include/abr_b200_lookahead.h"
 #include "../../include/abr_b200_mpc_pred.h"
+#include "../../include/abr_b200_mpc_scen.h"
 #include "../../include/abr_b200_obs.h"
 
 namespace abr {
@@ -719,6 +720,34 @@ int abr_env_mpc_decide_pred(AbrEnv* env, int horizon, int flags, const double* d
     a.error_count64 = v.errors;
     a.pred = d_pred;
     CUDA_TRY(launch_mpc(a, (cudaStream_t)stream));
+    return ABR_OK;
+}
+
+int abr_env_mpc_decide_scen(AbrEnv* env, int horizon, int n_scen, int objective, int flags, const double* d_pred,
+                            const double* d_weight, int32_t* d_action, double* d_best_j, int32_t* d_best_seq,
+                            void* stream) {
+    if (int rc = check_reset(env)) return rc;
+    if (env->v.n == 0) return ABR_OK;
+    if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
+    if (!d_pred) return fail(ABR_ERR_INVALID, "pred is NULL");
+    if (objective != ABR_MPC_SCEN_MEAN && objective != ABR_MPC_SCEN_WORST)
+        return fail(ABR_ERR_INVALID, "objective must be ABR_MPC_SCEN_MEAN or ABR_MPC_SCEN_WORST (got %d)", objective);
+    if (d_weight && objective == ABR_MPC_SCEN_WORST)
+        return fail(ABR_ERR_INVALID, "weights apply to ABR_MPC_SCEN_MEAN only");
+    if (flags != 0 && flags != ABR_MPC_EXHAUSTIVE)
+        return fail(ABR_ERR_INVALID, "flags must be 0 or ABR_MPC_EXHAUSTIVE (got %d)", flags);
+    if (int rc = check_mpc_shape(env->v.A, horizon)) return rc;
+    if (n_scen < 1 || n_scen > ABR_MPC_SCEN_MAX)
+        return fail(ABR_ERR_RANGE, "n_scen must be in [1, %d] (got %d)", ABR_MPC_SCEN_MAX, n_scen);
+    const EnvView& v = env->v;
+    MpcScenArgs a{};   // no history ring and no robust state: the kernel reads neither (SPEC 5.7)
+    a.sizes = v.sizes; a.util = v.util; a.V = v.V; a.A = v.A; a.p = v.p; a.N = v.n;
+    a.chunk_idx = v.chunk; a.prev_q = v.last_q; a.buffer = v.buffer; a.done = v.p.auto_reset ? nullptr : v.done;
+    a.H = horizon; a.K = n_scen; a.objective = objective; a.flags = flags;
+    a.pred = d_pred; a.weight = d_weight;
+    a.action = d_action; a.best_j = d_best_j; a.best_seq = d_best_seq;
+    a.error_count64 = v.errors;
+    CUDA_TRY(launch_mpc_scen(a, (cudaStream_t)stream));
     return ABR_OK;
 }
 

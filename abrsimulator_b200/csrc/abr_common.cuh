@@ -237,6 +237,18 @@ struct MpcArgs {
     const double* pred = nullptr;
 };
 cudaError_t launch_mpc(const MpcArgs& a, cudaStream_t st);
+// MPC over throughput scenarios (SPEC §5.7): pred [N][K][H], weight [N][K] (nullable, MEAN only)
+struct MpcScenArgs {
+    const double* sizes; const double* util; int V, A;
+    AbrParams p;
+    int N;
+    const int32_t* chunk_idx; const int32_t* prev_q; const double* buffer; const uint8_t* done;  // done nullable
+    int H, K, objective, flags;
+    const double* pred; const double* weight;
+    int32_t* action; double* best_j; int32_t* best_seq;   // best_j, best_seq nullable
+    unsigned long long* error_count64;
+};
+cudaError_t launch_mpc_scen(const MpcScenArgs& a, cudaStream_t st);
 cudaError_t launch_mpc_score(const double* d_sizes, const double* d_util, int V, int A, const AbrParams& p, int k,
                              int prev_q, double buffer, const double* d_hist, int n, int H, int mode, double max_err,
                              const int32_t* d_seqs, int M, double* d_scores, cudaStream_t st);

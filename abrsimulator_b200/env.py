@@ -132,6 +132,12 @@ def _out_dtype(t, dtype):
     return d
 
 
+def _float_rows(t, name, device):
+    if not isinstance(t, torch.Tensor) or t.device != device or t.dtype not in (torch.float64, torch.float32):
+        raise TypeError(f"{name} must be a float64 or float32 tensor on {device}")
+    return t
+
+
 class BatchedABREnv:
     """N sessions over shared trace / video tables.
 
@@ -580,6 +586,63 @@ class BatchedABREnv:
         act = self._empty(self.n, dtype=torch.int32)
         for _ in range(steps):
             self.mpc_decide_pred(predictor(self), horizon, out=act, exhaustive=exhaustive)
+            with self._on:
+                _lib.check(self._lib.abr_env_step(self._h, _addr(act), None, None, None, None, None, None, None, None,
+                                                  _stream()))   # live mode: speed 1.0
+        return act
+
+    # -- SPEC §5.7 --
+    def mpc_decide_scen(self, scenarios, horizon=5, weights=None, objective="mean", want_score=False, want_seq=False,
+                        out=None, exhaustive=False):
+        """MPC decision (SPEC §5.7) over K caller-supplied throughput scenarios: the sequence whose SPEC §5.2
+        objective values under the scenarios have the best weighted mean (``objective="mean"``) or the best worst case
+        (``"worst"``).  ``scenarios`` is a device tensor [N, K, horizon] (scenario k of session s at [s, k]), or
+        [N, K] for one throughput per scenario at every step, float64 or float32 (widened exactly), 1 <= K <= 16, in
+        environment order.  ``weights`` [N, K] (mean only; None: 1/K each).  Only the first min(horizon, V - chunk)
+        steps are read; a session with a throughput that is not finite and > 0, a weight that is not finite and >= 0,
+        or only zero weights gets action -1 and counts as an error.  Reads no history ring and writes no state.
+        Returns like ``mpc_decide_pred``."""
+        act = self._empty(self.n, dtype=torch.int32) if out is None else out
+        if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:
+            raise TypeError(f"out must be a contiguous int32 tensor of {self.n} elements on {self.device}")
+        objs = dict(mean=_lib.MPC_SCEN_MEAN, worst=_lib.MPC_SCEN_WORST)
+        if objective not in objs:
+            raise ValueError(f"objective must be 'mean' or 'worst' (got {objective!r})")
+        H = int(horizon)
+        p = _float_rows(scenarios, "scenarios", self.device)
+        if p.dim() == 2 and p.shape[0] == self.n:
+            p = p.unsqueeze(2).expand(self.n, p.shape[1], H)
+        if p.dim() != 3 or p.shape[0] != self.n or p.shape[2] != H:
+            raise ValueError(f"scenarios must be [N, K] or [N, K, horizon] with N = {self.n}, horizon = {H} "
+                             f"(got {tuple(p.shape)})")
+        K = p.shape[1]
+        p = p.to(torch.float64).contiguous()
+        w = None
+        if weights is not None:
+            w = _float_rows(weights, "weights", self.device)
+            if tuple(w.shape) != (self.n, K):
+                raise ValueError(f"weights must be [N, K] = [{self.n}, {K}] (got {tuple(w.shape)})")
+            w = w.to(torch.float64).contiguous()
+        bj = self._empty(self.n) if want_score else None
+        seq = self._empty(self.n, H, dtype=torch.int32) if want_seq else None
+        flags = _lib.MPC_EXHAUSTIVE if exhaustive else 0
+        with self._on:
+            _lib.check(self._lib.abr_env_mpc_decide_scen(self._h, H, K, objs[objective], flags, _addr(p), _addr(w),
+                                                         _addr(act), _addr(bj), _addr(seq), _stream()))
+        if not (want_score or want_seq):
+            return act
+        return (act,) + ((bj,) if want_score else ()) + ((seq,) if want_seq else ())
+
+    def mpc_episode_scen(self, steps, sampler, horizon=5, objective="mean", exhaustive=False):
+        """``sampler(env)`` -> mpc_decide_scen -> step for `steps` chunks (track_acc=1 for the per-session sums).
+        ``sampler`` returns the scenarios ([N, K] or [N, K, horizon] on the device) or a pair (scenarios, weights)
+        for the current state.  Nothing here synchronises with the host, so one chunk can be captured in a CUDA graph
+        when the sampler allows it."""
+        act = self._empty(self.n, dtype=torch.int32)
+        for _ in range(steps):
+            r = sampler(self)
+            scen, w = r if isinstance(r, tuple) else (r, None)
+            self.mpc_decide_scen(scen, horizon, weights=w, objective=objective, out=act, exhaustive=exhaustive)
             with self._on:
                 _lib.check(self._lib.abr_env_step(self._h, _addr(act), None, None, None, None, None, None, None, None,
                                                   _stream()))   # live mode: speed 1.0
