@@ -13,6 +13,7 @@ from . import _build
 NUM_ACC = 11
 NUM_STATS = 11
 POLICY_FIXED, POLICY_RANDOM, POLICY_BBA, POLICY_RATE, POLICY_BOLA = 0, 1, 2, 3, 4
+POLICY_DYNAMIC = 5                                   # include/abr_b200_dynamic.h
 MPC_REF, MPC_ROBUST = 0, 1
 MPC_TRUNCATE, MPC_EMPTY_DEFAULT, MPC_PRED_SES, MPC_EXHAUSTIVE = 1, 2, 4, 8
 MPC_MODE_EXHAUSTIVE = 0x100
@@ -23,7 +24,7 @@ FIELDS = dict(seg=(0, "int32"), chunk=(1, "int32"), last_q=(2, "int32"), trace_i
               buffer=(11, "float64"), bw_hist=(12, "float64"), last_pred=(13, "float64"),
               err_ring=(14, "float64"), acc=(15, "float64"), t_now=(16, "float64"), play_time=(17, "float64"),
               started=(7, "uint8"), play_id=(8, "int32"), play_len=(19, "float64"), sizes=(20, "float64"), utility=(21, "float64"),
-              trace_bw=(22, "float64"), order=(23, "int32"))
+              trace_bw=(22, "float64"), order=(23, "int32"), dyn_mode=(24, "uint8"))
 
 
 class AbrError(RuntimeError):
@@ -44,6 +45,11 @@ class AbrParams(C.Structure):
 class AbrPolicyParams(C.Structure):
     """Parameters of the RATE and BOLA policies (SPEC §4.2, §4.3)."""
     _fields_ = [(n, C.c_double) for n in ("rb_safety", "bola_min_buffer", "bola_target_buffer")]
+
+
+class AbrDynamicParams(C.Structure):
+    """The buffer thresholds of the DYNAMIC policy (SPEC §4.6, include/abr_b200_dynamic.h)."""
+    _fields_ = [(n, C.c_double) for n in ("switch_on_buffer", "switch_off_buffer")]
 
 
 class AbrObsSpec(C.Structure):
@@ -122,6 +128,12 @@ MPC_SCEN_MEAN, MPC_SCEN_WORST, MPC_SCEN_MAX = 0, 1, 16
 MPC_SCEN_SIGNATURES = {
     "abr_env_mpc_decide_scen": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
 }
+# include/abr_b200_dynamic.h: the DYNAMIC policy's parameters (SPEC §4.6).
+_DYNAMIC_PARAMS = C.POINTER(AbrDynamicParams)
+DYNAMIC_SIGNATURES = {
+    "abr_dynamic_params_default": (None, [_DYNAMIC_PARAMS]),
+    "abr_env_set_dynamic_params": (_I, [_P, _DYNAMIC_PARAMS]),
+}
 
 _lib = None
 
@@ -142,7 +154,7 @@ def load():
         _build.build_library()
     lib = C.CDLL(path)
     for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES,
-                                   **MPC_SCEN_SIGNATURES}.items():
+                                   **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

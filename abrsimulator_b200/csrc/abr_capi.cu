@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "abr_common.cuh"
+#include "../../include/abr_b200_dynamic.h"
 #include "../../include/abr_b200_lookahead.h"
 #include "../../include/abr_b200_mpc_pred.h"
 #include "../../include/abr_b200_mpc_scen.h"
@@ -192,6 +193,19 @@ static void install_policy_params(AbrEnv* env, const AbrPolicyParams* pp) {
     pol.bola_Vp = pp->bola_min_buffer / pol.bola_gp;
 }
 
+void abr_dynamic_params_default(AbrDynamicParams* p) {
+    if (!p) return;
+    p->switch_on_buffer = 12.0; p->switch_off_buffer = 6.0;
+}
+
+static int check_dynamic_params(const AbrDynamicParams* dp) {
+    if (!dp) return fail(ABR_ERR_INVALID, "dynamic params is NULL");
+    if (!std::isfinite(dp->switch_on_buffer) || !std::isfinite(dp->switch_off_buffer) || !(dp->switch_off_buffer >= 0.0) ||
+        !(dp->switch_off_buffer < dp->switch_on_buffer))
+        return fail(ABR_ERR_INVALID, "need finite 0 <= switch_off_buffer < switch_on_buffer");
+    return ABR_OK;
+}
+
 static int check_tables(const double* sizes, const double* bitrates, int V, int A) {
     if (!sizes || !bitrates) return fail(ABR_ERR_INVALID, "sizes/bitrates is NULL");
     if (V < 1 || A < 1 || A > 16) return fail(ABR_ERR_RANGE, "need V >= 1 and 1 <= A <= 16 (got V=%d A=%d)", V, A);
@@ -281,6 +295,9 @@ int abr_env_create(const double* h_trace_bw, const int32_t* h_trace_len, const d
         AbrPolicyParams pp;
         abr_policy_params_default(&pp);
         install_policy_params(e, &pp);
+        AbrDynamicParams dp;
+        abr_dynamic_params_default(&dp);
+        v.pol.dyn_on = dp.switch_on_buffer; v.pol.dyn_off = dp.switch_off_buffer;
     }
     // per-trace tables of SPEC §3.1 (cumulative capacity, search widths), built on the device
     // (+4 doubles of slack: the step reads C[j .. j+4] and discards what lies past its candidates)
@@ -315,6 +332,10 @@ int abr_env_create(const double* h_trace_bw, const int32_t* h_trace_len, const d
     CUDA_TRY(cudaMemset(v.errors, 0, sizeof(unsigned long long)));
     CUDA_TRY(cudaMemset(v.bw_hist, 0, sizeof(double) * cap * v.K));
     CUDA_TRY(cudaMemset(v.err_ring, 0, sizeof(double) * cap * v.K));
+    if (params->track_history) {   // DYNAMIC's active rule (SPEC §4.6); DYNAMIC is rejected without the history
+        CUDA_TRY(e->alloc(&v.pol.dyn_mode, cap));
+        CUDA_TRY(cudaMemset(v.pol.dyn_mode, 0, cap));
+    }
     e->n_partials_cap = stats_num_partials(max_sessions) > rollout_num_blocks(max_sessions)
                             ? stats_num_partials(max_sessions) : rollout_num_blocks(max_sessions);
     CUDA_TRY(e->alloc(&e->d_stats_partials, (size_t)e->n_partials_cap * ABR_NUM_ACC));
@@ -394,12 +415,17 @@ static void begin_batch(AbrEnv* env, int n_sessions, long long session_base) {
     env->step_base = 0;
 }
 
-// A built-in policy id the environment can run: RATE reads the history ring, BOLA the log table of positive sizes.
+// A built-in policy id the environment can run: RATE reads the history ring, BOLA the log table of positive sizes,
+// DYNAMIC both (checked in that order).
 static int check_policy(const AbrEnv* env, int policy) {
-    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_BOLA) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
+    if (policy < ABR_POLICY_FIXED || policy > ABR_POLICY_DYNAMIC) return fail(ABR_ERR_INVALID, "unknown policy %d", policy);
     if (policy == ABR_POLICY_RATE && !env->v.p.track_history)
         return fail(ABR_ERR_STATE, "ABR_POLICY_RATE needs the throughput history: create the environment with track_history = 1");
+    if (policy == ABR_POLICY_DYNAMIC && !env->v.p.track_history)
+        return fail(ABR_ERR_STATE, "ABR_POLICY_DYNAMIC needs the throughput history: create the environment with track_history = 1");
     if (policy == ABR_POLICY_BOLA && !env->v.pol.bola_v) return fail(ABR_ERR_INVALID, "BOLA needs positive chunk sizes");
+    if (policy == ABR_POLICY_DYNAMIC && !env->v.pol.bola_v)
+        return fail(ABR_ERR_INVALID, "ABR_POLICY_DYNAMIC runs BOLA, and BOLA needs positive chunk sizes");
     return ABR_OK;
 }
 
@@ -410,10 +436,19 @@ int abr_env_set_policy_params(AbrEnv* env, const AbrPolicyParams* params) {
     return ABR_OK;
 }
 
+int abr_env_set_dynamic_params(AbrEnv* env, const AbrDynamicParams* params) {
+    if (int rc = check_dynamic_params(params)) return rc;   // host-side only: bad values are reported without a device
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    env->v.pol.dyn_on = params->switch_on_buffer;
+    env->v.pol.dyn_off = params->switch_off_buffer;
+    return ABR_OK;
+}
+
 int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stream) {
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
-    if (policy != ABR_POLICY_BBA && policy != ABR_POLICY_RATE && policy != ABR_POLICY_BOLA)
-        return fail(ABR_ERR_INVALID, "abr_env_policy_decide takes ABR_POLICY_BBA, _RATE or _BOLA (got %d)", policy);
+    if (policy != ABR_POLICY_BBA && policy != ABR_POLICY_RATE && policy != ABR_POLICY_BOLA && policy != ABR_POLICY_DYNAMIC)
+        return fail(ABR_ERR_INVALID, "abr_env_policy_decide takes ABR_POLICY_BBA, _RATE or _BOLA (got %d), or ABR_POLICY_DYNAMIC",
+                    policy);
     if (int rc = check_policy(env, policy)) return rc;
     if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
@@ -803,6 +838,9 @@ int abr_env_state_ptr(AbrEnv* env, int field, void** d_ptr) {
         case ABR_F_ORDER:
             if (!v.perm) return fail(ABR_ERR_STATE, "no session order is installed");
             *d_ptr = (void*)v.perm; break;
+        case ABR_F_DYN_MODE:
+            if (!v.pol.dyn_mode) return fail(ABR_ERR_STATE, "dyn_mode needs track_history = 1");
+            *d_ptr = v.pol.dyn_mode; break;
         default: return fail(ABR_ERR_INVALID, "unknown state field %d", field);
     }
     return ABR_OK;

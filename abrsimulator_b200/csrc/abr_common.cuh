@@ -127,6 +127,13 @@ struct EnvView {
     struct Policy {
         const double* __restrict__ bola_v;      // [V][A] log(sizes[k][a] / sizes[k][0]); null when a size is not > 0
         double rb_safety, bola_Vp, bola_gp, bola_vmax;
+        // DYNAMIC (SPEC §4.6): the per-session active rule (0 = RATE, 1 = BOLA; allocated with track_history = 1)
+        // and the buffer thresholds that switch it; after the fields above for the same reason.  32 bytes with the
+        // padding: the kernel parameters that follow an EnvView keep their 16-byte alignment, which the compiler uses
+        // to load two of them at once (24 bytes turned such pairs into two loads in kernels that never read these).
+        uint8_t* dyn_mode;
+        double dyn_on, dyn_off;
+        double pad_;
     } pol;
 };
 
@@ -195,7 +202,8 @@ template <typename OT>
 cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, uint32_t step_base,
                            const int32_t* d_actions_in, const double* d_speed, const StepOutputs<OT>& o,
                            double* d_block_partials, const RolloutFused& f, cudaStream_t st);
-// abr_env_policy_decide: the action of policy BBA / RATE / BOLA for every session from the SoA state
+// abr_env_policy_decide: the action of policy BBA / RATE / BOLA / DYNAMIC for every session from the SoA state
+// (DYNAMIC also writes the session's active rule)
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st);
 // abr_env_lookahead_decide (SPEC §4.4): the clairvoyant best sequence over the next min(H, V - chunk) chunks against
 // every session's own trace, H in [1, 8]; d_best_value [N] and d_best_seq [N][H] nullable.  Writes nothing else but

@@ -32,6 +32,7 @@
 #include <type_traits>
 
 #include "abr_common.cuh"
+#include "../../include/abr_b200_dynamic.h"
 
 namespace abr {
 
@@ -529,6 +530,13 @@ __device__ __forceinline__ int policy_bola(const EnvView& v, const double b, con
         if (a == 0 || sc > best) { best = sc; q = a; }
     }
     return q;
+}
+
+// SPEC §4.6, DYNAMIC: the rule of this decision (1 = BOLA, 0 = RATE) from the one the session's last DYNAMIC decision
+// left, prev, and the pre-step buffer b.  Chunk 0 ignores prev, so every episode starts on the rate rule; the strict >
+// is dash.js's.
+__device__ __forceinline__ int dynamic_mode(const EnvView& v, const int chunk, const double b, const int prev) {
+    return b > (chunk != 0 && prev ? v.pol.dyn_off : v.pol.dyn_on) ? 1 : 0;
 }
 
 // The per-session words of a step that come straight from the SoA state (coalesced: thread i <-> session i).
@@ -1277,6 +1285,10 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     const bool hist = !FAST && v.p.track_history != 0;
     const bool prev_ladder = v.p.smooth_prev_ladder != 0;
     uint32_t packed = 0u;   // random policy: the eight actions of one Philox block, one per nibble
+    // DYNAMIC keeps the session's active rule in `packed` for the whole call and stores it back at its end.  (The
+    // register is shared, and every DYNAMIC statement is an `if constexpr`, so that the other policies' forms compile
+    // to the instructions they compiled to before DYNAMIC existed.)
+    if constexpr (POLICY == ABR_POLICY_DYNAMIC) packed = v.pol.dyn_mode[i];
     if (LIVE) load_live(v, s, i, o.speed, fresh);
     // SPEC §4 action of step t; must be called with increasing t.  FIXED clamps t to the last row so that the
     // calls that run ahead of the final step stay inside the caller's table.
@@ -1301,6 +1313,16 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
                 packed = two(r.x) | (two(r.y) << 8) | (two(r.z) << 16) | (two(r.w) << 24);
             }
             return (int)((packed >> (4 * (tg & 7u))) & 0xfu);
+        }
+        if constexpr (POLICY == ABR_POLICY_DYNAMIC) {   // only the active rule is evaluated
+            if (!FAST && s.done) return 0;   // chunk == V: no sizes row (the step is inert, the rule is kept)
+            const int row = s.chunk * v.A;
+            ABR_CHECK(s.chunk >= 0 && s.chunk < v.V, "policy row");
+            auto size_at = [&](const int a) -> double {
+                return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
+            };
+            packed = (uint32_t)dynamic_mode(v, s.chunk, s.buffer, (int)packed);
+            return packed ? policy_bola(v, s.buffer, row, size_at) : policy_rate(v, i, s.hist_len, size_at);
         }
         if (POLICY == ABR_POLICY_RATE || POLICY == ABR_POLICY_BOLA) {
             if (!FAST && s.done) return 0;   // chunk == V: no sizes row (the step is inert)
@@ -1406,6 +1428,7 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     }
     if (flagged || (LIVE && s.bad_speed)) atomicAdd(v.errors, 1ull);
     store_state<LIVE>(v, s, i);
+    if constexpr (POLICY == ABR_POLICY_DYNAMIC) v.pol.dyn_mode[i] = (uint8_t)packed;
     if (hist) v.hist_len[i] = s.hist_len;
     if (sum.reset_mpc) { v.last_pred[i] = 0.0; v.err_len[i] = 0; }
     if (!FAST && s.done) v.done[i] = 1;
@@ -1644,7 +1667,13 @@ abr_policy_decide_kernel(EnvView v, int32_t* __restrict__ action) {
         ABR_CHECK(chunk >= 0 && chunk < v.V, "policy row");
         const int row = chunk * v.A;
         auto size_at = [&](const int a) -> double { return __ldg(v.sizes + row + a); };
-        q = POLICY == ABR_POLICY_RATE ? policy_rate(v, i, v.hist_len[i], size_at) : policy_bola(v, b, row, size_at);
+        if constexpr (POLICY == ABR_POLICY_DYNAMIC) {
+            const int m = dynamic_mode(v, chunk, b, v.pol.dyn_mode[i]);
+            v.pol.dyn_mode[i] = (uint8_t)m;
+            q = m ? policy_bola(v, b, row, size_at) : policy_rate(v, i, v.hist_len[i], size_at);
+        } else {
+            q = POLICY == ABR_POLICY_RATE ? policy_rate(v, i, v.hist_len[i], size_at) : policy_bola(v, b, row, size_at);
+        }
     }
     action[i] = q;
 }
@@ -1762,6 +1791,9 @@ cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action
         case ABR_POLICY_BBA: abr_policy_decide_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
         case ABR_POLICY_RATE: abr_policy_decide_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
         case ABR_POLICY_BOLA: abr_policy_decide_kernel<ABR_POLICY_BOLA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+        case ABR_POLICY_DYNAMIC:
+            abr_policy_decide_kernel<ABR_POLICY_DYNAMIC><<<grid, kStepBlock, 0, st>>>(v, d_action);
+            break;
         default: return cudaErrorInvalidValue;
     }
     count_launch();
@@ -1883,7 +1915,8 @@ static cudaError_t launch_rollout_form(const Go& go, const RolloutOut<OT>& o, co
                                        const bool live, const bool fast, const bool none, const bool uni) {
     constexpr bool kAhead = P == ABR_POLICY_FIXED || P == ABR_POLICY_RANDOM;
     if (live) return go(abr_rollout_kernel<P, false, false, true, false, OT>, o);
-    if constexpr (P == ABR_POLICY_RATE) {   // reads the history ring: track_history = 1, never a FAST / NOOUT form
+    // RATE and DYNAMIC read the history ring: track_history = 1, never a FAST / NOOUT form
+    if constexpr (P == ABR_POLICY_RATE || P == ABR_POLICY_DYNAMIC) {
         if (fast || none) return cudaErrorInvalidValue;
         return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);
     } else {
@@ -1930,6 +1963,9 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
         case ABR_POLICY_BBA: e = launch_rollout_form<ABR_POLICY_BBA>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_RATE: e = launch_rollout_form<ABR_POLICY_RATE>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_BOLA: e = launch_rollout_form<ABR_POLICY_BOLA>(go, o, o_none, live, fast, none, uni); break;
+        case ABR_POLICY_DYNAMIC:
+            e = launch_rollout_form<ABR_POLICY_DYNAMIC>(go, o, o_none, live, fast, none, uni);
+            break;
         default: return cudaErrorInvalidValue;
     }
     if (e != cudaSuccess) return e;

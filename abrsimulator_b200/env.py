@@ -15,14 +15,14 @@ import torch
 
 from . import _lib
 from ._lib import (AbrError, MPC_REF, MPC_ROBUST, NUM_ACC, NUM_STATS, POLICY_BBA, POLICY_BOLA,  # noqa: F401
-                   POLICY_FIXED, POLICY_RANDOM, POLICY_RATE, _addr)
+                   POLICY_DYNAMIC, POLICY_FIXED, POLICY_RANDOM, POLICY_RATE, _addr)
 from .datamodel import MPD, NetworkInfo, QOEMetric, pack_traces
 
 StepResult = namedtuple("StepResult", "delay sleep buffer rebuffer reward next_sizes end_of_video throughput latency",
                         defaults=(None,))
 
 _POLICIES = {"fixed": POLICY_FIXED, "random": POLICY_RANDOM, "bba": POLICY_BBA, "buffer": POLICY_BBA,
-             "rate": POLICY_RATE, "rb": POLICY_RATE, "bola": POLICY_BOLA}
+             "rate": POLICY_RATE, "rb": POLICY_RATE, "bola": POLICY_BOLA, "dynamic": POLICY_DYNAMIC}
 _MODES = {"reference": MPC_REF, "ref": MPC_REF, "robust": MPC_ROBUST}
 
 
@@ -515,9 +515,24 @@ class BatchedABREnv:
         _lib.check(self._lib.abr_env_set_policy_params(self._h, pp))
         self._policy_params = pp
 
+    # -- SPEC §4.6 --
+    def set_dynamic_params(self, switch_on_buffer=None, switch_off_buffer=None):
+        """Buffer thresholds of the "dynamic" policy (SPEC §4.6) for the following calls: the rate rule hands over to
+        BOLA above ``switch_on_buffer`` and BOLA hands back at or below ``switch_off_buffer``; arguments left at None
+        keep their current value (defaults: 12 s, 6 s).  Invalid values raise before anything changes."""
+        cur = getattr(self, "_dynamic_params", None)
+        if cur is None:
+            cur = _lib.AbrDynamicParams()
+            self._lib.abr_dynamic_params_default(cur)
+        dp = _lib.AbrDynamicParams(cur.switch_on_buffer if switch_on_buffer is None else float(switch_on_buffer),
+                                   cur.switch_off_buffer if switch_off_buffer is None else float(switch_off_buffer))
+        _lib.check(self._lib.abr_env_set_dynamic_params(self._h, dp))
+        self._dynamic_params = dp
+
     def policy_decide(self, policy, out=None) -> torch.Tensor:
-        """The action of a state-dependent built-in policy ("bba", "rate" or "bola") for every session, from the
-        environment's own state (int32 [N] on the device); ``step`` with it is one step of the fused episode."""
+        """The action of a state-dependent built-in policy ("bba", "rate", "bola" or "dynamic") for every session, from
+        the environment's own state (int32 [N] on the device); ``step`` with it is one step of the fused episode.
+        "dynamic" also records each session's active rule (``state("dyn_mode")``)."""
         pid = _policy_id(policy)
         act = self._empty(self.n, dtype=torch.int32) if out is None else out
         if act.dtype != torch.int32 or act.device != self.device or not act.is_contiguous() or act.numel() != self.n:

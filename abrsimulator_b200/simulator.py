@@ -21,7 +21,7 @@ Controllers
 * any object with ``get_next_bitrate(chunk_id, previous_bitrates, previous_bandwidths, buffer_level) -> int``
   (the protocol ``Simulator.run`` calls, ``Simulator.py:155``) is driven chunk by chunk through the step kernel;
 * the markers ``RandomPolicy(seed)`` / ``BufferBasedPolicy()`` / ``RateBasedPolicy()`` / ``BolaPolicy()`` /
-  ``FixedPolicy(actions)`` and this package's ``MPCBitrateController`` run fully on the device (fused episode kernel,
+  ``DynamicPolicy()`` / ``FixedPolicy(actions)`` and this package's ``MPCBitrateController`` run fully on the device (fused episode kernel,
   or decide+step kernels for MPC);
 * ``LookaheadPolicy(horizon)`` is the clairvoyant reference of SPEC §4.4 (decide+step kernels, on-demand mode only).
 """
@@ -58,6 +58,15 @@ class BolaPolicy:
     [min_buffer, target_buffer] in seconds."""
     def __init__(self, min_buffer=10.0, target_buffer=30.0):
         self.min_buffer, self.target_buffer = float(min_buffer), float(target_buffer)
+
+
+class DynamicPolicy:
+    """The rate rule while the buffer is low, BOLA once it is high (SPEC §4.6, in the manner of dash.js's DYNAMIC
+    strategy): BOLA takes over when the buffer exceeds ``switch_on_buffer`` and hands back when it no longer exceeds
+    ``switch_off_buffer``; ``safety`` is the rate rule's and ``min_buffer`` / ``target_buffer`` are BOLA's."""
+    def __init__(self, switch_on_buffer=12.0, switch_off_buffer=6.0, safety=1.0, min_buffer=10.0, target_buffer=30.0):
+        self.switch_on_buffer, self.switch_off_buffer = float(switch_on_buffer), float(switch_off_buffer)
+        self.safety, self.min_buffer, self.target_buffer = float(safety), float(min_buffer), float(target_buffer)
 
 
 class LookaheadPolicy:
@@ -125,25 +134,30 @@ class Simulator:
                 q.startup_weight * start_up_time + getattr(q, "latency_weight", 0.0) * average_latency)
 
     # -- environment --
-    _MARKERS = (RandomPolicy, BufferBasedPolicy, RateBasedPolicy, BolaPolicy, FixedPolicy)
+    _MARKERS = (RandomPolicy, BufferBasedPolicy, RateBasedPolicy, BolaPolicy, DynamicPolicy, FixedPolicy)
 
     @staticmethod
     def _marker_policy(ctrl):
         """The fused-episode policy name of a built-in policy marker (None: buffer-based)."""
         return ("random" if isinstance(ctrl, RandomPolicy) else "fixed" if isinstance(ctrl, FixedPolicy) else
-                "rate" if isinstance(ctrl, RateBasedPolicy) else "bola" if isinstance(ctrl, BolaPolicy) else "bba")
+                "rate" if isinstance(ctrl, RateBasedPolicy) else "bola" if isinstance(ctrl, BolaPolicy) else
+                "dynamic" if isinstance(ctrl, DynamicPolicy) else "bba")
 
     def _marker_env(self, ctrl, n_sessions, **extra):
         """The environment of a built-in policy marker, with the marker's parameters installed."""
         if isinstance(ctrl, BufferBasedPolicy):
             extra.update(bba_reservoir=ctrl.reservoir, bba_cushion=ctrl.cushion)
-        if isinstance(ctrl, RateBasedPolicy):
+        if isinstance(ctrl, (RateBasedPolicy, DynamicPolicy)):
             extra.update(track_history=1)             # the rate-based rule reads the throughput history
         env = self._make_env(n_sessions, **extra)
         if isinstance(ctrl, RateBasedPolicy):
             env.set_policy_params(rb_safety=ctrl.safety)
         elif isinstance(ctrl, BolaPolicy):
             env.set_policy_params(bola_min_buffer=ctrl.min_buffer, bola_target_buffer=ctrl.target_buffer)
+        elif isinstance(ctrl, DynamicPolicy):
+            env.set_policy_params(rb_safety=ctrl.safety, bola_min_buffer=ctrl.min_buffer,
+                                  bola_target_buffer=ctrl.target_buffer)
+            env.set_dynamic_params(switch_on_buffer=ctrl.switch_on_buffer, switch_off_buffer=ctrl.switch_off_buffer)
         return env
 
     def _make_env(self, n_sessions, **extra):
