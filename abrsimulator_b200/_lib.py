@@ -52,6 +52,11 @@ class AbrDynamicParams(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("switch_on_buffer", "switch_off_buffer")]
 
 
+class AbrSpeedParams(C.Structure):
+    """The catch-up speed controller of live mode (SPEC §7.2, include/abr_b200_speed.h)."""
+    _fields_ = [(n, C.c_double) for n in ("target_latency", "max_drift", "gain", "dead_band", "min_buffer")]
+
+
 class AbrObsSpec(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
 
@@ -134,6 +139,14 @@ DYNAMIC_SIGNATURES = {
     "abr_dynamic_params_default": (None, [_DYNAMIC_PARAMS]),
     "abr_env_set_dynamic_params": (_I, [_P, _DYNAMIC_PARAMS]),
 }
+# include/abr_b200_speed.h: the catch-up speed controller of live mode (SPEC §7.2).  Its state field exists on live
+# environments only and has a table of its own next to FIELDS.
+SPEED_FIELDS = dict(play_speed=(25, "float64"))
+_SPEED_PARAMS = C.POINTER(AbrSpeedParams)
+SPEED_SIGNATURES = {
+    "abr_speed_params_default": (None, [_SPEED_PARAMS]),
+    "abr_env_set_speed_control": (_I, [_P, _SPEED_PARAMS]),
+}
 
 _lib = None
 
@@ -154,7 +167,7 @@ def load():
         _build.build_library()
     lib = C.CDLL(path)
     for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES,
-                                   **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES}.items():
+                                   **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES, **SPEED_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -15,6 +15,7 @@
 #include "../../include/abr_b200_mpc_pred.h"
 #include "../../include/abr_b200_mpc_scen.h"
 #include "../../include/abr_b200_obs.h"
+#include "../../include/abr_b200_speed.h"
 
 namespace abr {
 static std::atomic<long long> g_launches{0};
@@ -206,6 +207,22 @@ static int check_dynamic_params(const AbrDynamicParams* dp) {
     return ABR_OK;
 }
 
+void abr_speed_params_default(AbrSpeedParams* p) {
+    if (!p) return;
+    p->target_latency = 12.0; p->max_drift = 0.5; p->gain = 2.5; p->dead_band = 0.02; p->min_buffer = 6.0;
+}
+
+static int check_speed_params(const AbrSpeedParams* sp) {
+    const double x[5] = {sp->target_latency, sp->max_drift, sp->gain, sp->dead_band, sp->min_buffer};
+    for (double d : x)
+        if (!std::isfinite(d)) return fail(ABR_ERR_INVALID, "speed control parameters must be finite");
+    if (!(sp->target_latency >= 0.0) || !(sp->max_drift > 0.0) || !(sp->max_drift < 1.0) || !(sp->gain > 0.0) ||
+        !(sp->dead_band >= 0.0) || !(sp->min_buffer >= 0.0))
+        return fail(ABR_ERR_INVALID, "need target_latency >= 0, 0 < max_drift < 1, gain > 0, dead_band >= 0 and "
+                                     "min_buffer >= 0");
+    return ABR_OK;
+}
+
 static int check_tables(const double* sizes, const double* bitrates, int V, int A) {
     if (!sizes || !bitrates) return fail(ABR_ERR_INVALID, "sizes/bitrates is NULL");
     if (V < 1 || A < 1 || A > 16) return fail(ABR_ERR_RANGE, "need V >= 1 and 1 <= A <= 16 (got V=%d A=%d)", V, A);
@@ -336,6 +353,10 @@ int abr_env_create(const double* h_trace_bw, const int32_t* h_trace_len, const d
         CUDA_TRY(e->alloc(&v.pol.dyn_mode, cap));
         CUDA_TRY(cudaMemset(v.pol.dyn_mode, 0, cap));
     }
+    if (params->live) {   // the speed controller's decisions (SPEC §7.2); the controller needs live mode
+        CUDA_TRY(e->alloc(&v.spd.play_speed, cap));
+        CUDA_TRY(cudaMemset(v.spd.play_speed, 0, sizeof(double) * cap));
+    }
     e->n_partials_cap = stats_num_partials(max_sessions) > rollout_num_blocks(max_sessions)
                             ? stats_num_partials(max_sessions) : rollout_num_blocks(max_sessions);
     CUDA_TRY(e->alloc(&e->d_stats_partials, (size_t)e->n_partials_cap * ABR_NUM_ACC));
@@ -444,6 +465,26 @@ int abr_env_set_dynamic_params(AbrEnv* env, const AbrDynamicParams* params) {
     return ABR_OK;
 }
 
+int abr_env_set_speed_control(AbrEnv* env, const AbrSpeedParams* params) {
+    if (params)
+        if (int rc = check_speed_params(params)) return rc;   // host-side only: reported without a device
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (!env->v.p.live) return fail(ABR_ERR_STATE, "speed control belongs to live mode (SPEC 7.2): create the environment with live = 1");
+    EnvView::SpeedControl& c = env->v.spd;
+    c.on = params ? 1 : 0;
+    if (params) {
+        c.target_latency = params->target_latency; c.max_drift = params->max_drift; c.gain = params->gain;
+        c.dead_band = params->dead_band; c.min_buffer = params->min_buffer;
+    }
+    return ABR_OK;
+}
+
+// A speed table where the speed controller decides (SPEC §7.2).
+static int check_speed_table(const AbrEnv* env, const double* d_speed) {
+    if (d_speed && env->v.spd.on) return fail(ABR_ERR_INVALID, "a speed table and the speed controller are exclusive");
+    return ABR_OK;
+}
+
 int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stream) {
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
     if (policy != ABR_POLICY_BBA && policy != ABR_POLICY_RATE && policy != ABR_POLICY_BOLA && policy != ABR_POLICY_DYNAMIC)
@@ -535,6 +576,7 @@ static int env_step_any(AbrEnv* env, const int32_t* d_action, const double* d_sp
                         OT* d_buffer, OT* d_rebuf, OT* d_reward, OT* d_latency, OT* d_next_sizes,
                         uint8_t* d_end_of_video, OT* d_throughput, void* stream) {
     if (int rc = check_reset(env)) return rc;
+    if (int rc = check_speed_table(env, d_speed)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
     env->fresh_partials = 0;
@@ -666,6 +708,7 @@ static int env_rollout_any(AbrEnv* env, int policy, uint64_t seed, int steps, co
                            const double* d_speed, OT* d_delay, OT* d_sleep, OT* d_buffer, OT* d_rebuf, OT* d_reward,
                            OT* d_latency, uint8_t* d_end_of_video, int32_t* d_actions_out, void* stream) {
     if (int rc = check_reset(env)) return rc;
+    if (int rc = check_speed_table(env, d_speed)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
     if (int rc_p = check_policy(env, policy)) return rc_p;
@@ -841,6 +884,9 @@ int abr_env_state_ptr(AbrEnv* env, int field, void** d_ptr) {
         case ABR_F_DYN_MODE:
             if (!v.pol.dyn_mode) return fail(ABR_ERR_STATE, "dyn_mode needs track_history = 1");
             *d_ptr = v.pol.dyn_mode; break;
+        case ABR_F_PLAY_SPEED:
+            if (!v.spd.play_speed) return fail(ABR_ERR_STATE, "play_speed needs live = 1");
+            *d_ptr = v.spd.play_speed; break;
         default: return fail(ABR_ERR_INVALID, "unknown state field %d", field);
     }
     return ABR_OK;

@@ -135,6 +135,15 @@ struct EnvView {
         double dyn_on, dyn_off;
         double pad_;
     } pol;
+    // Catch-up speed control (SPEC §7.2): the speed of the chunk each live session is playing (allocated with
+    // live = 1), the controller's parameters and whether it is installed.  Last and 64 bytes, for the reasons given
+    // at Policy: the fields above keep their offsets and the parameters behind an EnvView their 16-byte alignment.
+    struct SpeedControl {
+        double* play_speed;
+        double target_latency, max_drift, gain, dead_band, min_buffer;
+        int32_t on;
+        int32_t pad_[3];
+    } spd;
 };
 
 // launchers implemented in abr_step.cu / abr_mpc.cu (C++ linkage, internal)
@@ -183,7 +192,8 @@ cudaError_t launch_step_policy(const EnvView& v, const StepPolicyWindow& pol, co
                                uint32_t* d_draw_counter, cudaStream_t st);
 // abr_env_observe_window (SPEC §4.5): the windowed observation of the state, both windows 0; pol.window and pol.obs set
 cudaError_t launch_observe_window(const EnvView& v, const StepPolicyWindow& pol, cudaStream_t st);
-// d_speed (live mode): the playback speed of content chunk k of session i is d_speed[k * N + i]; nullable = 1.0
+// d_speed (live mode): the playback speed of content chunk k of session i is d_speed[k * N + i]; nullable = 1.0.
+// With v.spd.on (live mode only) the catch-up controller of SPEC §7.2 decides the speeds instead; d_speed is null then.
 template <typename OT>
 cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double* d_speed, const StepOutputs<OT>& o,
                         cudaStream_t st, const StepPolicyWindow* policy = nullptr);

@@ -74,6 +74,8 @@ struct Sess {
     double t_now, play_time, play_len;   // wall clock, content played, content played of the chunk being played
     const double* __restrict__ speed;    // playback speed of content chunk k at speed[k * speed_stride] (null = 1.0)
     size_t speed_stride;
+    double play_speed;                   // LIVE = 2 (SPEC §7.2): the speed decided for chunk play_id
+    const EnvView::SpeedControl* ctl;    // LIVE = 2: the controller's parameters
     int play_id, V;                      // content chunk being played
     bool started, bad_speed;
 #ifdef ABR_CHECKED
@@ -207,13 +209,31 @@ __device__ __forceinline__ double position_of(const Sess& s, const int seg, cons
 // average_latency is that integral per tick (Simulator.py:179-180, see SPEC §7).
 struct LiveAcc { double startup, area, played, tc; };   // tc: wall clock inside the step
 
-__device__ __forceinline__ double live_speed(Sess& s) {
-    if (!s.speed) return 1.0;
-    const int k = s.play_id < s.V ? s.play_id : s.V - 1;
-    ABR_CHECK(k >= 0 && k < s.V, "playback-speed table row");
-    double v = __ldg(s.speed + (size_t)k * s.speed_stride);
-    if (!(v > 0.0)) { s.bad_speed = true; v = 1.0; }
-    return v;
+// LIVE: 1 = the speeds come from the caller's [V][N] table, 2 = the catch-up controller of SPEC §7.2 decides the speed
+// of a chunk when it starts to play, from the latency at wall clock tc and the buffer at that instant.
+template <int LIVE>
+__device__ __forceinline__ double live_speed(Sess& s, const double tc, const double buffer) {
+    if constexpr (LIVE == 2) {
+        if (s.play_len == 0.0 || !(s.play_speed > 0.0)) {   // chunk play_id has not played yet, or no decision is stored
+            const EnvView::SpeedControl& c = *s.ctl;
+            const double e = dsub(dsub(tc, s.play_time), c.target_latency);
+            double v = 1.0;
+            if (!(fabs(e) <= c.dead_band)) {
+                const double y = dmul(c.gain, e);
+                v = dadd(1.0, dmul(c.max_drift, ddiv(y, dadd(1.0, fabs(y)))));
+            }
+            if (v > 1.0 && buffer < c.min_buffer) v = 1.0;   // never speed up into a stall
+            s.play_speed = v;
+        }
+        return s.play_speed;
+    } else {
+        if (!s.speed) return 1.0;
+        const int k = s.play_id < s.V ? s.play_id : s.V - 1;
+        ABR_CHECK(k >= 0 && k < s.V, "playback-speed table row");
+        double v = __ldg(s.speed + (size_t)k * s.speed_stride);
+        if (!(v > 0.0)) { s.bad_speed = true; v = 1.0; }
+        return v;
+    }
 }
 
 // one stretch: d seconds of content in dw seconds of wall time at speed v
@@ -227,11 +247,12 @@ __device__ __forceinline__ void live_piece(Sess& s, double& buffer, LiveAcc& a, 
 }
 
 // playback during dt seconds of wall time; returns the stall time
+template <int LIVE>
 __device__ __forceinline__ double live_play_wall(Sess& s, double& buffer, LiveAcc& a, const double dt, const double L) {
     if (!s.started) { a.startup = dadd(a.startup, dt); a.tc = dadd(a.tc, dt); return 0.0; }
     double rem = dt;
     while (rem > 0.0 && buffer > 0.0) {
-        const double v = live_speed(s);
+        const double v = live_speed<LIVE>(s, a.tc, buffer);
         const double room = dsub(L, s.play_len);
         const double can = room < buffer ? room : buffer;
         const double need = dmul(v, rem);
@@ -254,10 +275,11 @@ __device__ __forceinline__ double live_play_wall(Sess& s, double& buffer, LiveAc
 }
 
 // playback until x seconds of content have drained (x <= buffer); returns the wall time it takes
+template <int LIVE>
 __device__ __forceinline__ double live_play_content(Sess& s, double& buffer, LiveAcc& a, double x, const double L) {
     double w = 0.0;
     while (x > 0.0) {
-        const double v = live_speed(s);
+        const double v = live_speed<LIVE>(s, a.tc, buffer);
         const double room = dsub(L, s.play_len);
         const bool finished = room <= x;
         const double d = finished ? room : x;
@@ -359,16 +381,16 @@ __device__ __forceinline__ void head(const Sess& s, const double raw, Head& h, b
 // position by the idle time.  Runs before the head of a live step.
 struct LiveGate { double buffer, rebuf, idle; LiveAcc a; };
 
-template <bool SMEM>
+template <bool SMEM, int LIVE>
 __device__ __forceinline__ void live_gate(const EnvView& v, Sess& s, LiveGate& g) {
     const AbrParams& p = v.p;
     g.buffer = s.buffer;
     g.a.startup = g.a.area = g.a.played = 0.0;
     g.a.tc = s.t_now;
     const double w1 = max0(dsub(dmul((double)(s.chunk + 1), p.chunk_length), s.t_now));
-    g.rebuf = live_play_wall(s, g.buffer, g.a, w1, p.chunk_length);
+    g.rebuf = live_play_wall<LIVE>(s, g.buffer, g.a, w1, p.chunk_length);
     const double w2 = (s.started && g.buffer > p.max_buffer)
-                          ? live_play_content(s, g.buffer, g.a, dsub(g.buffer, p.max_buffer), p.chunk_length) : 0.0;
+                          ? live_play_content<LIVE>(s, g.buffer, g.a, dsub(g.buffer, p.max_buffer), p.chunk_length) : 0.0;
     g.idle = dadd(w1, w2);
     if (g.idle > 0.0) {
         advance_trace(s.seg, s.phi, g.idle, s.I, s.inv_I, s.T);
@@ -379,11 +401,11 @@ __device__ __forceinline__ void live_gate(const EnvView& v, Sess& s, LiveGate& g
 // ---- tail of a step (SPEC §3.1 from the division on, §3.2-§3.5) for one session held in registers ----
 // `q` must already be a valid index; `lk` holds the step's table reads, `h` its head.
 // FAST: auto_reset is on (a session is never inert) — drops the done/inert bookkeeping.
-// LIVE: live-streaming semantics of SPEC §7 (`g` = the step's pause gate).
+// LIVE: live-streaming semantics of SPEC §7 (`g` = the step's pause gate); 2 = with the speed controller of §7.2.
 // Returns true when the step moved the trace position in time (sleep): s.pos was then recomputed from (seg, phi)
 // and a head issued ahead for the next step is stale.
 // `p` / `V`: the environment's parameters and chunk count; inv_q = pow2_inverse(p.sleep_quantum).
-template <bool SMEM, bool FAST, bool LIVE>
+template <bool SMEM, bool FAST, int LIVE>
 __device__ __forceinline__ bool step_tail(const AbrParams& p, const int V, Sess& s, const Head& h, const int q,
                                           const Lookup& lk, const LiveGate& g, StepRes& r, const bool want_thr,
                                           const double inv_q) {
@@ -413,7 +435,7 @@ __device__ __forceinline__ bool step_tail(const AbrParams& p, const int V, Sess&
     if (LIVE) {   // 7.2
         double live_buffer = g.buffer;
         LiveAcc a = g.a;
-        rebuf = dadd(g.rebuf, live_play_wall(s, live_buffer, a, delay, p.chunk_length));
+        rebuf = dadd(g.rebuf, live_play_wall<LIVE>(s, live_buffer, a, delay, p.chunk_length));
         buffer = dadd(live_buffer, p.chunk_length);
         s.t_now = dadd(dadd(s.t_now, g.idle), delay);
         if (!s.started && buffer >= p.start_up_length) s.started = true;
@@ -468,7 +490,7 @@ __device__ __forceinline__ bool step_tail(const AbrParams& p, const int V, Sess&
 }
 
 // One whole step (gate, head, tail) — the per-step kernel's form.
-template <bool SMEM, bool FAST, bool LIVE>
+template <bool SMEM, bool FAST, int LIVE>
 __device__ __forceinline__ void step_core(const EnvView& v, Sess& s, const int q, const Lookup& lk, StepRes& r,
                                           const bool want_thr) {
     r.walk_error = false;
@@ -479,7 +501,7 @@ __device__ __forceinline__ void step_core(const EnvView& v, Sess& s, const int q
     if (!FAST && s.done) {
         h.target = h.c_j = h.kx = 0.0; h.c_j1 = 1.0; h.j = 0;
     } else {
-        if (LIVE) live_gate<SMEM>(v, s, g);
+        if (LIVE) live_gate<SMEM, LIVE>(v, s, g);
         head<SMEM>(s, dadd(s.pos, lk.size), h, r.walk_error);
     }
     step_tail<SMEM, FAST, LIVE>(v.p, v.V, s, h, q, lk, g, r, want_thr, pow2_inverse(v.p.sleep_quantum));
@@ -787,7 +809,9 @@ __device__ __forceinline__ int policy_action(const EnvView& v, const StepPolicy&
 }
 
 // Live-mode words of session i (SPEC §7): from the SoA state, or those of a fresh reset.  speed: the [V][N] table of
-// playback speeds (the speed of content chunk k is speed[k][i]), nullable = 1.0.
+// playback speeds (the speed of content chunk k is speed[k][i]), nullable = 1.0.  LIVE = 2: the speed controller's
+// stored decision instead (SPEC §7.2; a reset does not touch it, and a fresh session decides at its first piece).
+template <int LIVE>
 __device__ __forceinline__ void load_live(const EnvView& v, Sess& s, const int i, const double* __restrict__ speed,
                                           const bool fresh) {
     if (fresh) { s.t_now = 0.0; s.play_time = 0.0; s.play_len = 0.0; s.play_id = 0; s.started = v.p.start_up_length <= 0.0; }
@@ -797,10 +821,11 @@ __device__ __forceinline__ void load_live(const EnvView& v, Sess& s, const int i
     }
     s.speed = speed ? speed + i : nullptr;
     s.speed_stride = (size_t)v.n; s.V = v.V; s.bad_speed = false;
+    if constexpr (LIVE == 2) { s.play_speed = v.spd.play_speed[i]; s.ctl = &v.spd; }
 }
 
 // The SoA state words a step changes (LIVE: with the live-mode ones).
-template <bool LIVE>
+template <int LIVE>
 __device__ __forceinline__ void store_state(const EnvView& v, const Sess& s, const int i) {
     v.seg[i] = s.seg; v.chunk[i] = s.chunk; v.last_q[i] = s.last_q; v.phi[i] = s.phi; v.pos[i] = s.pos;
     v.buffer[i] = s.buffer;
@@ -808,12 +833,13 @@ __device__ __forceinline__ void store_state(const EnvView& v, const Sess& s, con
         v.t_now[i] = s.t_now; v.play_time[i] = s.play_time; v.started[i] = s.started ? 1 : 0;
         v.play_id[i] = s.play_id; v.play_len[i] = s.play_len;
     }
+    if constexpr (LIVE == 2) v.spd.play_speed[i] = s.play_speed;
 }
 
 // A step's trajectory outputs at element ix of [steps][N], streamed out (st.global.cs).  FAST: the five f64 outputs and
 // end_of_video are all requested and stored without null checks; NOOUT: none is requested; LIVE: the latency too,
 // where requested.
-template <bool FAST, bool NOOUT, bool LIVE, typename OT>
+template <bool FAST, bool NOOUT, int LIVE, typename OT>
 __device__ __forceinline__ void store_step(const StepOutputs<OT>& o, const uint32_t ix, const StepRes& r) {
     if (NOOUT) {
     } else if (FAST) {
@@ -892,13 +918,13 @@ template <int POL> struct PolicyArg { using type = StepPolicy; };
 template <> struct PolicyArg<2> { using type = StepPolicyWindow; };
 template <int POL> using PolicyArgs = typename PolicyArg<POL>::type;
 
-template <bool SMEM, bool FAST, bool LIVE, int POL, typename OT>
+template <bool SMEM, bool FAST, int LIVE, int POL, typename OT>
 __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const int i, const int q, const Lookup& lk,
                                              const PolicyArgs<POL>& pol, const double* __restrict__ speed,
                                              OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer,
                                              OT* __restrict__ o_rebuf, OT* __restrict__ o_reward, uint8_t* __restrict__ o_eov,
                                              OT* __restrict__ o_latency, OT* __restrict__ o_thr, OT* __restrict__ o_next_sizes) {
-    if (LIVE) load_live(v, s, i, speed, false);
+    if (LIVE) load_live<LIVE>(v, s, i, speed, false);
     StepRes r;
     step_core<SMEM, FAST, LIVE>(v, s, q, lk, r, (!FAST && v.p.track_history) || o_thr != nullptr || (POL && pol.obs));
     if (r.walk_error || (LIVE && s.bad_speed)) atomicAdd(v.errors, 1ull);
@@ -976,7 +1002,8 @@ __device__ __forceinline__ void step_session(const EnvView& v, Sess& s, const in
 // that trace are LDS.  Every other lane reads the L2-resident tables directly (one index pair + one or two sectors of C).
 // POL: the actions come from the caller's logits (policy_action) instead of `action`, and the kernel also writes the
 // next observation (POL = 1: SPEC §4.1; POL = 2: the windowed observation of §4.5); never with FAST or LIVE.
-template <bool FAST, bool LIVE, int POL, typename OT>
+// LIVE: 1 = live mode with the caller's speed table, 2 = with the speed controller of SPEC §7.2.
+template <bool FAST, int LIVE, int POL, typename OT>
 __global__ void __launch_bounds__(kTile, (LIVE || POL) ? 4 : kTileBlocksPerSM)
 abr_step_kernel(EnvView v, const int32_t* __restrict__ action, const double* __restrict__ speed,
                 OT* __restrict__ o_delay, OT* __restrict__ o_sleep, OT* __restrict__ o_buffer, OT* __restrict__ o_rebuf,
@@ -1242,7 +1269,7 @@ struct EpisodeSums {
 
 // Adds one (not inert) step.  COUNT: count it and its end of episode here, note an auto-reset and record the
 // throughput sample in the history ring (hist); without COUNT the caller has all of that in closed form.
-template <bool LIVE, bool COUNT>
+template <int LIVE, bool COUNT>
 __device__ __forceinline__ void add_step(EpisodeSums& a, const StepRes& r, const EnvView& v, const Sess& s, const int i,
                                          const bool hist) {
     a.rew = dadd(a.rew, r.reward); a.reb = dadd(a.reb, r.rebuf); a.u = dadd(a.u, r.u);
@@ -1260,7 +1287,8 @@ __device__ __forceinline__ void add_step(EpisodeSums& a, const StepRes& r, const
 // FAST: the common shape — all six trajectory outputs requested, no action trace, no throughput history,
 // auto_reset on — compiled without the per-output null checks and the inert/history bookkeeping.
 // NOOUT (with FAST): no trajectory output at all (statistics / per-session accumulators only, e.g. abr_env_run_host).
-// LIVE (never with FAST): live-streaming semantics of SPEC §7.
+// LIVE (never with FAST): live-streaming semantics of SPEC §7; 2 = with the speed controller of §7.2, whose decision
+// for the chunk being played stays in a register for the whole call (load_live / store_state).
 //
 // Software pipeline (policies whose action does not depend on the state: FIXED, RANDOM; not LIVE, whose pause gate
 // moves the position before every download): iteration t holds the finished head of step t and issues the head of
@@ -1270,7 +1298,7 @@ __device__ __forceinline__ void add_step(EpisodeSums& a, const StepRes& r, const
 // The action and table reads run two steps ahead for the same reason.
 // UNI (with FAST, policies that run ahead): every chunk has the same utility row, so the previous step's utility is
 // the next step's "previous utility" (SPEC §3.4) — carried in a register instead of looked up.
-template <int POLICY, bool SMEM, bool FAST, bool NOOUT, bool LIVE, bool UNI, typename OT>
+template <int POLICY, bool SMEM, bool FAST, bool NOOUT, int LIVE, bool UNI, typename OT>
 __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const int i, const uint32_t seed_lo,
                                                 const uint32_t seed_hi, const int steps, const uint32_t step_base,
                                                 const int32_t* __restrict__ actions_in, const RolloutOut<OT>& o,
@@ -1289,7 +1317,7 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     // register is shared, and every DYNAMIC statement is an `if constexpr`, so that the other policies' forms compile
     // to the instructions they compiled to before DYNAMIC existed.)
     if constexpr (POLICY == ABR_POLICY_DYNAMIC) packed = v.pol.dyn_mode[i];
-    if (LIVE) load_live(v, s, i, o.speed, fresh);
+    if (LIVE) load_live<LIVE>(v, s, i, o.speed, fresh);
     // SPEC §4 action of step t; must be called with increasing t.  FIXED clamps t to the last row so that the
     // calls that run ahead of the final step stay inside the caller's table.
     auto action_at = [&](const int t) -> int {
@@ -1463,7 +1491,7 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
 // is followed by the index row (idx_stride(T_max) 16-bit words, 16-byte aligned) and the sizes and utility tables.
 // 8 blocks (16 warps) per SM: <= 128 registers, so that the 1 024 blocks of the 65 536-session shape are all
 // co-resident (6.9 per SM).
-template <int POLICY, bool FAST, bool NOOUT, bool LIVE, bool UNI, typename OT>
+template <int POLICY, bool FAST, bool NOOUT, int LIVE, bool UNI, typename OT>
 #ifndef ABR_ROLLOUT_MINBLOCKS
 #define ABR_ROLLOUT_MINBLOCKS 8   // <= 128 registers.  Registers are allocated per warp in steps of 32 per thread, so 129..160
                                   // registers mean 12 warps = six 64-thread blocks per SM (measured: 140 and 144 registers
@@ -1862,6 +1890,7 @@ cudaError_t launch_step(const EnvView& v, const int32_t* d_action, const double*
             e = pol.window > 0 ? go(abr_step_kernel<false, false, 2, OT>) : go(abr_step_kernel<false, false, 1, OT>);
         else return cudaErrorInvalidValue;
     }
+    else if (live && v.spd.on) e = go(abr_step_kernel<false, 2, 0, OT>);
     else if (live) e = go(abr_step_kernel<false, true, 0, OT>);
     else if (fast) e = go(abr_step_kernel<true, false, 0, OT>);
     else e = go(abr_step_kernel<false, false, 0, OT>);
@@ -1909,11 +1938,13 @@ cudaError_t launch_observe_window(const EnvView& v, const StepPolicyWindow& pol,
 
 // The episode kernel's compile-time form for policy P, launched by go(kernel, outputs).  The carried-utility form
 // (UNI) only exists where it pays: the run-ahead loop (not the buffer-based policy).  NOOUT stores no trajectory, so
-// its output type is never used: the double form serves the fp32 calls too.
+// its output type is never used: the double form serves the fp32 calls too.  live: 0 = VoD, 1 = live mode with a
+// speed table, 2 = with the speed controller of SPEC §7.2.
 template <int P, typename OT, typename Go>
 static cudaError_t launch_rollout_form(const Go& go, const RolloutOut<OT>& o, const RolloutOut<double>& o_none,
-                                       const bool live, const bool fast, const bool none, const bool uni) {
+                                       const int live, const bool fast, const bool none, const bool uni) {
     constexpr bool kAhead = P == ABR_POLICY_FIXED || P == ABR_POLICY_RANDOM;
+    if (live == 2) return go(abr_rollout_kernel<P, false, false, 2, false, OT>, o);
     if (live) return go(abr_rollout_kernel<P, false, false, true, false, OT>, o);
     // RATE and DYNAMIC read the history ring: track_history = 1, never a FAST / NOOUT form
     if constexpr (P == ABR_POLICY_RATE || P == ABR_POLICY_DYNAMIC) {
@@ -1938,7 +1969,7 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
     double* out_stats = d_block_partials ? f.out_stats : nullptr;
     const RolloutOut<OT> o{out, d_speed, f.in_trace_id, f.in_offset, f.out_cost, out_stats, f.scratch};
     const RolloutOut<double> o_none{StepOutputs<double>{}, d_speed, f.in_trace_id, f.in_offset, f.out_cost, out_stats, f.scratch};
-    const bool live = v.p.live != 0;
+    const int live = v.p.live == 0 ? 0 : (v.spd.on ? 2 : 1);
     // shared-memory buffer: the longest C row, the longest index row and the two tables
     int smem_doubles = cum_smem_doubles(v.T_max);
     size_t smem_bytes = ((size_t)smem_doubles + 2 * (size_t)v.V * v.A) * sizeof(double) +

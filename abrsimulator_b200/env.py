@@ -302,6 +302,7 @@ class BatchedABREnv:
         if speed is not None:
             if not live:
                 raise ValueError("speed is a live-mode action (create the environment with live=1)")
+            self._check_no_speed_control()
             v = self._speed_table(speed, n)
         if want_latency is None:
             want_latency = live
@@ -442,6 +443,7 @@ class BatchedABREnv:
         if speed is not None:
             if not self.params.live:
                 raise ValueError("speed is a live-mode action (create the environment with live=1)")
+            self._check_no_speed_control()
             v = self._speed_table(speed, n)
         if out is None:
             out = {}
@@ -528,6 +530,36 @@ class BatchedABREnv:
                                    cur.switch_off_buffer if switch_off_buffer is None else float(switch_off_buffer))
         _lib.check(self._lib.abr_env_set_dynamic_params(self._h, dp))
         self._dynamic_params = dp
+
+    # -- SPEC §7.2 --
+    def set_speed_control(self, params=(), **kw):
+        """Install the catch-up speed controller of live mode (SPEC §7.2) for the following calls, or remove it with
+        ``set_speed_control(None)``.  While it is installed, every live step and episode decides the playback speed
+        of each content chunk when the chunk starts to play, from the latency and the buffer at that instant, in
+        place of a ``speed`` table (passing one then raises).  Keyword arguments: ``target_latency`` [12 s],
+        ``max_drift`` [0.5], ``gain`` [2.5 /s], ``dead_band`` [0.02 s], ``min_buffer`` [6 s]; omitted ones take
+        their defaults.  Invalid values raise before anything changes."""
+        if params is None:
+            if kw:
+                raise TypeError("set_speed_control(None) removes the controller and takes no parameters")
+            _lib.check(self._lib.abr_env_set_speed_control(self._h, None))
+            self._speed_params = None
+            return
+        if params != ():
+            raise TypeError("set_speed_control takes keyword arguments, or None to remove the controller")
+        sp = _lib.AbrSpeedParams()
+        self._lib.abr_speed_params_default(sp)
+        for k, x in kw.items():
+            if k not in dict(_lib.AbrSpeedParams._fields_):
+                raise TypeError(f"unknown speed control parameter {k!r}")
+            setattr(sp, k, float(x))
+        _lib.check(self._lib.abr_env_set_speed_control(self._h, sp))
+        self._speed_params = sp
+
+    def _check_no_speed_control(self):
+        if getattr(self, "_speed_params", None) is not None:
+            raise ValueError("a speed table and the speed controller are exclusive: remove the controller with "
+                             "set_speed_control(None) to play a table")
 
     def policy_decide(self, policy, out=None) -> torch.Tensor:
         """The action of a state-dependent built-in policy ("bba", "rate", "bola" or "dynamic") for every session, from
@@ -719,7 +751,7 @@ class BatchedABREnv:
 
     def state(self, name) -> torch.Tensor:
         """Zero-copy view of a state field (library-owned device memory)."""
-        fid, dt = _lib.FIELDS[name]
+        fid, dt = _lib.FIELDS[name] if name in _lib.FIELDS else _lib.SPEED_FIELDS[name]
         p = np.zeros(1, np.uintp)
         _lib.check(self._lib.abr_env_state_ptr(self._h, fid, _addr(p)))
         cap = self.capacity

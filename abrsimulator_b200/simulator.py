@@ -24,6 +24,15 @@ Controllers
   ``DynamicPolicy()`` / ``FixedPolicy(actions)`` and this package's ``MPCBitrateController`` run fully on the device (fused episode kernel,
   or decide+step kernels for MPC);
 * ``LookaheadPolicy(horizon)`` is the clairvoyant reference of SPEC §4.4 (decide+step kernels, on-demand mode only).
+
+Speed controllers (live mode)
+-----------------------------
+* any object with ``get_next_speed() -> float`` (``Simulator.py:177``): its answers cannot depend on the session's
+  state, so they are drawn before the run into a ``[V, N]`` table, one per played chunk;
+* the marker ``CatchupSpeedController(target_latency, max_drift, gain, dead_band, min_buffer)`` is the closed-loop
+  catch-up rule of SPEC §7.2, installed on the environment (``BatchedABREnv.set_speed_control``): the kernels decide
+  each chunk's speed when it starts to play, from the latency and the buffer at that instant, on every live path
+  (MPC, the built-in policy markers, callback controllers).
 """
 from __future__ import annotations
 
@@ -67,6 +76,15 @@ class DynamicPolicy:
     def __init__(self, switch_on_buffer=12.0, switch_off_buffer=6.0, safety=1.0, min_buffer=10.0, target_buffer=30.0):
         self.switch_on_buffer, self.switch_off_buffer = float(switch_on_buffer), float(switch_off_buffer)
         self.safety, self.min_buffer, self.target_buffer = float(safety), float(min_buffer), float(target_buffer)
+
+
+class CatchupSpeedController:
+    """Latency catch-up of live mode (SPEC §7.2, in the manner of dash.js's catch-up rule): a chunk that starts to play
+    with the latency ``target_latency + e`` plays at ``1 + max_drift·y/(1+|y|)``, ``y = gain·e``, at 1 inside
+    ``|e| <= dead_band``, and never faster than 1 while the buffer is below ``min_buffer``."""
+    def __init__(self, target_latency=12.0, max_drift=0.5, gain=2.5, dead_band=0.02, min_buffer=6.0):
+        self.target_latency, self.max_drift, self.gain = float(target_latency), float(max_drift), float(gain)
+        self.dead_band, self.min_buffer = float(dead_band), float(min_buffer)
 
 
 class LookaheadPolicy:
@@ -226,15 +244,15 @@ class Simulator:
             env = self._make_env(n_sessions, track_history=1, **extra, **ctrl.extra_params)
             env.reset(tid, start_offset, session_base)
             mode = "robust" if ctrl.mode == MPC_ROBUST else "reference"
-            speed = self._speed_table(n_sessions, V)
+            speed = self._speed_for(env, n_sessions, V)
             for _ in range(V):
                 act = env.mpc_decide(ctrl.horizon, mode)
                 env.step(act, want_next_sizes=False, speed=speed)
         elif isinstance(ctrl, self._MARKERS) or ctrl is None:
-            # built-in policies: one fused live episode (abr_env_rollout_fused_live), speed table from the controller
+            # built-in policies: one fused live episode (abr_env_rollout_fused_live), speeds from the controller
             env = self._marker_env(ctrl, n_sessions, **extra)
             env.reset(tid, start_offset, session_base)
-            speed = self._speed_table(n_sessions, V)
+            speed = self._speed_for(env, n_sessions, V)
             env.rollout(self._marker_policy(ctrl), V, seed=getattr(ctrl, "seed", 0), actions=getattr(ctrl, "actions", None),
                         speed=speed, want=())
         else:
@@ -243,6 +261,14 @@ class Simulator:
         acc = env.session_acc().cpu().numpy()
         self.last_run = dict(zip(ACC_NAMES, acc))
         return env.qoe_cost().cpu().numpy()
+
+    def _speed_for(self, env, n_sessions, V):
+        """The speed table of the speed controller for a live run on ``env``; None (speed 1, or the catch-up marker,
+        which is installed on ``env`` instead)."""
+        if isinstance(self.speed_controller, CatchupSpeedController):
+            env.set_speed_control(**vars(self.speed_controller))
+            return None
+        return self._speed_table(n_sessions, V)
 
     def _speed_table(self, n_sessions, V):
         """[V, N] playback speeds: ``get_next_speed()`` is called once per content chunk of every session, in playing
@@ -280,7 +306,7 @@ class Simulator:
         marker = isinstance(ctrl, (RandomPolicy, BufferBasedPolicy, FixedPolicy))
         live = bool(env.params.live)
         env.reset(tid, start_offset, session_base)
-        speed = self._speed_table(n_sessions, V) if live else None
+        speed = self._speed_for(env, n_sessions, V) if live else None
         prev_q = [[] for _ in range(n_sessions)]
         prev_bw = [[] for _ in range(n_sessions)]
         buf = np.zeros(n_sessions)
