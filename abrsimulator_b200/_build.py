@@ -25,7 +25,8 @@ HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(CSRC, "abr_mpc_sea
            os.path.join(HERE, "..", "include", "abr_b200_mpc_scen.h"),
            os.path.join(HERE, "..", "include", "abr_b200_obs.h"),
            os.path.join(HERE, "..", "include", "abr_b200_dynamic.h"),
-           os.path.join(HERE, "..", "include", "abr_b200_speed.h")]
+           os.path.join(HERE, "..", "include", "abr_b200_speed.h"),
+           os.path.join(HERE, "..", "include", "abr_b200_session_params.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"] + os.environ.get("ABR_EXTRA_NVCC_FLAGS", "").split()

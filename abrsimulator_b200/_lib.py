@@ -57,6 +57,12 @@ class AbrSpeedParams(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("target_latency", "max_drift", "gain", "dead_band", "min_buffer")]
 
 
+class AbrSessionPolicyParams(C.Structure):
+    """Device pointers to the per-session policy parameters of SPEC §4.7 (include/abr_b200_session_params.h)."""
+    _fields_ = [(n, C.c_void_p) for n in ("d_bba_reservoir", "d_bba_cushion", "d_rb_safety", "d_bola_min_buffer",
+                                          "d_bola_target_buffer", "d_switch_on_buffer", "d_switch_off_buffer")]
+
+
 class AbrObsSpec(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("buffer_scale", "throughput_scale", "delay_scale", "size_scale")]
 
@@ -147,6 +153,15 @@ SPEED_SIGNATURES = {
     "abr_speed_params_default": (None, [_SPEED_PARAMS]),
     "abr_env_set_speed_control": (_I, [_P, _SPEED_PARAMS]),
 }
+# include/abr_b200_session_params.h: per-session parameters of the built-in policies (SPEC §4.7), fields in the order
+# of AbrSessionPolicyParams and of the getter's rows.
+SESSION_PARAM_FIELDS = ("bba_reservoir", "bba_cushion", "rb_safety", "bola_min_buffer", "bola_target_buffer",
+                        "switch_on_buffer", "switch_off_buffer")
+_SESSION_PARAMS = C.POINTER(AbrSessionPolicyParams)
+SESSION_PARAMS_SIGNATURES = {
+    "abr_env_set_session_policy_params": (_I, [_P, _SESSION_PARAMS, _I, _P]),
+    "abr_env_get_session_policy_params": (_I, [_P, _P, _I, _P]),
+}
 
 _lib = None
 
@@ -167,7 +182,8 @@ def load():
         _build.build_library()
     lib = C.CDLL(path)
     for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES,
-                                   **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES, **SPEED_SIGNATURES}.items():
+                                   **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES, **SPEED_SIGNATURES,
+                                   **SESSION_PARAMS_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

@@ -15,6 +15,7 @@
 #include "../../include/abr_b200_mpc_pred.h"
 #include "../../include/abr_b200_mpc_scen.h"
 #include "../../include/abr_b200_obs.h"
+#include "../../include/abr_b200_session_params.h"
 #include "../../include/abr_b200_speed.h"
 
 namespace abr {
@@ -90,6 +91,11 @@ struct AbrEnv {
     double* d_offset = nullptr;
     DeviceBuffer actions, reward_traj;        // abr_env_run_host's [steps][N] actions in and reward trajectory out
     double bola_vmax = 0.0;   // max over the log table of SPEC §4.3 (when every size is > 0, i.e. v.pol.bola_v is set)
+    AbrPolicyParams policy_params{};          // the environment-wide values installed last (SPEC §4.2, §4.3)
+    // per-session policy parameters (SPEC §4.7): the [kSessFields][cap] table v.sp.tab points into once allocated, and
+    // the validation's result word
+    double* d_sess = nullptr;
+    unsigned long long* d_sess_first = nullptr;
 
     ~AbrEnv() {
         for (void* p : allocs) cudaFree(p);
@@ -187,6 +193,7 @@ static int check_policy_params(const AbrPolicyParams* pp) {
 
 // SPEC §4.2 / §4.3 parameters (already validated): BOLA's (Vp, gp) derived from the buffer range as dash.js does
 static void install_policy_params(AbrEnv* env, const AbrPolicyParams* pp) {
+    env->policy_params = *pp;
     EnvView::Policy& pol = env->v.pol;
     pol.rb_safety = pp->rb_safety;
     pol.bola_vmax = env->bola_vmax;
@@ -450,9 +457,27 @@ static int check_policy(const AbrEnv* env, int policy) {
     return ABR_OK;
 }
 
+// The environment-wide knobs cannot change under installed per-session parameters (SPEC §4.7): the fields the caller
+// left out were filled in with the values current at installation.
+static int check_no_session_params(const AbrEnv* env, const char* name) {
+    if (env->v.sp.on)
+        return fail(ABR_ERR_STATE, "%s: per-session policy parameters are installed (remove them with "
+                                   "abr_env_set_session_policy_params(env, NULL, ...) first)", name);
+    return ABR_OK;
+}
+
+// A built-in-policy call on a batch of n sessions fits the per-session parameters installed for it, if any.
+static int check_session_params(const AbrEnv* env, int policy, int n_sessions) {
+    if (env->v.sp.on && policy >= ABR_POLICY_BBA && policy <= ABR_POLICY_DYNAMIC && env->v.sp.n != n_sessions)
+        return fail(ABR_ERR_STATE, "the installed per-session policy parameters cover %d sessions, the batch %d "
+                                   "(abr_env_set_session_policy_params)", env->v.sp.n, n_sessions);
+    return ABR_OK;
+}
+
 int abr_env_set_policy_params(AbrEnv* env, const AbrPolicyParams* params) {
     if (int rc = check_policy_params(params)) return rc;   // host-side only: bad values are reported without a device
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (int rc = check_no_session_params(env, "abr_env_set_policy_params")) return rc;
     install_policy_params(env, params);
     return ABR_OK;
 }
@@ -460,6 +485,7 @@ int abr_env_set_policy_params(AbrEnv* env, const AbrPolicyParams* params) {
 int abr_env_set_dynamic_params(AbrEnv* env, const AbrDynamicParams* params) {
     if (int rc = check_dynamic_params(params)) return rc;   // host-side only: bad values are reported without a device
     if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (int rc = check_no_session_params(env, "abr_env_set_dynamic_params")) return rc;
     env->v.pol.dyn_on = params->switch_on_buffer;
     env->v.pol.dyn_off = params->switch_off_buffer;
     return ABR_OK;
@@ -479,6 +505,56 @@ int abr_env_set_speed_control(AbrEnv* env, const AbrSpeedParams* params) {
     return ABR_OK;
 }
 
+static const char* const kSessFieldNames[7] = {"bba_reservoir", "bba_cushion", "rb_safety", "bola_min_buffer",
+                                                "bola_target_buffer", "switch_on_buffer", "switch_off_buffer"};
+
+int abr_env_set_session_policy_params(AbrEnv* env, const AbrSessionPolicyParams* params, int n_sessions,
+                                      void* stream) {
+    if (!env) return fail(ABR_ERR_INVALID, "env is NULL");
+    if (!params) { env->v.sp.on = 0; env->v.sp.n = 0; return ABR_OK; }
+    if (n_sessions < 1 || n_sessions > env->v.cap)
+        return fail(ABR_ERR_RANGE, "n_sessions must be in [1, %d] (got %d)", env->v.cap, n_sessions);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!env->d_sess) {   // first installation: the table never moves afterwards, so captured graphs stay valid
+        CUDA_TRY(env->alloc(&env->d_sess, (size_t)kSessFields * env->v.cap));
+        CUDA_TRY(env->alloc(&env->d_sess_first, 1));
+    }
+    const EnvView& v = env->v;
+    const AbrPolicyParams& pp = env->policy_params;
+    SessionParamsSrc a{{params->d_bba_reservoir, params->d_bba_cushion, params->d_rb_safety, params->d_bola_min_buffer,
+                        params->d_bola_target_buffer, params->d_switch_on_buffer, params->d_switch_off_buffer},
+                       {v.p.bba_reservoir, v.p.bba_cushion, pp.rb_safety, pp.bola_min_buffer, pp.bola_target_buffer,
+                        v.pol.dyn_on, v.pol.dyn_off},
+                       env->bola_vmax};
+    // validate everything before writing anything, so that a failed call leaves the installed table as it was
+    unsigned long long first = 0;
+    CUDA_TRY(launch_session_params(a, n_sessions, v.cap, env->d_sess, env->d_sess_first, st));
+    CUDA_TRY(cudaMemcpyAsync(&first, env->d_sess_first, sizeof(first), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (first != ~0ull) {
+        const int s = (int)(first / 8), f = (int)(first % 8);
+        static const char* const need[7] = {"finite", "finite and > 0", "finite and > 0", "finite and > 0",
+                                            "finite and > bola_min_buffer", "finite",
+                                            "finite, >= 0 and < switch_on_buffer"};
+        return fail(ABR_ERR_INVALID, "session %d: %s must be %s", s, kSessFieldNames[f], need[f]);
+    }
+    CUDA_TRY(launch_session_params(a, n_sessions, v.cap, env->d_sess, nullptr, st));
+    env->v.sp.tab = env->d_sess;
+    env->v.sp.n = n_sessions;
+    env->v.sp.on = 1;
+    return ABR_OK;
+}
+
+int abr_env_get_session_policy_params(AbrEnv* env, double* d_out, int n_sessions, void* stream) {
+    if (!env || !d_out) return fail(ABR_ERR_INVALID, "env or out is NULL");
+    if (!env->v.sp.on) return fail(ABR_ERR_STATE, "no per-session policy parameters are installed");
+    if (n_sessions != env->v.sp.n)
+        return fail(ABR_ERR_RANGE, "the installed parameters cover %d sessions, not %d", env->v.sp.n, n_sessions);
+    CUDA_TRY(cudaMemcpy2DAsync(d_out, sizeof(double) * n_sessions, env->d_sess, sizeof(double) * env->v.cap,
+                               sizeof(double) * n_sessions, 7, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return ABR_OK;
+}
+
 // A speed table where the speed controller decides (SPEC §7.2).
 static int check_speed_table(const AbrEnv* env, const double* d_speed) {
     if (d_speed && env->v.spd.on) return fail(ABR_ERR_INVALID, "a speed table and the speed controller are exclusive");
@@ -494,6 +570,7 @@ int abr_env_policy_decide(AbrEnv* env, int policy, int32_t* d_action, void* stre
     if (int rc = check_reset(env)) return rc;
     if (env->v.n == 0) return ABR_OK;
     if (!d_action) return fail(ABR_ERR_INVALID, "action is NULL");
+    if (int rc = check_session_params(env, policy, env->v.n)) return rc;
     CUDA_TRY(launch_policy_decide(env->v, policy, d_action, (cudaStream_t)stream));
     return ABR_OK;
 }
@@ -715,6 +792,7 @@ static int env_rollout_any(AbrEnv* env, int policy, uint64_t seed, int steps, co
     if (policy == ABR_POLICY_FIXED && !d_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
     if (!env->v.p.live && (d_speed || d_latency))
         return fail(ABR_ERR_STATE, "speed / latency belong to live mode (SPEC 7): create the environment with live = 1");
+    if (int rc = check_session_params(env, policy, env->v.n)) return rc;
     StepOutputs<OT> o;
     o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
     o.eov = d_end_of_video; o.actions = d_actions_out; o.latency = d_latency;
@@ -930,6 +1008,7 @@ int abr_env_run(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t
     if (policy == ABR_POLICY_FIXED && !d_actions_in && n_sessions > 0 && steps > 0)
         return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
     if (int rc = check_order(env, n_sessions)) return rc;
+    if (int rc = check_session_params(env, policy, n_sessions)) return rc;
     StepOutputs<double> o;
     o.delay = d_delay; o.sleep = d_sleep; o.buffer = d_buffer; o.rebuf = d_rebuf; o.reward = d_reward;
     o.eov = d_end_of_video; o.actions = d_actions_out;
@@ -958,6 +1037,7 @@ int abr_env_run_host(AbrEnv* env, int policy, uint64_t seed, int steps, const in
     if (int rc = check_policy(env, policy)) return rc;
     if (policy == ABR_POLICY_FIXED && !h_actions_in) return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs h_actions_in");
     if (int rc = check_order(env, n_sessions)) return rc;
+    if (int rc = check_session_params(env, policy, n_sessions)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // inputs: device aliases of page-locked buffers (read over PCIe by the kernels), else copies into the scratch
     const int32_t* tid = (const int32_t*)device_alias(h_trace_id);

@@ -144,7 +144,21 @@ struct EnvView {
         int32_t on;
         int32_t pad_[3];
     } spd;
+    // Per-session policy parameters (SPEC §4.7, abr_env_set_session_policy_params): the environment's [kSessFields][cap]
+    // table, row f of caller index c at f * cap + c (rows in the order of SessField), for the n sessions it was
+    // installed for; used while `on`.  Last and 16 bytes, for the reasons given at Policy.
+    struct SessionParams {
+        const double* __restrict__ tab;
+        int32_t n, on;
+    } sp;
 };
+
+// Rows of EnvView::SessionParams::tab: the seven fields of AbrSessionPolicyParams in their order, then BOLA's (Vp, gp)
+// derived from them as install_policy_params derives the environment-wide pair.
+enum SessField { kSpBbaReservoir, kSpBbaCushion, kSpRbSafety, kSpBolaMin, kSpBolaTarget, kSpSwitchOn, kSpSwitchOff,
+                 kSpBolaVp, kSpBolaGp, kSessFields };
+// Bit OR-ed into the POLICY template argument of the episode kernel: its forms with the per-session knobs of SPEC §4.7.
+constexpr int kPolicySession = 16;
 
 // launchers implemented in abr_step.cu / abr_mpc.cu (C++ linkage, internal)
 cudaError_t launch_trace_table(const EnvView& v, double* d_cum, uint16_t* d_idx, int32_t* d_ok, TraceMeta* d_meta,
@@ -215,6 +229,13 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
 // abr_env_policy_decide: the action of policy BBA / RATE / BOLA / DYNAMIC for every session from the SoA state
 // (DYNAMIC also writes the session's active rule)
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st);
+// abr_env_set_session_policy_params (SPEC §4.7): src[f] is the caller's [n] array of field f, or null for the
+// environment-wide value env_wide[f].  With d_first: validation only, which sets *d_first to the smallest
+// 8 * session + field that fails its check (all ones when none does) and writes nothing else.  Without: writes rows
+// 0..6 of the [kSessFields][cap] table d_tab and derives rows 7 and 8.
+struct SessionParamsSrc { const double* src[7]; double env_wide[7]; double bola_vmax; };
+cudaError_t launch_session_params(const SessionParamsSrc& a, int n, int cap, double* d_tab,
+                                  unsigned long long* d_first, cudaStream_t st);
 // abr_env_lookahead_decide (SPEC §4.4): the clairvoyant best sequence over the next min(H, V - chunk) chunks against
 // every session's own trace, H in [1, 8]; d_best_value [N] and d_best_seq [N][H] nullable.  Writes nothing else but
 // the error counter.

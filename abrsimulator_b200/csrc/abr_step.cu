@@ -507,6 +507,26 @@ __device__ __forceinline__ void step_core(const EnvView& v, Sess& s, const int q
     step_tail<SMEM, FAST, LIVE>(v.p, v.V, s, h, q, lk, g, r, want_thr, pow2_inverse(v.p.sleep_quantum));
 }
 
+// Per-session knobs (SPEC §4.7): session c's row of the per-session table, c being the caller's index of the session
+// (the parameters are keyed like the draws of §8).  Only the fields policy P reads are loaded.
+struct SessKnobs { double bba_reservoir, bba_cushion, rb_safety, bola_Vp, bola_gp, dyn_on, dyn_off; };
+
+template <int P>
+__device__ __forceinline__ SessKnobs session_knobs(const EnvView& v, const int i) {
+    const int c = v.perm ? __ldg(v.perm + i) : i;
+    const double* __restrict__ t = v.sp.tab + c;
+    const size_t cap = (size_t)v.cap;
+    SessKnobs k{};
+    if (P == ABR_POLICY_BBA) { k.bba_reservoir = __ldg(t + kSpBbaReservoir * cap); k.bba_cushion = __ldg(t + kSpBbaCushion * cap); }
+    if (P == ABR_POLICY_RATE || P == ABR_POLICY_DYNAMIC) k.rb_safety = __ldg(t + kSpRbSafety * cap);
+    if (P == ABR_POLICY_BOLA || P == ABR_POLICY_DYNAMIC) { k.bola_Vp = __ldg(t + kSpBolaVp * cap); k.bola_gp = __ldg(t + kSpBolaGp * cap); }
+    if (P == ABR_POLICY_DYNAMIC) { k.dyn_on = __ldg(t + kSpSwitchOn * cap); k.dyn_off = __ldg(t + kSpSwitchOff * cap); }
+    return k;
+}
+
+// The rules below come twice: with the environment-wide knobs read from the view, as they were before SPEC §4.7 (so
+// that every form without per-session knobs compiles to the instructions it compiled to before), and with a session's
+// knobs (SessKnobs).  The two versions of a rule must stay the same operations in the same order.
 // SPEC §4, buffer-based policy on the pre-step buffer level.
 __device__ __forceinline__ int policy_bba(const EnvView& v, const double b) {
     const int A = v.A;
@@ -559,6 +579,53 @@ __device__ __forceinline__ int policy_bola(const EnvView& v, const double b, con
 // is dash.js's.
 __device__ __forceinline__ int dynamic_mode(const EnvView& v, const int chunk, const double b, const int prev) {
     return b > (chunk != 0 && prev ? v.pol.dyn_off : v.pol.dyn_on) ? 1 : 0;
+}
+
+// SPEC §4 / §4.2 / §4.3 / §4.6 with session knobs k (SPEC §4.7)
+__device__ __forceinline__ int policy_bba(const EnvView& v, const SessKnobs& k, const double b) {
+    const int A = v.A;
+    if (b < k.bba_reservoir) return 0;
+    if (b >= dadd(k.bba_reservoir, k.bba_cushion)) return A - 1;
+    const int q = (int)floor(ddiv(dmul((double)(A - 1), dsub(b, k.bba_reservoir)), k.bba_cushion));
+    return q > A - 1 ? A - 1 : q;
+}
+
+template <typename SizeAt>
+__device__ __forceinline__ int policy_rate(const EnvView& v, const SessKnobs& k, const int i, const int hist_len,
+                                           const SizeAt& size_at) {
+    const int A = v.A, K = v.K;
+    const int n = hist_len < K ? hist_len : K;
+    if (n == 0) {
+        const int d = v.p.default_quality;
+        return d < 0 ? 0 : (d > A - 1 ? A - 1 : d);
+    }
+    double S = 0.0;
+    for (int j = 0; j < n; ++j) {   // oldest first
+        const int slot = (hist_len - n + j) % K;
+        S = dadd(S, ddiv(1.0, v.bw_hist[(size_t)slot * v.cap + i]));
+    }
+    const double budget = dmul(dmul(k.rb_safety, ddiv((double)n, S)), v.p.chunk_length);
+    int q = 0;
+    for (int a = 0; a < A; ++a)
+        if (size_at(a) <= budget) q = a;
+    return q;
+}
+
+template <typename SizeAt>
+__device__ __forceinline__ int policy_bola(const EnvView& v, const SessKnobs& k, const double b, const int row,
+                                           const SizeAt& size_at) {
+    if (v.pol.bola_vmax <= 0.0) return 0;
+    int q = 0;
+    double best = 0.0;
+    for (int a = 0; a < v.A; ++a) {
+        const double sc = ddiv(dsub(dmul(k.bola_Vp, dadd(__ldg(v.pol.bola_v + row + a), k.bola_gp)), b), size_at(a));
+        if (a == 0 || sc > best) { best = sc; q = a; }
+    }
+    return q;
+}
+
+__device__ __forceinline__ int dynamic_mode(const SessKnobs& k, const int chunk, const double b, const int prev) {
+    return b > (chunk != 0 && prev ? k.dyn_off : k.dyn_on) ? 1 : 0;
 }
 
 // The per-session words of a step that come straight from the SoA state (coalesced: thread i <-> session i).
@@ -1298,11 +1365,16 @@ __device__ __forceinline__ void add_step(EpisodeSums& a, const StepRes& r, const
 // The action and table reads run two steps ahead for the same reason.
 // UNI (with FAST, policies that run ahead): every chunk has the same utility row, so the previous step's utility is
 // the next step's "previous utility" (SPEC §3.4) — carried in a register instead of looked up.
-template <int POLICY, bool SMEM, bool FAST, bool NOOUT, int LIVE, bool UNI, typename OT>
+// POLICY_BITS: the policy, with kPolicySession OR-ed in for the per-session knobs of SPEC §4.7 (BBA, RATE, BOLA and
+// DYNAMIC, general and live forms only), which are loaded once per call, through the session order.
+template <int POLICY_BITS, bool SMEM, bool FAST, bool NOOUT, int LIVE, bool UNI, typename OT>
 __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const int i, const uint32_t seed_lo,
                                                 const uint32_t seed_hi, const int steps, const uint32_t step_base,
                                                 const int32_t* __restrict__ actions_in, const RolloutOut<OT>& o,
                                                 double (&acc_new)[ABR_NUM_ACC], const bool fresh) {
+    constexpr int POLICY = POLICY_BITS & ~kPolicySession;
+    constexpr bool SESS = (POLICY_BITS & kPolicySession) != 0;
+    static_assert(!SESS || (!FAST && !NOOUT && !UNI), "per-session knobs run in the general and live forms only");
     constexpr bool AHEAD = (POLICY == ABR_POLICY_FIXED || POLICY == ABR_POLICY_RANDOM) && !LIVE;
     // the random policy is keyed by the caller's session index, whatever order the environment keeps the sessions in
     const unsigned long long gsession = (unsigned long long)(v.session_base + (v.perm ? __ldg(v.perm + i) : i));
@@ -1318,6 +1390,8 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
     // to the instructions they compiled to before DYNAMIC existed.)
     if constexpr (POLICY == ABR_POLICY_DYNAMIC) packed = v.pol.dyn_mode[i];
     if (LIVE) load_live<LIVE>(v, s, i, o.speed, fresh);
+    SessKnobs kn;
+    if constexpr (SESS) kn = session_knobs<POLICY>(v, i);
     // SPEC §4 action of step t; must be called with increasing t.  FIXED clamps t to the last row so that the
     // calls that run ahead of the final step stay inside the caller's table.
     auto action_at = [&](const int t) -> int {
@@ -1349,6 +1423,10 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             auto size_at = [&](const int a) -> double {
                 return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
             };
+            if constexpr (SESS) {
+                packed = (uint32_t)dynamic_mode(kn, s.chunk, s.buffer, (int)packed);
+                return packed ? policy_bola(v, kn, s.buffer, row, size_at) : policy_rate(v, kn, i, s.hist_len, size_at);
+            }
             packed = (uint32_t)dynamic_mode(v, s.chunk, s.buffer, (int)packed);
             return packed ? policy_bola(v, s.buffer, row, size_at) : policy_rate(v, i, s.hist_len, size_at);
         }
@@ -1360,9 +1438,14 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             auto size_at = [&](const int a) -> double {
                 return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
             };
+            if constexpr (SESS) {
+                if (POLICY == ABR_POLICY_RATE) return policy_rate(v, kn, i, s.hist_len, size_at);
+                return policy_bola(v, kn, s.buffer, row, size_at);
+            }
             if (POLICY == ABR_POLICY_RATE) return policy_rate(v, i, s.hist_len, size_at);
             return policy_bola(v, s.buffer, row, size_at);
         }
+        if constexpr (SESS) return policy_bba(v, kn, s.buffer);
         return policy_bba(v, s.buffer);
     };
     // chunk index / previous quality the step after (chunk, q) will see (SPEC §3.5), without running the step
@@ -1706,6 +1789,35 @@ abr_policy_decide_kernel(EnvView v, int32_t* __restrict__ action) {
     action[i] = q;
 }
 
+// abr_policy_decide_kernel with session knobs (SPEC §4.7): each thread reads only the fields its policy uses.
+template <int POLICY>
+__global__ void __launch_bounds__(kStepBlock)
+abr_policy_decide_session_kernel(EnvView v, int32_t* __restrict__ action) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= v.n) return;
+    const double b = v.buffer[i];
+    const SessKnobs k = session_knobs<POLICY>(v, i);
+    int q;
+    if (POLICY == ABR_POLICY_BBA) {
+        q = policy_bba(v, k, b);
+    } else if (!v.p.auto_reset && v.done[i]) {
+        q = 0;   // chunk == V: no sizes row
+    } else {
+        const int chunk = v.chunk[i];
+        ABR_CHECK(chunk >= 0 && chunk < v.V, "policy row");
+        const int row = chunk * v.A;
+        auto size_at = [&](const int a) -> double { return __ldg(v.sizes + row + a); };
+        if constexpr (POLICY == ABR_POLICY_DYNAMIC) {
+            const int m = dynamic_mode(k, chunk, b, v.pol.dyn_mode[i]);
+            v.pol.dyn_mode[i] = (uint8_t)m;
+            q = m ? policy_bola(v, k, b, row, size_at) : policy_rate(v, k, i, v.hist_len[i], size_at);
+        } else {
+            q = POLICY == ABR_POLICY_RATE ? policy_rate(v, k, i, v.hist_len[i], size_at) : policy_bola(v, k, b, row, size_at);
+        }
+    }
+    action[i] = q;
+}
+
 // ---- SPEC §4.4: clairvoyant lookahead (abr_env_lookahead_decide) ----
 // One thread per (session, first action a0); the A threads of a session sit in consecutive lanes of one warp
 // (32 / A sessions per warp, the remaining lanes idle).  A thread walks the A^(h-1) completions of its a0 depth first
@@ -1815,6 +1927,17 @@ cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double*
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;
     const unsigned grid = (v.n + kStepBlock - 1) / kStepBlock;
+    if (v.sp.on) {   // the per-session knobs of SPEC §4.7
+        switch (policy) {
+            case ABR_POLICY_BBA: abr_policy_decide_session_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+            case ABR_POLICY_RATE: abr_policy_decide_session_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+            case ABR_POLICY_BOLA: abr_policy_decide_session_kernel<ABR_POLICY_BOLA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+            case ABR_POLICY_DYNAMIC: abr_policy_decide_session_kernel<ABR_POLICY_DYNAMIC><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
+            default: return cudaErrorInvalidValue;
+        }
+        count_launch();
+        return cudaGetLastError();
+    }
     switch (policy) {
         case ABR_POLICY_BBA: abr_policy_decide_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
         case ABR_POLICY_RATE: abr_policy_decide_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
@@ -1824,6 +1947,48 @@ cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action
             break;
         default: return cudaErrorInvalidValue;
     }
+    count_launch();
+    return cudaGetLastError();
+}
+
+// SPEC §4.7: one thread per session.  The first field that fails the check the environment-wide setters apply (in the
+// field order), as 8 * session + field, into the minimum at *first; or, without `first`, the session's column of the
+// table with BOLA's (Vp, gp) derived as install_policy_params derives them (fp64, no FMA).
+__global__ void __launch_bounds__(kStepBlock)
+abr_session_params_kernel(const SessionParamsSrc a, int n, int cap, double* __restrict__ tab,
+                          unsigned long long* __restrict__ first) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n) return;
+    double x[7];
+#pragma unroll
+    for (int f = 0; f < 7; ++f) x[f] = a.src[f] ? a.src[f][c] : a.env_wide[f];
+    if (first) {
+        int bad = -1;
+        if (!isfinite(x[kSpBbaReservoir])) bad = kSpBbaReservoir;
+        else if (!isfinite(x[kSpBbaCushion]) || !(x[kSpBbaCushion] > 0.0)) bad = kSpBbaCushion;
+        else if (!isfinite(x[kSpRbSafety]) || !(x[kSpRbSafety] > 0.0)) bad = kSpRbSafety;
+        else if (!isfinite(x[kSpBolaMin]) || !(x[kSpBolaMin] > 0.0)) bad = kSpBolaMin;
+        else if (!isfinite(x[kSpBolaTarget]) || !(x[kSpBolaMin] < x[kSpBolaTarget])) bad = kSpBolaTarget;
+        else if (!isfinite(x[kSpSwitchOn])) bad = kSpSwitchOn;
+        else if (!isfinite(x[kSpSwitchOff]) || !(x[kSpSwitchOff] >= 0.0) || !(x[kSpSwitchOff] < x[kSpSwitchOn]))
+            bad = kSpSwitchOff;
+        if (bad >= 0) atomicMin(first, 8ull * (unsigned long long)c + (unsigned long long)bad);
+        return;
+    }
+#pragma unroll
+    for (int f = 0; f < 7; ++f) tab[(size_t)f * cap + c] = x[f];
+    const double gp = ddiv(a.bola_vmax, dsub(ddiv(x[kSpBolaTarget], x[kSpBolaMin]), 1.0));
+    tab[(size_t)kSpBolaGp * cap + c] = gp;
+    tab[(size_t)kSpBolaVp * cap + c] = ddiv(x[kSpBolaMin], gp);
+}
+
+cudaError_t launch_session_params(const SessionParamsSrc& a, int n, int cap, double* d_tab,
+                                  unsigned long long* d_first, cudaStream_t st) {
+    if (d_first) {
+        cudaError_t e = cudaMemsetAsync(d_first, 0xff, sizeof(unsigned long long), st);
+        if (e != cudaSuccess) return e;
+    }
+    abr_session_params_kernel<<<(n + kStepBlock - 1) / kStepBlock, kStepBlock, 0, st>>>(a, n, cap, d_tab, d_first);
     count_launch();
     return cudaGetLastError();
 }
@@ -1959,6 +2124,16 @@ static cudaError_t launch_rollout_form(const Go& go, const RolloutOut<OT>& o, co
     }
 }
 
+// The episode kernel's per-session form (SPEC §4.7) of a policy that reads the knobs: the general form, also where the
+// environment-wide knobs would take a FAST / NOOUT form (its outputs may be null), or the live form.
+template <int P, typename OT, typename Go>
+static cudaError_t launch_rollout_session_form(const Go& go, const RolloutOut<OT>& o, const int live) {
+    constexpr int PS = P | kPolicySession;
+    if (live == 2) return go(abr_rollout_kernel<PS, false, false, 2, false, OT>, o);
+    if (live == 1) return go(abr_rollout_kernel<PS, false, false, 1, false, OT>, o);
+    return go(abr_rollout_kernel<PS, false, false, 0, false, OT>, o);
+}
+
 template <typename OT>
 cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int steps, uint32_t step_base,
                            const int32_t* d_actions_in, const double* d_speed, const StepOutputs<OT>& out,
@@ -1988,7 +2163,11 @@ cudaError_t launch_rollout(const EnvView& v, int policy, uint64_t seed, int step
         return e;
     };
     cudaError_t e;
-    switch (policy) {
+    if (v.sp.on && policy == ABR_POLICY_BBA) e = launch_rollout_session_form<ABR_POLICY_BBA>(go, o, live);
+    else if (v.sp.on && policy == ABR_POLICY_RATE) e = launch_rollout_session_form<ABR_POLICY_RATE>(go, o, live);
+    else if (v.sp.on && policy == ABR_POLICY_BOLA) e = launch_rollout_session_form<ABR_POLICY_BOLA>(go, o, live);
+    else if (v.sp.on && policy == ABR_POLICY_DYNAMIC) e = launch_rollout_session_form<ABR_POLICY_DYNAMIC>(go, o, live);
+    else switch (policy) {
         case ABR_POLICY_FIXED: e = launch_rollout_form<ABR_POLICY_FIXED>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_RANDOM: e = launch_rollout_form<ABR_POLICY_RANDOM>(go, o, o_none, live, fast, none, uni); break;
         case ABR_POLICY_BBA: e = launch_rollout_form<ABR_POLICY_BBA>(go, o, o_none, live, fast, none, uni); break;

@@ -561,6 +561,53 @@ class BatchedABREnv:
             raise ValueError("a speed table and the speed controller are exclusive: remove the controller with "
                              "set_speed_control(None) to play a table")
 
+    # -- SPEC §4.7 --
+    def set_session_policy_params(self, params=(), n=None, **fields):
+        """Install per-session parameters of the "bba", "rate", "bola" and "dynamic" policies for the following calls,
+        or remove them with ``set_session_policy_params(None)``.  Keyword arguments: any of ``bba_reservoir``,
+        ``bba_cushion``, ``rb_safety``, ``bola_min_buffer``, ``bola_target_buffer``, ``switch_on_buffer`` and
+        ``switch_off_buffer``, each ``[N]`` values in caller order (tensors or array-likes); omitted ones take the
+        environment-wide value current now.  ``n`` defaults to the active batch size.  While they are installed, every
+        fused episode, ``run`` and ``policy_decide`` of those policies must have N sessions, and ``set_policy_params`` /
+        ``set_dynamic_params`` raise.  Invalid values raise, naming the first bad session and field, and leave the
+        previous installation as it was."""
+        if params is None:
+            if fields or n is not None:
+                raise TypeError("set_session_policy_params(None) removes the parameters and takes no others")
+            with self._on:
+                _lib.check(self._lib.abr_env_set_session_policy_params(self._h, None, 0, _stream()))
+            self._session_params_n = 0
+            return
+        if params != ():
+            raise TypeError("set_session_policy_params takes keyword arguments, or None to remove the parameters")
+        for k in fields:
+            if k not in _lib.SESSION_PARAM_FIELDS:
+                raise TypeError(f"unknown per-session policy parameter {k!r}")
+        n = self.n if n is None else int(n)
+        arrays = {}
+        for k, x in fields.items():
+            t = torch.as_tensor(x, dtype=torch.float64, device=self.device).contiguous()
+            if t.dim() != 1 or t.numel() != n:
+                raise ValueError(f"{k} must hold {n} values (one per session), got shape {tuple(t.shape)}")
+            arrays[k] = t
+        sp = _lib.AbrSessionPolicyParams(*[arrays[k].data_ptr() if k in arrays else None
+                                           for k in _lib.SESSION_PARAM_FIELDS])
+        with self._on:
+            # the arrays are copied by a kernel on the current stream, so releasing them afterwards is stream-ordered
+            _lib.check(self._lib.abr_env_set_session_policy_params(self._h, sp, n, _stream()))
+        self._session_params_n = n
+
+    def session_policy_params(self):
+        """The installed per-session parameters (omitted fields filled in) as a dict of seven float64 ``[N]`` tensors
+        in caller order, or None when none are installed."""
+        n = getattr(self, "_session_params_n", 0)
+        if not n:
+            return None
+        out = self._empty(len(_lib.SESSION_PARAM_FIELDS), n)
+        with self._on:
+            _lib.check(self._lib.abr_env_get_session_policy_params(self._h, _addr(out), n, _stream()))
+        return {k: out[j] for j, k in enumerate(_lib.SESSION_PARAM_FIELDS)}
+
     def policy_decide(self, policy, out=None) -> torch.Tensor:
         """The action of a state-dependent built-in policy ("bba", "rate", "bola" or "dynamic") for every session, from
         the environment's own state (int32 [N] on the device); ``step`` with it is one step of the fused episode.
