@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 _SUFFIX = os.environ.get("ABR_LIB_SUFFIX", "")
 LIB = os.path.join(HERE, "lib", f"libabr_b200{_SUFFIX}.so")
 STAMP = LIB + ".srchash"
-SOURCES = ["abr_step.cu", "abr_mpc.cu", "abr_mpc_scen.cu", "abr_capi.cu", "abr_sort.cu"]
+SOURCES = ["abr_step.cu", "abr_mpc.cu", "abr_mpc_scen.cu", "abr_capi.cu", "abr_sort.cu", "abr_shared.cu"]
 HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(CSRC, "abr_mpc_search.cuh"),
            os.path.join(HERE, "..", "include", "abr_b200.h"),
            os.path.join(HERE, "..", "include", "abr_b200_lookahead.h"),
@@ -26,7 +26,8 @@ HEADERS = [os.path.join(CSRC, "abr_common.cuh"), os.path.join(CSRC, "abr_mpc_sea
            os.path.join(HERE, "..", "include", "abr_b200_obs.h"),
            os.path.join(HERE, "..", "include", "abr_b200_dynamic.h"),
            os.path.join(HERE, "..", "include", "abr_b200_speed.h"),
-           os.path.join(HERE, "..", "include", "abr_b200_session_params.h")]
+           os.path.join(HERE, "..", "include", "abr_b200_session_params.h"),
+           os.path.join(HERE, "..", "include", "abr_b200_shared.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"] + os.environ.get("ABR_EXTRA_NVCC_FLAGS", "").split()

@@ -163,6 +163,19 @@ SESSION_PARAMS_SIGNATURES = {
     "abr_env_get_session_policy_params": (_I, [_P, _P, _I, _P]),
 }
 
+# include/abr_b200_shared.h: G players sharing one trace's capacity (SPEC §9).
+class AbrSharedOutputs(C.Structure):
+    """Nullable device pointers of the outputs of abr_env_run_shared: [steps][N] per player, [n_links] per link."""
+    _fields_ = [(n, C.c_void_p) for n in ("d_delay", "d_sleep", "d_buffer", "d_rebuf", "d_reward", "d_request_time",
+                                          "d_end_of_video", "d_actions", "d_link_time", "d_link_capacity",
+                                          "d_link_delivered")]
+
+
+SHARED_SIGNATURES = {
+    "abr_env_run_shared": (_I, [_P, _I, _P, _U64, _I, _I, _P, _P, _P, _I, _LL, _P, C.POINTER(AbrSharedOutputs), _P,
+                                _P, _P]),
+}
+
 _lib = None
 
 
@@ -183,7 +196,7 @@ def load():
     lib = C.CDLL(path)
     for name, (restype, argtypes) in {**SIGNATURES, **EXTRA_SIGNATURES, **MPC_PRED_SIGNATURES, **OBS_SIGNATURES,
                                    **MPC_SCEN_SIGNATURES, **DYNAMIC_SIGNATURES, **SPEED_SIGNATURES,
-                                   **SESSION_PARAMS_SIGNATURES}.items():
+                                   **SESSION_PARAMS_SIGNATURES, **SHARED_SIGNATURES}.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes
     _lib = lib

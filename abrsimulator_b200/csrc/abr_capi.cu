@@ -16,6 +16,7 @@
 #include "../../include/abr_b200_mpc_scen.h"
 #include "../../include/abr_b200_obs.h"
 #include "../../include/abr_b200_session_params.h"
+#include "../../include/abr_b200_shared.h"
 #include "../../include/abr_b200_speed.h"
 
 namespace abr {
@@ -1014,6 +1015,52 @@ int abr_env_run(AbrEnv* env, int policy, uint64_t seed, int steps, const int32_t
     o.eov = d_end_of_video; o.actions = d_actions_out;
     return run_batch(env, policy, seed, steps, d_trace_id, d_start_offset, n_sessions, session_base, d_actions_in, o,
                      d_qoe_cost, d_stats, (cudaStream_t)stream);
+}
+
+int abr_env_run_shared(AbrEnv* env, int policy, const int32_t* h_player_policy, uint64_t seed, int steps,
+                       int players_per_link, const int32_t* d_link_trace_id, const double* d_link_offset,
+                       const double* d_join_delay, int n_links, long long session_base, const int32_t* d_actions_in,
+                       const AbrSharedOutputs* out, double* d_qoe_cost, double* d_stats, void* stream) {
+    if (!env || (!d_link_trace_id && n_links > 0)) return fail(ABR_ERR_INVALID, "env or link_trace_id is NULL");
+    if (env->v.p.live) return fail(ABR_ERR_STATE, "abr_env_run_shared is not available in live mode");
+    if (env->v.perm)
+        return fail(ABR_ERR_STATE, "abr_env_run_shared keeps the players of a link together: remove the session order "
+                                   "(abr_env_set_order(env, NULL, 0, stream)) first");
+    const int G = players_per_link;
+    if (G < 1 || G > 32) return fail(ABR_ERR_RANGE, "players_per_link must be in [1, 32], got %d", G);
+    if (n_links < 0 || (long long)n_links * G > env->v.cap)
+        return fail(ABR_ERR_RANGE, "n_links * players_per_link = %lld exceeds capacity %d (or n_links < 0)",
+                    (long long)n_links * G, env->v.cap);
+    if (steps < 0) return fail(ABR_ERR_RANGE, "steps must be >= 0");
+    const int n_sessions = n_links * G;
+    SharedRun r{};
+    for (int p = 0; p < G; ++p) {
+        const int pol = h_player_policy ? h_player_policy[p] : policy;
+        if (int rc = check_policy(env, pol)) return rc;
+        if (pol == ABR_POLICY_FIXED && !d_actions_in && n_sessions > 0 && steps > 0)
+            return fail(ABR_ERR_INVALID, "ABR_POLICY_FIXED needs d_actions_in");
+        r.policy[p >> 3] |= (uint32_t)pol << (4 * (p & 7));
+    }
+    for (int p = 0; p < G; ++p)
+        if (int rc = check_session_params(env, h_player_policy ? h_player_policy[p] : policy, n_sessions)) return rc;
+    if ((unsigned long long)steps * (unsigned long long)n_sessions > 0xffffffffull)
+        return fail(ABR_ERR_RANGE, "steps * sessions = %llu exceeds 2^32 - 1: split the run into several calls",
+                    (unsigned long long)steps * (unsigned long long)n_sessions);
+    const cudaStream_t st = (cudaStream_t)stream;
+    begin_batch(env, n_sessions, session_base);
+    r.link_trace_id = d_link_trace_id; r.link_offset = d_link_offset; r.join_delay = d_join_delay;
+    r.actions_in = d_actions_in; r.n_links = n_links; r.G = G; r.steps = steps;
+    r.seed_lo = (uint32_t)seed; r.seed_hi = (uint32_t)(seed >> 32);
+    if (out) {
+        r.traj.delay = out->d_delay; r.traj.sleep = out->d_sleep; r.traj.buffer = out->d_buffer;
+        r.traj.rebuf = out->d_rebuf; r.traj.reward = out->d_reward; r.traj.eov = out->d_end_of_video;
+        r.traj.actions = out->d_actions; r.request_time = out->d_request_time;
+        r.link_time = out->d_link_time; r.link_capacity = out->d_link_capacity; r.link_delivered = out->d_link_delivered;
+    }
+    r.qoe_cost = d_qoe_cost;
+    CUDA_TRY(launch_shared(env->v, r, st));
+    env->step_base = (uint32_t)steps;   // every player made `steps` downloads: a later episode draws on from there
+    return d_stats ? abr_stats_partial(env, d_stats, st) : ABR_OK;
 }
 
 // Zero-copy: a host pointer inside page-locked memory (cudaHostAlloc / cudaHostRegister, e.g. a pinned torch tensor)

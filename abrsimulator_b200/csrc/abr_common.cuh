@@ -241,6 +241,19 @@ cudaError_t launch_session_params(const SessionParamsSrc& a, int n, int cap, dou
 // the error counter.
 cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double* d_best_value, int32_t* d_best_seq,
                              cudaStream_t st);
+// abr_env_run_shared (SPEC §9): n_links links of G players, session l*G + p is player p of link l (v.n = n_links*G).
+// policy: the built-in policy of player slot p in bits 4p .. 4p+3 (a packed value: the kernel selects by lane).  Writes the trajectory, request_time and the per-link outputs where
+// non-null, the accumulators, qoe_cost (nullable) and the state of every player.
+struct SharedRun {
+    const int32_t* link_trace_id; const double* link_offset; const double* join_delay; const int32_t* actions_in;
+    int n_links, G, steps;
+    uint32_t seed_lo, seed_hi;
+    uint32_t policy[4];
+    StepOutputs<double> traj;   // [steps][N]: delay, sleep, buffer, rebuf, reward, eov, actions
+    double* request_time;       // [steps][N]
+    double *link_time, *link_capacity, *link_delivered, *qoe_cost;
+};
+cudaError_t launch_shared(const EnvView& v, const SharedRun& r, cudaStream_t st);
 cudaError_t launch_stats(const EnvView& v, double* d_partials, int n_partials, bool have_partials, double* d_out,
                          const StatsScratch& scratch,
                          cudaStream_t st);

@@ -1912,6 +1912,9 @@ abr_lookahead_kernel(EnvView v, const int H, int32_t* __restrict__ action, doubl
 
 }  // namespace
 
+// abr_shared.cu compiles everything above (the step functions its kernel is built from) and none of what follows.
+#ifndef ABR_STEP_DEVICE_ONLY
+
 cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double* d_best_value, int32_t* d_best_seq,
                              cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;
@@ -2227,5 +2230,7 @@ cudaError_t launch_stats(const EnvView& v, double* d_partials, int n_partials, b
     count_launch();
     return cudaGetLastError();
 }
+
+#endif  // ABR_STEP_DEVICE_ONLY
 
 }  // namespace abr

@@ -38,6 +38,13 @@ def _mode_id(mode):
     return int(mode)
 
 
+def jain_index(x) -> torch.Tensor:
+    """Jain's fairness index of each row of ``x`` [n_links, G] (e.g. each player's mean utility or throughput on a
+    shared link): (Σx)² / (G·Σx²), 1 when all G values are equal, 1/G when one player takes everything."""
+    x = torch.as_tensor(x, dtype=torch.float64)
+    return x.sum(-1) ** 2 / (x.shape[-1] * (x * x).sum(-1))
+
+
 class _DevPtr:
     """Minimal __cuda_array_interface__ holder so torch can view library-owned device memory."""
 
@@ -502,6 +509,63 @@ class BatchedABREnv:
         self.n = n
         self.session_base = int(session_base)
         return out, qoe_cost, stats
+
+    # -- SPEC §9: players sharing a bottleneck --
+    def run_shared(self, policy, steps, link_trace_id, players_per_link, link_offset=None, join_delay=None,
+                   player_policy=None, seed=0, session_base=0, actions=None,
+                   want=("delay", "sleep", "buffer", "rebuffer", "reward", "end_of_video", "request_time"),
+                   link_want=("time", "capacity", "delivered"), qoe_cost=None, stats=None):
+        """``n_links`` links of ``players_per_link`` = G players each, sharing each link's trace equally while their
+        downloads overlap (``abr_env_run_shared``, SPEC §9).  Player p of link l is session l*G + p; link l plays trace
+        ``link_trace_id[l]`` from ``link_offset[l]``.  ``join_delay`` [N]: when each player makes its first request.
+        ``player_policy``: G policy names (or ids), slot p of every link runs ``player_policy[p]``; otherwise every
+        player runs ``policy``.  ``want`` names the [steps, N] outputs ("actions" may be added), ``link_want`` the
+        [n_links] ones ("time", "capacity", "delivered").  Returns (out, link_out, qoe_cost, stats), with qoe_cost [N]
+        and stats [NUM_STATS] allocated when None (pass False to skip).  Afterwards the environment holds the N
+        players, as after ``run``."""
+        G = int(players_per_link)
+        tid = self._dev(link_trace_id, torch.int32)
+        n_links = tid.numel()
+        n = n_links * G
+        off = None if link_offset is None else self._dev(link_offset, torch.float64)
+        if off is not None and off.numel() != n_links:
+            raise ValueError("link_offset must have one entry per link")
+        join = None if join_delay is None else self._dev(join_delay, torch.float64)
+        if join is not None and join.numel() != n:
+            raise ValueError(f"join_delay must have one entry per player ({n})")
+        pp = None
+        pids = [_policy_id(policy)]
+        if player_policy is not None:
+            pids = [_policy_id(x) for x in player_policy]
+            if len(pids) != G:
+                raise ValueError(f"player_policy must name {G} policies, one per player slot")
+            pp = np.ascontiguousarray(pids, dtype=np.int32)
+        a_in = None
+        if POLICY_FIXED in pids:
+            if actions is None:
+                raise ValueError("policy 'fixed' needs an actions table [steps, N]")
+            a_in = self._dev(actions, torch.int32)
+            if a_in.numel() != steps * n:
+                raise ValueError("actions must be [steps, N]")
+        out = {}
+        for k in want:
+            dt = torch.uint8 if k == "end_of_video" else torch.int32 if k == "actions" else torch.float64
+            out[k] = self._empty(steps, n, dtype=dt)
+        link_out = {k: self._empty(n_links) for k in link_want}
+        qoe_cost = self._empty(n) if qoe_cost is None else (None if qoe_cost is False else qoe_cost)
+        stats = self._empty(NUM_STATS) if stats is None else (None if stats is False else stats)
+        g, lg = out.get, link_out.get
+        o = _lib.AbrSharedOutputs(_addr(g("delay")), _addr(g("sleep")), _addr(g("buffer")), _addr(g("rebuffer")),
+                                  _addr(g("reward")), _addr(g("request_time")), _addr(g("end_of_video")),
+                                  _addr(g("actions")), _addr(lg("time")), _addr(lg("capacity")),
+                                  _addr(lg("delivered")))
+        with self._on:
+            _lib.check(self._lib.abr_env_run_shared(
+                self._h, pids[0], _addr(pp), seed, steps, G, _addr(tid), _addr(off), _addr(join), n_links,
+                session_base, _addr(a_in), o, _addr(qoe_cost), _addr(stats), _stream()))
+        self.n = n
+        self.session_base = int(session_base)
+        return out, link_out, qoe_cost, stats
 
     # -- SPEC §4.2 / §4.3 --
     def set_policy_params(self, rb_safety=None, bola_min_buffer=None, bola_target_buffer=None):
