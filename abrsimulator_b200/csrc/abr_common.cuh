@@ -157,7 +157,8 @@ struct EnvView {
 // derived from them as install_policy_params derives the environment-wide pair.
 enum SessField { kSpBbaReservoir, kSpBbaCushion, kSpRbSafety, kSpBolaMin, kSpBolaTarget, kSpSwitchOn, kSpSwitchOff,
                  kSpBolaVp, kSpBolaGp, kSessFields };
-// Bit OR-ed into the POLICY template argument of the episode kernel: its forms with the per-session knobs of SPEC §4.7.
+// Bit OR-ed into the POLICY template argument of the episode and decision kernels: their forms with the per-session
+// knobs of SPEC §4.7.
 constexpr int kPolicySession = 16;
 
 // launchers implemented in abr_step.cu / abr_mpc.cu (C++ linkage, internal)

@@ -12,8 +12,8 @@
 // per block) when they fit, the global read-only path otherwise; the choice is launch-uniform (launch_shared).
 //
 // The kernel is built from the step functions of abr_step.cu (head, advance_trace, position_of, lookup_tables,
-// reset_seg_phase, the policy rules and session_knobs), not a restatement of them: this unit compiles that file's
-// device part (ABR_STEP_DEVICE_ONLY).  A unit of its own, so that the module of the step kernels stays as it was.
+// reset_seg_phase, the policy rules, session_knobs and env_knobs), not a restatement of them: this unit compiles that
+// file's device part (ABR_STEP_DEVICE_ONLY).  A unit of its own, so that the module of the step kernels stays as it was.
 #define ABR_STEP_DEVICE_ONLY
 #include "abr_step.cu"
 
@@ -39,11 +39,11 @@ __host__ __device__ __forceinline__ size_t shared_slice_bytes(int T_max) {
     return shared_cum_bytes(T_max) + (size_t)idx_stride(T_max) * 2u;
 }
 
-// SPEC §4 / §4.7 action of a player's download k from its own state.  DYNAMIC updates `mode`.
+// SPEC §4 action of a player's download k from its own state and knobs kn (SPEC §4.7).  DYNAMIC updates `mode`.
 template <bool SMEM>
 __device__ __forceinline__ int shared_action(const EnvView& v, const SharedRun& r, const Sess& s, const int pol,
-                                             const bool sess, const SessKnobs& kn, const int i, const int k,
-                                             uint32_t& mode, bool& flagged) {
+                                             const SessKnobs& kn, const int i, const int k, uint32_t& mode,
+                                             bool& flagged) {
     const int A = v.A;
     if (pol == ABR_POLICY_FIXED) {
         int a = __ldg(r.actions_in + (size_t)k * (size_t)v.n + i);
@@ -57,7 +57,7 @@ __device__ __forceinline__ int shared_action(const EnvView& v, const SharedRun& 
         const uint32_t w = (m >> 1) == 0 ? x.x : (m >> 1) == 1 ? x.y : (m >> 1) == 2 ? x.z : x.w;
         return (int)((((w >> (16u * (m & 1u))) & 0xffffu) * (uint32_t)A) >> 16);
     }
-    if (pol == ABR_POLICY_BBA) return sess ? policy_bba(v, kn, s.buffer) : policy_bba(v, s.buffer);
+    if (pol == ABR_POLICY_BBA) return policy_bba(v, kn, s.buffer);
     if (s.done) return 0;   // chunk == V: no sizes row (the download is inert; DYNAMIC keeps its rule)
     const int row = s.chunk * A;
     ABR_CHECK(s.chunk >= 0 && s.chunk < v.V, "policy row");
@@ -65,12 +65,12 @@ __device__ __forceinline__ int shared_action(const EnvView& v, const SharedRun& 
         return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
     };
     if (pol == ABR_POLICY_DYNAMIC) {
-        mode = (uint32_t)(sess ? dynamic_mode(kn, s.chunk, s.buffer, (int)mode) : dynamic_mode(v, s.chunk, s.buffer, (int)mode));
-        if (mode) return sess ? policy_bola(v, kn, s.buffer, row, size_at) : policy_bola(v, s.buffer, row, size_at);
-        return sess ? policy_rate(v, kn, i, s.hist_len, size_at) : policy_rate(v, i, s.hist_len, size_at);
+        mode = (uint32_t)dynamic_mode(kn, s.chunk, s.buffer, (int)mode);
+        if (mode) return policy_bola(v, kn, s.buffer, row, size_at);
+        return policy_rate(v, kn, i, s.hist_len, size_at);
     }
-    if (pol == ABR_POLICY_RATE) return sess ? policy_rate(v, kn, i, s.hist_len, size_at) : policy_rate(v, i, s.hist_len, size_at);
-    return sess ? policy_bola(v, kn, s.buffer, row, size_at) : policy_bola(v, s.buffer, row, size_at);
+    if (pol == ABR_POLICY_RATE) return policy_rate(v, kn, i, s.hist_len, size_at);
+    return policy_bola(v, kn, s.buffer, row, size_at);
 }
 
 template <bool SMEM>
@@ -127,13 +127,13 @@ abr_shared_kernel(EnvView v, SharedRun r) {
     const double inv_q = pow2_inverse(p.sleep_quantum);
     const uint32_t pw = (lane >> 3) == 0 ? r.policy[0] : (lane >> 3) == 1 ? r.policy[1] : (lane >> 3) == 2 ? r.policy[2] : r.policy[3];
     const int pol = valid ? (int)((pw >> (4 * (lane & 7))) & 0xfu) : ABR_POLICY_FIXED;
-    const bool sess = v.sp.on && pol >= ABR_POLICY_BBA && pol <= ABR_POLICY_DYNAMIC;
-    SessKnobs kn{};
-    if (valid && sess) {
+    // the player's knobs: its own while per-session knobs are installed, the environment-wide ones otherwise
+    SessKnobs kn = env_knobs(v);
+    if (valid && v.sp.on) {
         if (pol == ABR_POLICY_BBA) kn = session_knobs<ABR_POLICY_BBA>(v, i);
         else if (pol == ABR_POLICY_RATE) kn = session_knobs<ABR_POLICY_RATE>(v, i);
         else if (pol == ABR_POLICY_BOLA) kn = session_knobs<ABR_POLICY_BOLA>(v, i);
-        else kn = session_knobs<ABR_POLICY_DYNAMIC>(v, i);
+        else if (pol == ABR_POLICY_DYNAMIC) kn = session_knobs<ABR_POLICY_DYNAMIC>(v, i);
     }
     uint32_t mode = (valid && pol == ABR_POLICY_DYNAMIC) ? v.pol.dyn_mode[i] : 0u;
     bool flagged = false;
@@ -154,7 +154,7 @@ abr_shared_kernel(EnvView v, SharedRun r) {
     auto requests = [&]() {
         while (state == kWaiting && wait <= 0.0) {
             if (k >= steps) { state = kFinished; break; }   // the sleep after the last download is over
-            q = shared_action<SMEM>(v, r, s, pol, sess, kn, i, k, mode, flagged);
+            q = shared_action<SMEM>(v, r, s, pol, kn, i, k, mode, flagged);
             req_time = clock;
             if (!p.auto_reset && s.done) {   // SPEC §3's inert step: no link time, counts as a download
                 const size_t ix = (size_t)k * N + i;

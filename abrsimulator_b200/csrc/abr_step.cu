@@ -507,8 +507,9 @@ __device__ __forceinline__ void step_core(const EnvView& v, Sess& s, const int q
     step_tail<SMEM, FAST, LIVE>(v.p, v.V, s, h, q, lk, g, r, want_thr, pow2_inverse(v.p.sleep_quantum));
 }
 
-// Per-session knobs (SPEC §4.7): session c's row of the per-session table, c being the caller's index of the session
-// (the parameters are keyed like the draws of §8).  Only the fields policy P reads are loaded.
+// The knobs of the policy rules below: a session's (SPEC §4.7) or the environment-wide ones.  session_knobs: session
+// c's row of the per-session table, c being the caller's index of the session (the parameters are keyed like the draws
+// of §8); only the fields policy P reads are loaded.
 struct SessKnobs { double bba_reservoir, bba_cushion, rb_safety, bola_Vp, bola_gp, dyn_on, dyn_off; };
 
 template <int P>
@@ -524,64 +525,13 @@ __device__ __forceinline__ SessKnobs session_knobs(const EnvView& v, const int i
     return k;
 }
 
-// The rules below come twice: with the environment-wide knobs read from the view, as they were before SPEC §4.7 (so
-// that every form without per-session knobs compiles to the instructions it compiled to before), and with a session's
-// knobs (SessKnobs).  The two versions of a rule must stay the same operations in the same order.
+// The environment-wide knobs, all seven: kernel parameters, so a field no rule of the caller reads is never loaded.
+__device__ __forceinline__ SessKnobs env_knobs(const EnvView& v) {
+    return SessKnobs{v.p.bba_reservoir, v.p.bba_cushion, v.pol.rb_safety, v.pol.bola_Vp, v.pol.bola_gp, v.pol.dyn_on,
+                     v.pol.dyn_off};
+}
+
 // SPEC §4, buffer-based policy on the pre-step buffer level.
-__device__ __forceinline__ int policy_bba(const EnvView& v, const double b) {
-    const int A = v.A;
-    if (b < v.p.bba_reservoir) return 0;
-    if (b >= dadd(v.p.bba_reservoir, v.p.bba_cushion)) return A - 1;
-    const int q = (int)floor(ddiv(dmul((double)(A - 1), dsub(b, v.p.bba_reservoir)), v.p.bba_cushion));
-    return q > A - 1 ? A - 1 : q;
-}
-
-// SPEC §4.2, rate-based policy: the highest quality whose size fits rb_safety * (harmonic mean of the last
-// min(hist_len, K) throughput samples) * L.  Session i's ring is column i of bw_hist[K][cap], newest sample at slot
-// (hist_len - 1) mod K; it is read with plain loads (the fused episode writes it as it goes).  size_at(a): the size of
-// quality a of the session's current chunk.
-template <typename SizeAt>
-__device__ __forceinline__ int policy_rate(const EnvView& v, const int i, const int hist_len, const SizeAt& size_at) {
-    const int A = v.A, K = v.K;
-    const int n = hist_len < K ? hist_len : K;
-    if (n == 0) {
-        const int d = v.p.default_quality;
-        return d < 0 ? 0 : (d > A - 1 ? A - 1 : d);
-    }
-    double S = 0.0;
-    for (int j = 0; j < n; ++j) {   // oldest first
-        const int slot = (hist_len - n + j) % K;
-        S = dadd(S, ddiv(1.0, v.bw_hist[(size_t)slot * v.cap + i]));
-    }
-    const double budget = dmul(dmul(v.pol.rb_safety, ddiv((double)n, S)), v.p.chunk_length);
-    int q = 0;
-    for (int a = 0; a < A; ++a)
-        if (size_at(a) <= budget) q = a;   // a NaN budget fits nothing
-    return q;
-}
-
-// SPEC §4.3, BOLA: the first quality of the largest score (Vp * (v[chunk][a] + gp) - buffer) / size[chunk][a] on the
-// pre-step buffer b; v is the host-built log table (bola_v, read-only path).  row: first element of the chunk's row.
-template <typename SizeAt>
-__device__ __forceinline__ int policy_bola(const EnvView& v, const double b, const int row, const SizeAt& size_at) {
-    if (v.pol.bola_vmax <= 0.0) return 0;   // every ladder flat
-    int q = 0;
-    double best = 0.0;
-    for (int a = 0; a < v.A; ++a) {
-        const double sc = ddiv(dsub(dmul(v.pol.bola_Vp, dadd(__ldg(v.pol.bola_v + row + a), v.pol.bola_gp)), b), size_at(a));
-        if (a == 0 || sc > best) { best = sc; q = a; }
-    }
-    return q;
-}
-
-// SPEC §4.6, DYNAMIC: the rule of this decision (1 = BOLA, 0 = RATE) from the one the session's last DYNAMIC decision
-// left, prev, and the pre-step buffer b.  Chunk 0 ignores prev, so every episode starts on the rate rule; the strict >
-// is dash.js's.
-__device__ __forceinline__ int dynamic_mode(const EnvView& v, const int chunk, const double b, const int prev) {
-    return b > (chunk != 0 && prev ? v.pol.dyn_off : v.pol.dyn_on) ? 1 : 0;
-}
-
-// SPEC §4 / §4.2 / §4.3 / §4.6 with session knobs k (SPEC §4.7)
 __device__ __forceinline__ int policy_bba(const EnvView& v, const SessKnobs& k, const double b) {
     const int A = v.A;
     if (b < k.bba_reservoir) return 0;
@@ -590,6 +540,10 @@ __device__ __forceinline__ int policy_bba(const EnvView& v, const SessKnobs& k, 
     return q > A - 1 ? A - 1 : q;
 }
 
+// SPEC §4.2, rate-based policy: the highest quality whose size fits rb_safety * (harmonic mean of the last
+// min(hist_len, K) throughput samples) * L.  Session i's ring is column i of bw_hist[K][cap], newest sample at slot
+// (hist_len - 1) mod K; it is read with plain loads (the fused episode writes it as it goes).  size_at(a): the size of
+// quality a of the session's current chunk.
 template <typename SizeAt>
 __device__ __forceinline__ int policy_rate(const EnvView& v, const SessKnobs& k, const int i, const int hist_len,
                                            const SizeAt& size_at) {
@@ -607,14 +561,16 @@ __device__ __forceinline__ int policy_rate(const EnvView& v, const SessKnobs& k,
     const double budget = dmul(dmul(k.rb_safety, ddiv((double)n, S)), v.p.chunk_length);
     int q = 0;
     for (int a = 0; a < A; ++a)
-        if (size_at(a) <= budget) q = a;
+        if (size_at(a) <= budget) q = a;   // a NaN budget fits nothing
     return q;
 }
 
+// SPEC §4.3, BOLA: the first quality of the largest score (Vp * (v[chunk][a] + gp) - buffer) / size[chunk][a] on the
+// pre-step buffer b; v is the host-built log table (bola_v, read-only path).  row: first element of the chunk's row.
 template <typename SizeAt>
 __device__ __forceinline__ int policy_bola(const EnvView& v, const SessKnobs& k, const double b, const int row,
                                            const SizeAt& size_at) {
-    if (v.pol.bola_vmax <= 0.0) return 0;
+    if (v.pol.bola_vmax <= 0.0) return 0;   // every ladder flat
     int q = 0;
     double best = 0.0;
     for (int a = 0; a < v.A; ++a) {
@@ -624,6 +580,9 @@ __device__ __forceinline__ int policy_bola(const EnvView& v, const SessKnobs& k,
     return q;
 }
 
+// SPEC §4.6, DYNAMIC: the rule of this decision (1 = BOLA, 0 = RATE) from the one the session's last DYNAMIC decision
+// left, prev, and the pre-step buffer b.  Chunk 0 ignores prev, so every episode starts on the rate rule; the strict >
+// is dash.js's.
 __device__ __forceinline__ int dynamic_mode(const SessKnobs& k, const int chunk, const double b, const int prev) {
     return b > (chunk != 0 && prev ? k.dyn_off : k.dyn_on) ? 1 : 0;
 }
@@ -1416,6 +1375,10 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             }
             return (int)((packed >> (4 * (tg & 7u))) & 0xfu);
         }
+        // the rules' knobs: the session's, loaded once per call, or the environment-wide ones, read from the view here
+        SessKnobs k;
+        if constexpr (SESS) k = kn;
+        else k = env_knobs(v);
         if constexpr (POLICY == ABR_POLICY_DYNAMIC) {   // only the active rule is evaluated
             if (!FAST && s.done) return 0;   // chunk == V: no sizes row (the step is inert, the rule is kept)
             const int row = s.chunk * v.A;
@@ -1423,12 +1386,8 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             auto size_at = [&](const int a) -> double {
                 return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
             };
-            if constexpr (SESS) {
-                packed = (uint32_t)dynamic_mode(kn, s.chunk, s.buffer, (int)packed);
-                return packed ? policy_bola(v, kn, s.buffer, row, size_at) : policy_rate(v, kn, i, s.hist_len, size_at);
-            }
-            packed = (uint32_t)dynamic_mode(v, s.chunk, s.buffer, (int)packed);
-            return packed ? policy_bola(v, s.buffer, row, size_at) : policy_rate(v, i, s.hist_len, size_at);
+            packed = (uint32_t)dynamic_mode(k, s.chunk, s.buffer, (int)packed);
+            return packed ? policy_bola(v, k, s.buffer, row, size_at) : policy_rate(v, k, i, s.hist_len, size_at);
         }
         if (POLICY == ABR_POLICY_RATE || POLICY == ABR_POLICY_BOLA) {
             if (!FAST && s.done) return 0;   // chunk == V: no sizes row (the step is inert)
@@ -1438,15 +1397,10 @@ __device__ __forceinline__ void rollout_session(const EnvView& v, Sess& s, const
             auto size_at = [&](const int a) -> double {
                 return SMEM ? lds_f64(s.tab_s + 16u * (uint32_t)(row + a)) : __ldg(&s.tab[row + a].x);
             };
-            if constexpr (SESS) {
-                if (POLICY == ABR_POLICY_RATE) return policy_rate(v, kn, i, s.hist_len, size_at);
-                return policy_bola(v, kn, s.buffer, row, size_at);
-            }
-            if (POLICY == ABR_POLICY_RATE) return policy_rate(v, i, s.hist_len, size_at);
-            return policy_bola(v, s.buffer, row, size_at);
+            if (POLICY == ABR_POLICY_RATE) return policy_rate(v, k, i, s.hist_len, size_at);
+            return policy_bola(v, k, s.buffer, row, size_at);
         }
-        if constexpr (SESS) return policy_bba(v, kn, s.buffer);
-        return policy_bba(v, s.buffer);
+        return policy_bba(v, k, s.buffer);
     };
     // chunk index / previous quality the step after (chunk, q) will see (SPEC §3.5), without running the step
     const int V_ = v.V, dq_ = v.p.default_quality;
@@ -1761,42 +1715,19 @@ abr_qoe_cost_kernel(EnvView v, double* __restrict__ out) {
 }
 
 // abr_env_policy_decide: one thread per session, the same policy functions as the fused episode's action_at, on the
-// state the next step starts from (in live mode the buffer before the pause gate, as in the episode).
-template <int POLICY>
+// state the next step starts from (in live mode the buffer before the pause gate, as in the episode).  POLICY_BITS: the
+// policy, with kPolicySession OR-ed in for the per-session knobs of SPEC §4.7 (each thread reads only the fields its
+// policy uses).
+template <int POLICY_BITS>
 __global__ void __launch_bounds__(kStepBlock)
 abr_policy_decide_kernel(EnvView v, int32_t* __restrict__ action) {
+    constexpr int POLICY = POLICY_BITS & ~kPolicySession;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= v.n) return;
     const double b = v.buffer[i];
-    int q;
-    if (POLICY == ABR_POLICY_BBA) {
-        q = policy_bba(v, b);
-    } else if (!v.p.auto_reset && v.done[i]) {
-        q = 0;   // chunk == V: no sizes row
-    } else {
-        const int chunk = v.chunk[i];
-        ABR_CHECK(chunk >= 0 && chunk < v.V, "policy row");
-        const int row = chunk * v.A;
-        auto size_at = [&](const int a) -> double { return __ldg(v.sizes + row + a); };
-        if constexpr (POLICY == ABR_POLICY_DYNAMIC) {
-            const int m = dynamic_mode(v, chunk, b, v.pol.dyn_mode[i]);
-            v.pol.dyn_mode[i] = (uint8_t)m;
-            q = m ? policy_bola(v, b, row, size_at) : policy_rate(v, i, v.hist_len[i], size_at);
-        } else {
-            q = POLICY == ABR_POLICY_RATE ? policy_rate(v, i, v.hist_len[i], size_at) : policy_bola(v, b, row, size_at);
-        }
-    }
-    action[i] = q;
-}
-
-// abr_policy_decide_kernel with session knobs (SPEC §4.7): each thread reads only the fields its policy uses.
-template <int POLICY>
-__global__ void __launch_bounds__(kStepBlock)
-abr_policy_decide_session_kernel(EnvView v, int32_t* __restrict__ action) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= v.n) return;
-    const double b = v.buffer[i];
-    const SessKnobs k = session_knobs<POLICY>(v, i);
+    SessKnobs k;
+    if constexpr ((POLICY_BITS & kPolicySession) != 0) k = session_knobs<POLICY>(v, i);
+    else k = env_knobs(v);
     int q;
     if (POLICY == ABR_POLICY_BBA) {
         q = policy_bba(v, k, b);
@@ -1927,27 +1858,21 @@ cudaError_t launch_lookahead(const EnvView& v, int H, int32_t* d_action, double*
     return cudaGetLastError();
 }
 
+// The decision kernel of policy P: its per-session form (SPEC §4.7) while the per-session knobs are installed.
+template <int P>
+static void launch_decide_form(const EnvView& v, int32_t* d_action, cudaStream_t st) {
+    const unsigned grid = (v.n + kStepBlock - 1) / kStepBlock;
+    if (v.sp.on) abr_policy_decide_kernel<P | kPolicySession><<<grid, kStepBlock, 0, st>>>(v, d_action);
+    else abr_policy_decide_kernel<P><<<grid, kStepBlock, 0, st>>>(v, d_action);
+}
+
 cudaError_t launch_policy_decide(const EnvView& v, int policy, int32_t* d_action, cudaStream_t st) {
     if (v.n == 0) return cudaSuccess;
-    const unsigned grid = (v.n + kStepBlock - 1) / kStepBlock;
-    if (v.sp.on) {   // the per-session knobs of SPEC §4.7
-        switch (policy) {
-            case ABR_POLICY_BBA: abr_policy_decide_session_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-            case ABR_POLICY_RATE: abr_policy_decide_session_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-            case ABR_POLICY_BOLA: abr_policy_decide_session_kernel<ABR_POLICY_BOLA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-            case ABR_POLICY_DYNAMIC: abr_policy_decide_session_kernel<ABR_POLICY_DYNAMIC><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-            default: return cudaErrorInvalidValue;
-        }
-        count_launch();
-        return cudaGetLastError();
-    }
     switch (policy) {
-        case ABR_POLICY_BBA: abr_policy_decide_kernel<ABR_POLICY_BBA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-        case ABR_POLICY_RATE: abr_policy_decide_kernel<ABR_POLICY_RATE><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-        case ABR_POLICY_BOLA: abr_policy_decide_kernel<ABR_POLICY_BOLA><<<grid, kStepBlock, 0, st>>>(v, d_action); break;
-        case ABR_POLICY_DYNAMIC:
-            abr_policy_decide_kernel<ABR_POLICY_DYNAMIC><<<grid, kStepBlock, 0, st>>>(v, d_action);
-            break;
+        case ABR_POLICY_BBA: launch_decide_form<ABR_POLICY_BBA>(v, d_action, st); break;
+        case ABR_POLICY_RATE: launch_decide_form<ABR_POLICY_RATE>(v, d_action, st); break;
+        case ABR_POLICY_BOLA: launch_decide_form<ABR_POLICY_BOLA>(v, d_action, st); break;
+        case ABR_POLICY_DYNAMIC: launch_decide_form<ABR_POLICY_DYNAMIC>(v, d_action, st); break;
         default: return cudaErrorInvalidValue;
     }
     count_launch();

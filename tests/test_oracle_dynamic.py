@@ -311,14 +311,14 @@ def test_the_gpu_cases_reach_every_form():
         assert re.search(rf"^def {name}\(", src, re.M), name
 
 
-def test_the_restated_dispatch_matches_the_source():
+def test_the_restated_dispatch_matches_the_source_of_one_decision_kernel():
     with open(os.path.join(ROOT, "abrsimulator_b200", "csrc", "abr_step.cu")) as f:
         src = " ".join(f.read().split())
     assert "if constexpr (P == ABR_POLICY_RATE || P == ABR_POLICY_DYNAMIC) { if (fast || none) return cudaErrorInvalidValue; " \
            "return go(abr_rollout_kernel<P, false, false, false, false, OT>, o);" in src
     assert "if (live) return go(abr_rollout_kernel<P, false, false, true, false, OT>, o);" in src
     assert "case ABR_POLICY_DYNAMIC: e = launch_rollout_form<ABR_POLICY_DYNAMIC>(go, o, o_none, live, fast, none, uni);" in src
-    assert ("case ABR_POLICY_DYNAMIC: abr_policy_decide_kernel<ABR_POLICY_DYNAMIC><<<grid, kStepBlock, 0, st>>>(v, d_action);"
-            in src)
+    assert "case ABR_POLICY_DYNAMIC: launch_decide_form<ABR_POLICY_DYNAMIC>(v, d_action, st); break;" in src
+    assert "else abr_policy_decide_kernel<P><<<grid, kStepBlock, 0, st>>>(v, d_action);" in src
     # the episode's forms exist for fp64 and fp32 outputs: launch_rollout is instantiated for both
     assert "template cudaError_t launch_rollout<double>(" in src and "template cudaError_t launch_rollout<float>(" in src

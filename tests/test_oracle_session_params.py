@@ -205,7 +205,7 @@ EPISODE_FORMS = {(p, live, ot) for p in NAMES for live in (0, 1, 2) for ot in ("
 DECIDE_FORMS = set(NAMES)
 
 
-def test_the_dispatch_names_exactly_the_new_forms():
+def test_the_dispatch_names_exactly_the_per_session_forms():
     with open(os.path.join(ROOT, "abrsimulator_b200", "csrc", "abr_step.cu")) as f:
         src = " ".join(f.read().split())
     # the episode: one per-session form per live mode, for each of the four policies, instantiated for both output types
@@ -216,7 +216,10 @@ def test_the_dispatch_names_exactly_the_new_forms():
                       src)
     assert sorted(a for a, b in pols if a == b) == sorted(NAMES.values())
     assert "template cudaError_t launch_rollout<double>(" in src and "template cudaError_t launch_rollout<float>(" in src
-    dec = re.findall(r"case ABR_POLICY_(\w+): abr_policy_decide_session_kernel<ABR_POLICY_(\w+)>", src)
+    # the decision: the per-session form of each of the four policies while the knobs are installed
+    assert ("if (v.sp.on) abr_policy_decide_kernel<P | kPolicySession><<<grid, kStepBlock, 0, st>>>(v, d_action); "
+            "else abr_policy_decide_kernel<P><<<grid, kStepBlock, 0, st>>>(v, d_action);") in src
+    dec = re.findall(r"case ABR_POLICY_(\w+): launch_decide_form<ABR_POLICY_(\w+)>\(v, d_action, st\);", src)
     assert sorted(a for a, b in dec if a == b) == sorted(NAMES.values())
     assert len(EPISODE_FORMS) == 24 and len(DECIDE_FORMS) == 4
 
